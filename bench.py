@@ -6,7 +6,7 @@ hg19-vs-hg18-shaped set (3,095,677,412 target bp), STRONG scaling over N GPUs: t
 the C++ multi-GPU layer (sccg_mgpu_assign), every rank works through its own pairs, and the encoded record streams are
 gathered to rank 0 over NCCL (sccg_mgpu_gather) inside the timed region.  A "step" is one pass over the whole genome.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0):
     value / ms_per_step   compression, inputs resident in HBM: per rank the device time of its calls (CUDA events on the
@@ -20,6 +20,14 @@ One JSON line on stdout (rank 0):
     chr1_sharded (N > 1)  one chromosome over all ranks by segment range (sccg_mgpu_compress_sharded)
     cpu_baseline          the reference's CPU implementation on a bounded sample, same box (N = 1 only)
     verified_against_oracle / parity_vs_reference   untimed byte comparisons of the outputs that were timed
+
+--dump-outputs DIR (rank 0) writes what the timed legs returned in their last step as DIR/<name>.npy, one float32 value per
+output byte (float64 for lengths), so that two builds can be compared output for output on the same seeded inputs:
+    genome_compressed          the 24 encoded streams of the headline leg, back to back in pair order (sampled)
+    genome_compressed_lengths  their lengths
+    genome_decompressed_pair<i>  the FASTA image of rank 0's last pair from the end-to-end decompression leg (sampled)
+    <global pair>_compressed / _decompressed   the end-to-end outputs of the two global-mode pairs (sampled)
+An output longer than its share of the 64 MB budget is sampled: 4 KiB blocks at positions drawn with a fixed seed.
 """
 from __future__ import annotations
 
@@ -38,6 +46,8 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
+if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # run as the benchmark, it leaves the tree as it found it (it may be read-only)
 
 METRIC = "compress Mbp/s (decompress Gbp/s in `decompress`), whole-genome 24-pair synthetic hg19-vs-hg18 shape"
 CHR1_HEADER = b">chr1 synthetic hg19-vs-hg18 shape"
@@ -127,8 +137,8 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------------------------
-# reference arm / CPU baseline: the reference's own CPU implementation (oracle/_ref when it was
-# compiled from /root/reference, else the C oracle port), timed on this box's host cores.
+# reference arm / CPU baseline: the reference's own CPU implementation (oracle/_ref where build() could
+# compile it from the reference's sources, else the C oracle port), timed on this box's host cores.
 # ----------------------------------------------------------------------------------------------
 def _ref_compress_worker(args):
     """one process: reference `compress` + `decompress` executables on one FASTA slice; keeps the two output files"""
@@ -264,6 +274,21 @@ def fasta_image(header: bytes, tgt) -> bytes:
     return header + b"\n" + body.tobytes() + (tail + b"\n" if tail else b"")
 
 
+DUMP_BLOCK = 4096
+
+
+def dump_sample(data, cap: int):
+    """bytes / uint8 array -> float32 array of every byte, or of `cap` bytes in DUMP_BLOCK-sized blocks whose positions are
+    drawn with a fixed seed (in ascending order) when the output is longer than that"""
+    import numpy as np
+    a = np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray)) else np.asarray(data, dtype=np.uint8)
+    if a.size > cap:
+        blocks = a[:a.size // DUMP_BLOCK * DUMP_BLOCK].reshape(-1, DUMP_BLOCK)
+        pick = np.sort(np.random.default_rng(0).choice(blocks.shape[0], cap // DUMP_BLOCK, replace=False))
+        a = blocks[pick].ravel()
+    return a.astype(np.float32)
+
+
 def oracle_compress_many(items: list) -> list[bytes]:
     """the C oracle (test infrastructure: the checker) on several pairs at once: ctypes releases the GIL, one thread per pair"""
     import concurrent.futures as cf
@@ -295,7 +320,12 @@ def main() -> None:
     ap.add_argument("--no-ref-full", action="store_true", help="reference arm: skip the one-off full chr1-sized run")
     ap.add_argument("--size", type=int, default=0, help="reference arm: bp of the chr1-sized pair generated for the slices (default: as many as the cores need)")
     ap.add_argument("--cpu-sample", type=int, default=20_000_000, help="bp of the chr1-sized pair timed on 1 host core as cpu_baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -386,14 +416,15 @@ def main() -> None:
         return dev_ms, nl, items
 
     def genome_decompress(device_resident: bool):
-        dev_ms, nl = 0.0, 0
+        """one pass over this rank's pairs -> (device ms, launches, output length of the last pair)"""
+        dev_ms, nl, n_out = 0.0, 0, 0
         for i, p in pairs.items():
             if device_resident:
-                ctx.reconstruct_device(p["d_ref"].data_ptr(), p["nr"], p["d_body"].data_ptr(), p["n_body"], d_n.data_ptr(), 0, p["d_low"].data_ptr(), p["n_low"])
+                _, n_out = ctx.reconstruct_device(p["d_ref"].data_ptr(), p["nr"], p["d_body"].data_ptr(), p["n_body"], d_n.data_ptr(), 0, p["d_low"].data_ptr(), p["n_low"])
             else:
-                ctx.decompress_into(_cbuf(p["h_ref"], p["nr"]), _cbuf(p["h_inter"]), h_out.data_ptr(), h_out.numel())
+                n_out = ctx.decompress_into(_cbuf(p["h_ref"], p["nr"]), _cbuf(p["h_inter"]), h_out.data_ptr(), h_out.numel())
             pr = ctx.profile(); dev_ms += pr["kernels_ms"]; nl += pr["launches"]
-        return dev_ms, nl
+        return dev_ms, nl, n_out
 
     for _ in range(args.warmup):
         genome_compress(True); genome_decompress(True); genome_compress(False); genome_decompress(False)
@@ -414,12 +445,21 @@ def main() -> None:
 
     K = args.steps
     res = {}
+    dump = {} if args.dump_outputs and rank == 0 else None
     with ClockSampler(local_rank) as clocks:
         res["c_dev"] = timed(lambda: genome_compress(True), K)
+        if dump is not None:                                      # the gathered streams live until the next gather
+            d_streams, spans = res["c_dev"][2][2]
+            streams = b"".join(ctx.download(d_streams + spans[i][0], spans[i][1]) for i in sorted(spans))
+            dump["genome_compressed"] = dump_sample(streams, 5 << 20)
+            dump["genome_compressed_lengths"] = np.array([spans[i][1] for i in sorted(spans)], dtype=np.float64)
+            del streams
         res["d_dev"] = timed(lambda: genome_decompress(True), K)
         res["c_e2e"] = timed(lambda: genome_compress(False), K)
         gathered = res["c_e2e"][2][2]
         res["d_e2e"] = timed(lambda: genome_decompress(False), K)
+        if dump is not None:                                      # h_out holds the last pair's image until the chr1 leg below
+            dump[f"genome_decompressed_pair{list(pairs)[-1]}"] = dump_sample(h_out[:res["d_e2e"][2][2]].numpy(), 3 << 20)
 
         # ---- chr1-sized pair on ONE GPU (BASELINE configs[1]): rank 0 owns pair 0; the other ranks wait at the barrier
         chr1 = None
@@ -479,10 +519,15 @@ def main() -> None:
         if rank == 0 and not args.no_global:
             for name, cfg, gen in (("global_gap_chr19", 1, lambda s: synth.global_gap_pair(int(63_811_651 * s), int(59_128_983 * s), synth.seed_for(1, 0))),
                                    ("global_divergent_chr21", 3, lambda s: synth.divergent_pair(int(48_129_895 * s), synth.seed_for(3, 0)))):
-                glob[name] = global_bench(ctx, ol, gen, args, name, cfg)
+                glob[name] = global_bench(ctx, ol, gen, args, name, cfg, dump)
                 launches += glob[name].pop("_launches")
         barrier()
     launches = int(reduce(float(launches), "sum"))
+    if dump is not None:
+        assert sum(a.nbytes for a in dump.values()) <= 64_000_000
+        args.dump_outputs.mkdir(parents=True, exist_ok=True)
+        for name, a in dump.items():
+            np.save(args.dump_outputs / f"{name}.npy", a)
 
     # ---- the host's PCIe ceiling with all ranks copying at once (plain cudaMemcpyAsync from / to page-locked memory, no kernels):
     #      what the end-to-end numbers above can reach at most on this box
@@ -618,9 +663,10 @@ def main() -> None:
         dist.destroy_process_group()
 
 
-def global_bench(ctx, ol, gen, args, name: str, cfg: int) -> dict:
+def global_bench(ctx, ol, gen, args, name: str, cfg: int, dump: dict | None) -> dict:
     """one global-mode pair at full size on one GPU: device-resident + end to end, rooflines of the index build and of the
-    parse, the reference beside it on a bounded sample, output verified against the oracle (untimed)"""
+    parse, the reference beside it on a bounded sample, output verified against the oracle (untimed); the end-to-end
+    outputs of the last step go to `dump` when it is given"""
     import torch
     full = args.scale == 1.0
     ref_np, tgt_np = gen(1.0 if full else args.scale)
@@ -629,7 +675,7 @@ def global_bench(ctx, ol, gen, args, name: str, cfg: int) -> dict:
     pad = torch.zeros(64, dtype=torch.uint8)
     h_ref = torch.cat([torch.from_numpy(ref_np), pad]).pin_memory(); h_tgt = torch.cat([torch.from_numpy(tgt_np), pad]).pin_memory()
     d_ref, d_tgt = h_ref.cuda(), h_tgt.cuda()
-    K = max(3, args.steps // 2)
+    K = args.steps
     for _ in range(2):
         ptr, n, mode = ctx.compress_device(d_ref.data_ptr(), nr, d_tgt.data_ptr(), nt, header)
     assert mode == 1, "pair did not take the global path"
@@ -649,6 +695,8 @@ def global_bench(ctx, ol, gen, args, name: str, cfg: int) -> dict:
         nl += ctx.profile()["launches"]
     e2e_ms = (time.perf_counter() - t0) * 1e3 / K
     assert bytes(h_enc[:e_len].numpy()) == enc
+    if dump is not None:
+        dump[name + "_compressed"] = dump_sample(h_enc[:e_len].numpy(), 2 << 20)
     # decompression of the same record stream
     h_inter = torch.frombuffer(bytearray(enc), dtype=torch.uint8).pin_memory()
     h_out = torch.empty(nt + nt // 50 + 4096, dtype=torch.uint8).pin_memory()
@@ -658,6 +706,8 @@ def global_bench(ctx, ol, gen, args, name: str, cfg: int) -> dict:
         d_len = ctx.decompress_into(_cbuf(h_ref, nr), _cbuf(h_inter), h_out.data_ptr(), h_out.numel())
         dpr = ctx.profile(); nl += dpr["launches"]
     d_e2e_ms = (time.perf_counter() - t0) * 1e3 / K
+    if dump is not None:
+        dump[name + "_decompressed"] = dump_sample(h_out[:d_len].numpy(), 1 << 20)
     hbm, which = peaks()
     n_strip_r = nr - int((ref_np == ord("N")).sum()); n_strip_t = nt - int((tgt_np == ord("N")).sum())
     idx_bytes = 5 * n_strip_r + 4 * ((1 << 20) + 1)       # SURVEY 8d: R' read once + one 4-byte position per k-mer written + the bucket table

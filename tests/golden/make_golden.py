@@ -2,10 +2,10 @@
 """Regenerates tests/golden/reference_outputs.json by running the UNMODIFIED reference
 (compiled by oracle/Makefile into oracle/_ref/, 7z replaced by oracle/7z_shim.sh) on every case
 of tests/cases.py.  The reference ships no golden vectors of its own (SURVEY.md section 4), so
-these are the pin: outputs of the reference itself, produced in the build container where
-/root/reference exists.  Never edit the JSON by hand.
+these are the pin: outputs of the reference itself, produced from a checkout of its sources.
+Never edit the JSON by hand.
 
-    python tests/golden/make_golden.py
+    SCCG_REFERENCE_SRC=<checkout of the reference> python tests/golden/make_golden.py
 """
 from __future__ import annotations
 
@@ -18,7 +18,7 @@ import zlib
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
-sys.path.insert(0, str(HERE.parent))
+sys.path[:0] = [str(HERE.parent), str(HERE.parent.parent)]
 
 import oracle_lib as ol  # noqa: E402
 from cases import cases, fasta_cases  # noqa: E402
@@ -48,7 +48,7 @@ def run_files(ref_file: bytes, tgt_file: bytes) -> dict:
 
 
 def main() -> None:
-    assert ol.build_reference(), "reference not available: run in the build container"
+    assert ol.build_reference(), "reference not available: set SCCG_REFERENCE_SRC to a checkout of its sources"
     out = {"generator": "tests/golden/make_golden.py", "reference": "Jan-Celin/SCCG-genome-compression (unmodified, g++ -O3 -std=c++17)",
            "cases": {}, "fasta_cases": {}}
     for c in cases():

@@ -27,9 +27,10 @@ def build_oracle(force: bool = False) -> Path:
 
 
 def build_reference() -> bool:
-    """Compile the reference from /root/reference if it is present; True if oracle/_ref is usable."""
-    if Path("/root/reference/compression.cpp").exists():
-        subprocess.check_call(["make", "-C", str(ORACLE_DIR), "ref"], stdout=subprocess.DEVNULL)
+    """Compile the reference into oracle/_ref where its sources are readable (__graft_entry__.oracle_make says where they
+    are looked for); True if oracle/_ref is usable."""
+    import __graft_entry__ as g
+    subprocess.check_call(g.oracle_make("ref"), stdout=subprocess.DEVNULL)
     return have_reference()
 
 

@@ -1,6 +1,6 @@
 """INTEGRATION.md section 2, compiled and run: the reference's OWN programs (its main, argv handling, FASTA readers, 7z calls)
 with only compress_genome's middle and reconstruct_genome's body replaced by the C-ABI calls (integration/patch_reference.py).
-  * CPU: the patched sources are linked against the SIMT-emulator build of the library (needs /root/reference);
+  * CPU: the patched sources are linked against the SIMT-emulator build of the library (needs the reference's sources);
   * GPU (`-m gpu`): the binaries that build() leaves in oracle/_ref/patched, linked against libsccg_b200.so.
 Both run the FASTA-level goldens -- files produced by the unmodified reference -- through the patched executables."""
 import base64
@@ -11,11 +11,12 @@ from pathlib import Path
 
 import pytest
 
+import __graft_entry__ as g
 import oracle_lib as ol
 from cases import fasta_cases
 
 ROOT = Path(__file__).resolve().parent.parent
-HAVE_SRC = Path("/root/reference/compression.cpp").exists()
+REF_SRC = g.reference_sources()
 
 
 def unpack(s):
@@ -46,12 +47,11 @@ def run_goldens(bindir: Path, golden, tmp_path, extra_env=None):
     assert r.returncode == 1 and b"exceeds reference genome size" in r.stderr
 
 
-@pytest.mark.skipif(not (HAVE_SRC and ol.have_reference()), reason="needs the reference checkout (/root/reference) and oracle/_ref")
+@pytest.mark.skipif(not (REF_SRC and ol.have_reference()), reason="needs the reference's sources (not part of this repository; SCCG_REFERENCE_SRC) and oracle/_ref")
 def test_patched_reference_on_the_emulator(golden, tmp_path):
-    import __graft_entry__ as g
     from emu_lib import EMU_DIR, emu_context
     emu_context().close()
-    bindir = g.build_patched_reference(lib_dir=EMU_DIR, lib_name="sccg_b200_emu", out_dir=tmp_path / "patched_bin")
+    bindir = g.build_patched_reference(REF_SRC, lib_dir=EMU_DIR, lib_name="sccg_b200_emu", out_dir=tmp_path / "patched_bin")
     run_goldens(bindir, golden, tmp_path, {"SCCG_EMU_THREADS": "2"})
 
 
@@ -59,5 +59,5 @@ def test_patched_reference_on_the_emulator(golden, tmp_path):
 def test_patched_reference_on_the_gpu(golden, tmp_path):
     bindir = ROOT / "oracle" / "_ref" / "patched"
     if not (bindir / "compress").exists() or not ol.have_reference():
-        pytest.skip("oracle/_ref/patched not built (build() creates it where /root/reference exists)")
+        pytest.skip("oracle/_ref/patched not built (build() creates it where the reference's sources are readable)")
     run_goldens(bindir, golden, tmp_path)
