@@ -147,6 +147,31 @@ int sccg_compress_resident_into(sccg_ctx* ctx, const char* tgt, int64_t tgt_len,
                                 char* out, int64_t out_cap, int64_t* out_len, int* mode_out);
 int sccg_decompress_resident_into(sccg_ctx* ctx, const char* intermediate, int64_t inter_len, char* out, int64_t out_cap, int64_t* out_len);
 
+/* Region extraction: pieces of the decoded sequence without producing the whole image (what `samtools faidx` /
+ * `bedtools getfasta` do with a plain FASTA).  D is the decoded sequence of the intermediate file: the reconstructed_genome.fa
+ * image that sccg_decompress produces for the same inputs, without its first line ("<header>\n") and without any '\n' -- N runs
+ * re-inserted, lowercase restored.  *seq_len receives len(D).  A region {start, end} is 0-based and half-open in D,
+ * 0 <= start <= end <= len(D); empty regions are allowed, and regions may come in any order, overlap and repeat.  out receives
+ * D[start_0:end_0] + D[start_1:end_1] + ... in the order given, with no separators: region i begins at the sum of the lengths
+ * before it, and *out_len is the total.
+ * Errors, in this order:
+ *   SCCG_E_ARG before any device work: a NULL pointer with a non-zero count, start < 0 or start > end, a total of 2^31 bytes or
+ *     more or n_regions >= 2^31, out_cap smaller than the total (*out_len then holds the required size);
+ *   SCCG_E_FORMAT / SCCG_E_BOUNDS exactly when sccg_decompress fails on the same inputs, whatever the regions;
+ *   SCCG_E_ARG when a region ends past len(D) (*seq_len holds len(D), so the caller can clamp).
+ * Local-mode files upload and prepare only the reference chunks that the regions copy from; global-mode files need the whole
+ * reference (every N of it is removed first).  Profile: h2d_ms (host -> device copies), serialize_ms (front end), gather_ms
+ * (region gather), kernels_ms (all kernels), d2h_ms (device -> host copy of the result), launches. */
+typedef struct { int64_t start, end; } sccg_region;
+int sccg_extract(sccg_ctx* ctx, const char* ref_raw, int64_t ref_len, const char* intermediate, int64_t inter_len,
+                 const sccg_region* regions, int64_t n_regions, char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len);
+/* the same with the reference FASTA file image (as sccg_decompress_fasta takes it) */
+int sccg_extract_fasta(sccg_ctx* ctx, const char* ref_file, int64_t ref_file_len, const char* intermediate, int64_t inter_len,
+                       const sccg_region* regions, int64_t n_regions, char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len);
+/* the same against the resident reference (sccg_reference_set; SCCG_E_ARG without one) */
+int sccg_extract_resident(sccg_ctx* ctx, const char* intermediate, int64_t inter_len,
+                          const sccg_region* regions, int64_t n_regions, char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len);
+
 /* FASTA file images in: read_genomes_from_files (compression.cpp:181-220) and the reference reader of decompress_genome
  * (decompression.cpp:47-58) run on the device -- header lines skipped ('>' at a line start; in the target only the first one,
  * which becomes the header line of the output), isspace() bytes removed -- followed by sccg_compress / sccg_decompress.

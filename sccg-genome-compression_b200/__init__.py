@@ -133,6 +133,9 @@ def load_library(path: str | os.PathLike | None = None) -> C.CDLL:
     lib.sccg_decompress_fasta_into.argtypes = [vp, cp, i64, cp, i64, vp, i64, i64p]
     lib.sccg_decompress_stream.argtypes = [vp, cp, i64, cp, i64, SINK_FN, vp, i64p]
     lib.sccg_decompress_fasta_stream.argtypes = [vp, cp, i64, cp, i64, SINK_FN, vp, i64p]
+    lib.sccg_extract.argtypes = [vp, cp, i64, cp, i64, vp, i64, vp, i64, i64p, i64p]
+    lib.sccg_extract_fasta.argtypes = [vp, cp, i64, cp, i64, vp, i64, vp, i64, i64p, i64p]
+    lib.sccg_extract_resident.argtypes = [vp, cp, i64, vp, i64, vp, i64, i64p, i64p]
     lib.sccg_mgpu_unique_id.argtypes = [C.c_char_p]
     lib.sccg_mgpu_init.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.POINTER(vp)]
     lib.sccg_mgpu_destroy.argtypes = [vp]
@@ -470,6 +473,45 @@ class Context:
         self._check(fn(self.handle, _as_char_p(ref), len(ref), intermediate, len(intermediate), cb, None, C.byref(total)))
         assert sum(len(p) for _, p in pieces) == total.value
         return pieces
+
+    # region extraction (include/sccg.h): D[start_0:end_0] + D[start_1:end_1] + ... of the decoded sequence D
+    def _extract(self, call, regions, out_ptr: int, out_cap: int):
+        import numpy as np
+        reg = np.ascontiguousarray(np.asarray(regions, dtype=np.int64).reshape(-1, 2))     # sccg_region[] layout, no copy for int64 (n, 2)
+        n = C.c_int64(-1); seq = C.c_int64(-1)
+        rp = reg.ctypes.data if len(reg) else None
+
+        def run(ptr, cap):
+            rc = call(rp, len(reg), ptr, cap, C.byref(n), C.byref(seq))
+            if rc != SCCG_OK:
+                err = SccgError(rc, self.lib.sccg_last_error().decode())
+                err.out_len, err.seq_len = n.value, seq.value      # required size / length of D, where the library set them
+                raise err
+            self.last_seq_len = seq.value
+        if out_ptr:
+            run(out_ptr, out_cap)
+            return n.value
+        lens = reg[:, 1] - reg[:, 0]
+        cap = max(int(lens.sum()), 0) if len(reg) and bool((lens >= 0).all()) else 0
+        buf = C.create_string_buffer(max(cap, 1))
+        run(C.cast(buf, C.c_void_p), cap)
+        return buf.raw[:n.value]
+
+    def extract(self, ref_raw, intermediate: bytes, regions, out_ptr: int = 0, out_cap: int = 0):
+        """regions: an (n, 2) int64 numpy array or a sequence of (start, end) pairs, 0-based half-open in the decoded sequence ->
+        the concatenated pieces (bytes), or their total length when written into the caller's buffer (out_ptr / out_cap).
+        The length of the decoded sequence is left in self.last_seq_len (and in SccgError.seq_len for a region past its end)."""
+        return self._extract(lambda *t: self.lib.sccg_extract(self.handle, _as_char_p(ref_raw), len(ref_raw), intermediate, len(intermediate), *t),
+                             regions, out_ptr, out_cap)
+
+    def extract_fasta(self, ref_file, intermediate: bytes, regions, out_ptr: int = 0, out_cap: int = 0):
+        """extract with the reference FASTA file image"""
+        return self._extract(lambda *t: self.lib.sccg_extract_fasta(self.handle, _as_char_p(ref_file), len(ref_file), intermediate, len(intermediate), *t),
+                             regions, out_ptr, out_cap)
+
+    def extract_resident(self, intermediate: bytes, regions, out_ptr: int = 0, out_cap: int = 0):
+        """extract against the resident reference (set_reference)"""
+        return self._extract(lambda *t: self.lib.sccg_extract_resident(self.handle, intermediate, len(intermediate), *t), regions, out_ptr, out_cap)
 
     # decompress_genome (in-memory part) + reconstruct_genome + header line (decompression.cpp:66-110, :117-279, :322)
     def decompress(self, ref_raw: bytes, intermediate: bytes) -> bytes:

@@ -3,6 +3,7 @@
 #include "sccg_compress.cuh"
 #include "sccg_global.cuh"
 #include "sccg_decode.cuh"
+#include "sccg_extract.cuh"
 #include "sccg_fasta.cuh"
 #include "sccg_shard.cuh"
 #include "sccg_mgpu.cuh"
@@ -101,8 +102,7 @@ void sccg_destroy(sccg_ctx* c) {
         for (int i = 0; i < 64; ++i) { cudaEventDestroy(c->ev_h2d[i]); cudaEventDestroy(c->ev_g[i]); cudaEventDestroy(c->ev_d2h[i]); }
     }
     for (int i = 0; i < 2; ++i) if (c->h_stream[i]) cudaFreeHost(c->h_stream[i]);
-    {
-    }
+    if (c->h_ext) cudaFreeHost(c->h_ext);
     delete c;
 }
 
@@ -500,6 +500,43 @@ int sccg_decompress_stream(sccg_ctx* c, const char* ref_raw, int64_t ref_len, co
     prof_reset(c);
     SinkSpec sp{sink, user};
     return decompress_host(c, ref_raw, ref_len, inter, inter_len, nullptr, 0, nullptr, total_len, nullptr, nullptr, &sp);
+}
+
+// ---- region extraction (csrc/sccg_extract.cuh) ----------------------------------------------------------------------------
+int sccg_extract(sccg_ctx* c, const char* ref_raw, int64_t ref_len, const char* inter, int64_t inter_len, const sccg_region* regions, int64_t n_regions,
+                 char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len) {
+    if (!c || (ref_len > 0 && !ref_raw) || (inter_len > 0 && !inter)) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_TRY(check_sizes(ref_len, inter_len));
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    return extract_host(c, ref_raw, ref_len, nullptr, inter, inter_len, regions, n_regions, out, out_cap, out_len, seq_len);
+}
+
+int sccg_extract_fasta(sccg_ctx* c, const char* ref_file, int64_t ref_file_len, const char* inter, int64_t inter_len, const sccg_region* regions,
+                       int64_t n_regions, char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len) {
+    if (!c || (ref_file_len > 0 && !ref_file) || (inter_len > 0 && !inter)) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_TRY(check_sizes(ref_file_len, inter_len));
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    // the region list is checked before the reference FASTA goes to the device (argument errors come before any device work)
+    SCCG_TRY(extract_check_regions(regions, n_regions, out, out_cap, out_len, seq_len));
+    u8* d_rf = nullptr;
+    u32* sc = nullptr;
+    SCCG_TRY(buf(c, B_SCALARS, (size_t)S_COUNT, &sc));
+    SCCG_TRY(upload_file(c, B_FILE_R, ref_file, ref_file_len, &d_rf));
+    FastaSeq R;
+    SCCG_TRY(fasta_ingest(c, d_rf, ref_file_len, false, B_TGT, B_FA_TMP, B_FA_RNG, sc + S_G7, &R));      // decompression.cpp:47-58
+    return extract_host(c, nullptr, R.len, R.d_seq, inter, inter_len, regions, n_regions, out, out_cap, out_len, seq_len);
+}
+
+int sccg_extract_resident(sccg_ctx* c, const char* inter, int64_t inter_len, const sccg_region* regions, int64_t n_regions,
+                          char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len) {
+    if (!c || (inter_len > 0 && !inter)) return set_error(SCCG_E_ARG, "null argument");
+    if (!c->res_ref_set) return set_error(SCCG_E_ARG, "no resident reference (call sccg_reference_set first)");
+    SCCG_TRY(check_sizes(c->res_ref_len, inter_len));
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    return extract_host(c, nullptr, c->res_ref_len, c->res_ref, inter, inter_len, regions, n_regions, out, out_cap, out_len, seq_len);
 }
 
 void* sccg_pinned_alloc(int64_t bytes) {

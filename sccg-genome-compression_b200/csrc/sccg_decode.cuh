@@ -787,11 +787,15 @@ __global__ void __launch_bounds__(GATHER_CTA) dec_gather_k(GatherArgs a) {
 
 // reconstruct_genome.  header_reserve bytes are left free in front of the text (multiple of 16) so that the caller
 // can place "<header>\n" right before it.  *d_out points at the text itself.
-struct ReconPlan { GatherArgs a; u32* sc; int* tok_len; u32 ntok; unsigned ntiles; RunTable lows, ns; u32 soft; };
+struct ReconPlan {
+    GatherArgs a; u32* sc; int* tok_len; u32 ntok; unsigned ntiles; RunTable lows, ns; u32 soft;
+    i64 nr; const int* tok_delta; const u32* delta_excl;        // inputs of dec_resolve_k
+};
 
-// everything of reconstruct_genome that does not read the reference symbols: run lists, tokenizer, sizes, output buffer
-static int reconstruct_prepare(sccg_ctx* c, i64 nr, const u8* d_enc, i64 ne, const u8* d_n, i64 nn, const u8* d_low, i64 nl,
-                               i64 header_reserve, ReconPlan* plan) {
+// The front end of reconstruct_genome, shared by the whole-image decoder and region extraction: run lists, tokenizer, sizes,
+// the segment tables (plan->a without an output: a.out / a.tile_win stay NULL).  Reads no reference symbols.  On return the
+// main lane may still be producing delta_excl (tokens) and the side lane the lowercase-run table (event ev_side[3]).
+static int reconstruct_front(sccg_ctx* c, i64 nr, const u8* d_enc, i64 ne, const u8* d_n, i64 nn, const u8* d_low, i64 nl, ReconPlan* plan) {
     u32* sc = nullptr;
     SCCG_TRY(buf(c, B_SCALARS, (size_t)S_COUNT, &sc));
     SCCG_CK(cudaMemsetAsync(sc, 0, sizeof(u32) * S_COUNT, c->stream));
@@ -856,20 +860,42 @@ static int reconstruct_prepare(sccg_ctx* c, i64 nr, const u8* d_enc, i64 ne, con
     const i64 nchunks = (Lm + WRAP - 1) / WRAP;
     const i64 total = Lm > 0 ? Lm + nchunks : 1;
     if (total >= 0xffffffffLL) return set_error(SCCG_E_ARG, "decoded output would exceed 4 GiB");
-    u8* out = nullptr;
-    SCCG_TRY(buf(c, B_OUT, (size_t)(header_reserve + total + 32), &out));
     plan->lows = lows; plan->ns = ns; plan->soft = 0;
     GatherArgs& a = plan->a;
     a.ref = nullptr; a.enc = d_enc; a.seg_dst = seg_dst; a.seg_src = seg_src; a.tok_abs = tok_abs; a.nseg = (int)nseg;
     a.n_start = ns.start; a.n_len = ns.len; a.n_cum = ns.cum; a.n_k = (int)ns.K;
     a.l_start = lows.start; a.l_len = lows.len; a.l_k = (int)lows.K;
-    a.Ls = Ls; a.Lm = Lm; a.total = total; a.out = out + header_reserve; a.tile0 = 0; a.err = sc + D_ERR;
-    plan->sc = sc; plan->tok_len = tok_len; plan->ntok = ntok; plan->ntiles = div_up(total, GATHER_TILE);
-    // resolved segment sources and per-tile entry points: the gather itself starts from two table loads
-    i64* seg_ptr = nullptr; int4* tile_win = nullptr;
+    a.Ls = Ls; a.Lm = Lm; a.total = total; a.out = nullptr; a.tile0 = 0; a.err = sc + D_ERR; a.tile_win = nullptr;
+    plan->sc = sc; plan->tok_len = tok_len; plan->ntok = ntok; plan->ntiles = 0;
+    plan->nr = nr; plan->tok_delta = tok_delta; plan->delta_excl = delta_excl;
+    // resolved segment sources: the gathers start from two table loads
+    i64* seg_ptr = nullptr;
     SCCG_TRY(buf(c, B_SEG_PTR, (size_t)nseg + 1, &seg_ptr));
+    a.seg_ptr = seg_ptr;
+    return SCCG_OK;
+}
+
+// seg_ptr of every segment and the bounds check of every token (main lane)
+static int reconstruct_resolve(sccg_ctx* c, const ReconPlan* plan) {
+    const GatherArgs& a = plan->a;
+    if (a.nseg) LAUNCH(c, dec_resolve_k, dim3(div_up(a.nseg, 256)), dim3(256), 0, a.seg_src, plan->tok_delta, (const int*)plan->tok_len,
+                       plan->delta_excl, a.nseg, plan->nr, const_cast<int*>(a.tok_abs), const_cast<i64*>(a.seg_ptr), plan->sc);
+    return SCCG_OK;
+}
+
+// everything of reconstruct_genome that does not read the reference symbols: front end, output buffer, per-tile windows
+static int reconstruct_prepare(sccg_ctx* c, i64 nr, const u8* d_enc, i64 ne, const u8* d_n, i64 nn, const u8* d_low, i64 nl,
+                               i64 header_reserve, ReconPlan* plan) {
+    SCCG_TRY(reconstruct_front(c, nr, d_enc, ne, d_n, nn, d_low, nl, plan));
+    GatherArgs& a = plan->a;
+    u8* out = nullptr;
+    SCCG_TRY(buf(c, B_OUT, (size_t)(header_reserve + a.total + 32), &out));
+    a.out = out + header_reserve;
+    plan->ntiles = div_up(a.total, GATHER_TILE);
+    // per-tile entry points: the gather itself starts from two table loads
+    int4* tile_win = nullptr;
     SCCG_TRY(buf(c, B_TILE_WIN, (size_t)plan->ntiles + 1, &tile_win));
-    a.seg_ptr = seg_ptr; a.tile_win = tile_win;
+    a.tile_win = tile_win;
     {   // the window searches need the run tables (made on the side lane) and seg_dst: they run there, next to the token scan
         // and dec_resolve_k of the main lane
         SideLane side(c);
@@ -877,8 +903,7 @@ static int reconstruct_prepare(sccg_ctx* c, i64 nr, const u8* d_enc, i64 ne, con
         LAUNCH(c, dec_tile_win_k, dim3(div_up(plan->ntiles, 128)), dim3(128), 0, a, plan->ntiles, tile_win);
         SCCG_CK(cudaEventRecord(c->ev_side[5], c->stream));
     }
-    if (nseg) LAUNCH(c, dec_resolve_k, dim3(div_up(nseg, 256)), dim3(256), 0, (const i64*)seg_src, (const int*)tok_delta, (const int*)tok_len,
-                     (const u32*)delta_excl, (int)nseg, nr, tok_abs, seg_ptr, sc);
+    SCCG_TRY(reconstruct_resolve(c, plan));
     SCCG_CK(cudaStreamWaitEvent(c->stream, c->ev_side[5], 0));                  // run tables + windows complete (device-side wait)
     SCCG_CK(cudaEventRecord(c->ev[1], c->stream));                              // everything up to here is "tokenizer" time
     return SCCG_OK;
@@ -888,8 +913,8 @@ static int reconstruct_prepare(sccg_ctx* c, i64 nr, const u8* d_enc, i64 ne, con
 // decompression.cpp:138-164 / :176-207): runs out of order, lowercase runs that overlap.  Rare and off the hot path: the
 // (start, length) tables come to the host, are sorted -- lowercase: overlapping runs united (tolower is idempotent); N: an
 // overlap or a run past the end makes the reference's merge loop read out of range (:244-252) and stays an error -- and go
-// back; the per-tile windows are searched again.  Clears the soft flags.
-static int reconstruct_normalize(sccg_ctx* c, ReconPlan* plan) {
+// back.  Clears the soft flags.
+static int normalize_runs(sccg_ctx* c, ReconPlan* plan) {
     GatherArgs& a = plan->a;
     for (int which = 0; which < 2; ++which) {
         const u32 bit = which == 0 ? DE_LOW_UNSORTED : DE_N_UNSORTED;
@@ -925,6 +950,12 @@ static int reconstruct_normalize(sccg_ctx* c, ReconPlan* plan) {
     }
     plan->soft = 0;
     SCCG_CK(cudaMemsetAsync(plan->sc + D_ERR, 0, sizeof(u32), c->stream));
+    return SCCG_OK;
+}
+// the same for the whole-image decoder: the per-tile windows are searched again
+static int reconstruct_normalize(sccg_ctx* c, ReconPlan* plan) {
+    SCCG_TRY(normalize_runs(c, plan));
+    const GatherArgs& a = plan->a;
     LAUNCH(c, dec_tile_win_k, dim3(div_up(plan->ntiles, 128)), dim3(128), 0, a, plan->ntiles, const_cast<int4*>(a.tile_win));
     return SCCG_OK;
 }
@@ -1011,6 +1042,43 @@ __global__ void dec_need_k(GatherArgs a, const int* __restrict__ tok_len, i64 ch
 static const int PIPE_MAX_CHUNKS = 64;
 
 
+// the lines of an intermediate file (decompression.cpp:66-101): optional "<header>", lowercase runs, N runs, body
+struct InterLines { const char* header; i64 nh; const char* low; i64 nl; const char* nline; i64 nn; const char* body; i64 nb; bool local_mode; };
+static int split_intermediate(const char* inter, i64 inter_len, InterLines* L) {
+    i64 cur = 0;
+    auto next_line = [&](const char** b, i64* n) -> bool {
+        if (cur >= inter_len) return false;
+        const char* q = (const char*)memchr(inter + cur, '\n', (size_t)(inter_len - cur));
+        *b = inter + cur;
+        if (q) { *n = (q - inter) - cur; cur = (q - inter) + 1; } else { *n = inter_len - cur; cur = inter_len; }
+        return true;
+    };
+    const char* first = inter; i64 n0 = 0;
+    if (!next_line(&first, &n0)) return set_error(SCCG_E_FORMAT, "Greska pri citanju datoteke (empty intermediate file)");
+    L->nh = 0; L->header = inter;
+    if (n0 > 0 && first[0] == '>') {
+        L->header = first; L->nh = n0;
+        if (!next_line(&L->low, &L->nl)) return set_error(SCCG_E_FORMAT, "Greska pri citanju indeksa malih slova");
+    } else { L->low = first; L->nl = n0; }
+    if (!next_line(&L->nline, &L->nn)) return set_error(SCCG_E_FORMAT, "Greska pri citanju indeksa nepoznatih nukleotida");
+    if (!next_line(&L->body, &L->nb)) return set_error(SCCG_E_FORMAT, "Greska pri citanju kodiranog genoma");
+    L->local_mode = (L->nn == 1 && L->nline[0] == ',');                          // :105
+    return SCCG_OK;
+}
+// the three text lines -> device (a local-mode file's N line "," stays on the host: nothing is re-inserted)
+static int upload_lines(sccg_ctx* c, const InterLines& L, u8** d_enc, u8** d_n, u8** d_low) {
+    SCCG_TRY(upload(c, B_ENC, L.body, L.nb, d_enc));
+    SCCG_TRY(upload(c, B_NIDX, L.nline, L.local_mode ? 0 : L.nn, d_n));
+    SCCG_TRY(upload(c, B_LOW, L.low, L.nl, d_low));
+    return SCCG_OK;
+}
+// the decoder's error word after the front end -> error code (the soft flags are handled by the caller)
+static int decoder_flags_error(u32 flags) {
+    if (flags & DE_BOUNDS) return set_error(SCCG_E_BOUNDS, "ERROR: absolute_start + length exceeds reference genome size");
+    if (flags & DE_HARD) return set_error(SCCG_E_FORMAT, "malformed record stream or run list");
+    return SCCG_OK;
+}
+
 // decompress_genome's in-memory part (decompression.cpp:66-110) + reconstruct_genome + main's "<header>\n" (:322)
 // d_raw_in != NULL: the raw reference symbols are already in device memory (FASTA ingest on the device); ref_raw is unused then
 // part / n_parts (n_parts > 1): only the part-th of n_parts contiguous pieces of the file image is produced -- output-range
@@ -1036,33 +1104,15 @@ static int decompress_host_impl(sccg_ctx* c, const char* ref_raw, i64 ref_len, c
     const bool parts = ps && ps->n_parts > 1;
     if (sink && parts) return set_error(SCCG_E_ARG, "streaming and output-range sharding cannot be combined");
     // ---- the 3 / 4 getline calls (:66-101)
-    const char* lines[4] = {inter, inter, inter, inter};
-    i64 lens[4] = {0, 0, 0, 0};
-    i64 cur = 0;
-    auto next_line = [&](const char** b, i64* n) -> bool {
-        if (cur >= inter_len) return false;
-        const char* q = (const char*)memchr(inter + cur, '\n', (size_t)(inter_len - cur));
-        *b = inter + cur;
-        if (q) { *n = (q - inter) - cur; cur = (q - inter) + 1; } else { *n = inter_len - cur; cur = inter_len; }
-        return true;
-    };
-    if (!next_line(&lines[0], &lens[0])) return set_error(SCCG_E_FORMAT, "Greska pri citanju datoteke (empty intermediate file)");
-    i64 nh = 0; const char* header = inter;
-    const char *low, *nline, *body; i64 nl, nn, nb;
-    if (lens[0] > 0 && lines[0][0] == '>') {
-        header = lines[0]; nh = lens[0];
-        if (!next_line(&low, &nl)) return set_error(SCCG_E_FORMAT, "Greska pri citanju indeksa malih slova");
-    } else { low = lines[0]; nl = lens[0]; }
-    if (!next_line(&nline, &nn)) return set_error(SCCG_E_FORMAT, "Greska pri citanju indeksa nepoznatih nukleotida");
-    if (!next_line(&body, &nb)) return set_error(SCCG_E_FORMAT, "Greska pri citanju kodiranog genoma");
-    const bool local_mode = (nn == 1 && nline[0] == ',');                      // :105
+    InterLines L;
+    SCCG_TRY(split_intermediate(inter, inter_len, &L));
+    const char* header = L.header; const i64 nh = L.nh, nl = L.nl, nn = L.nn, nb = L.nb;
+    const bool local_mode = L.local_mode;
     // ---- uploads: the three text lines first (small), then the reference in chunks on its own copy stream
     SCCG_TRY(pipe_streams(c));
     u8 *d_raw = nullptr, *d_ref = nullptr, *d_enc = nullptr, *d_n = nullptr, *d_low = nullptr;
     SCCG_CK(cudaEventRecord(c->ev[4], c->stream));
-    SCCG_TRY(upload(c, B_ENC, body, nb, &d_enc));
-    SCCG_TRY(upload(c, B_NIDX, nline, local_mode ? 0 : nn, &d_n));
-    SCCG_TRY(upload(c, B_LOW, low, nl, &d_low));
+    SCCG_TRY(upload_lines(c, L, &d_enc, &d_n, &d_low));
     if (d_raw_in) d_raw = const_cast<u8*>(d_raw_in);
     else SCCG_TRY(buf(c, B_TGT, (size_t)ref_len + 128, &d_raw));
     SCCG_TRY(buf(c, B_REF, (size_t)ref_len + 128, &d_ref));
@@ -1148,8 +1198,7 @@ static int decompress_host_impl(sccg_ctx* c, const char* ref_raw, i64 ref_len, c
             SCCG_CK(cudaMemcpyAsync(h_need + 2 * PIPE_MAX_CHUNKS, sc + D_ERR, sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
             SCCG_CK(cudaStreamSynchronize(c->stream));
             const u32 flags = h_need[2 * PIPE_MAX_CHUNKS];
-            if (flags & DE_BOUNDS) return set_error(SCCG_E_BOUNDS, "ERROR: absolute_start + length exceeds reference genome size");
-            if (flags & DE_HARD) return set_error(SCCG_E_FORMAT, "malformed record stream or run list");
+            SCCG_TRY(decoder_flags_error(flags));
             if (!(flags & DE_SOFT)) break;
             plan.soft = flags & DE_SOFT;                                     // a run list out of order (legal for the reference's parser): sort it, ask again
             SCCG_TRY(reconstruct_normalize(c, &plan));

@@ -6,6 +6,10 @@
 // "<compressed_file> <reference_file> <output_folder>" -- over N GPUs with two workers per GPU (host/batch.hpp).
 // The reconstructed FASTA is STREAMED: the library hands it over piece by piece from a page-locked double buffer
 // (sccg_decompress_fasta_stream) and every piece is written to the output file while the next one crosses PCIe.
+//
+// Additive: `decompress --regions <regions.bed> <compressed_file> <reference_file> <output_folder>` writes only the BED regions
+// (name, 0-based start, exclusive end) to <output_folder>/regions.fa, one record per region labelled ">name:start-end" as
+// `bedtools getfasta` does, 50 columns per line; the whole image is never produced (sccg_extract_fasta).
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
@@ -67,14 +71,105 @@ static int decompress_one(Worker& w, const Job& job, Timing& tm, bool verbose) {
     return 0;
 }
 
+// BED lines: "name start end [more columns]", separated by tabs or spaces; blank lines and "#", "track", "browser" lines are
+// skipped.  false (with a message) on anything else.
+struct BedRegion { std::string name; int64_t start, end; };
+static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std::string* err) {
+    std::istringstream in(text);
+    std::string line;
+    for (int64_t no = 1; std::getline(in, line); ++no) {
+        if (!line.empty() && line.back() == '\r') line.pop_back();
+        std::vector<std::string> f;
+        for (size_t i = 0; i < line.size();) {
+            while (i < line.size() && (line[i] == ' ' || line[i] == '\t')) ++i;
+            size_t j = i;
+            while (j < line.size() && line[j] != ' ' && line[j] != '\t') ++j;
+            if (j > i) f.push_back(line.substr(i, j - i));
+            i = j;
+        }
+        if (f.empty() || f[0][0] == '#' || f[0] == "track" || f[0] == "browser") continue;
+        auto num = [](const std::string& t, int64_t* v) {
+            if (t.empty() || t.size() > 18 || t.find_first_not_of("0123456789") != std::string::npos) return false;
+            *v = std::stoll(t);
+            return true;
+        };
+        BedRegion r;
+        if (f.size() < 3 || !num(f[1], &r.start) || !num(f[2], &r.end) || r.start > r.end) {
+            *err = "malformed BED line " + std::to_string(no) + ": " + line;
+            return false;
+        }
+        r.name = f[0];
+        out->push_back(r);
+    }
+    return true;
+}
+
+static int extract_regions(const char* bed_path, const Job& job) {
+    std::ifstream bf(bed_path, std::ios::binary);
+    if (!bf) { std::cerr << "Error opening BED file: " << bed_path << "\n"; return 1; }
+    std::stringstream ss; ss << bf.rdbuf();
+    std::vector<BedRegion> bed;
+    std::string err;
+    if (!parse_bed(ss.str(), &bed, &err)) { std::cerr << "Error: " << err << "\n"; return 1; }
+    std::error_code ec;
+    if (!fs::exists(job.out)) fs::create_directory(job.out, ec);
+    const std::string cmd = "7z e \"" + job.a + "\" -o\"" + job.out + "\" -y > /dev/null";                        // as the 3-argument form
+    if (system(cmd.c_str()) != 0) { std::cerr << "Greska pri dekompresiji: " << job.a << "\n"; return 1; }
+    const std::string inter_path = job.out + "/" + fs::path(job.a).stem().string();
+    const char* dev = getenv("SCCG_DEVICE");
+    Worker w; w.device = dev ? atoi(dev) : 0;
+    w.ctx = sccg_create(w.device);
+    if (!w.ctx) { std::cerr << "Error: " << sccg_last_error() << "\n"; return 1; }
+    int64_t nf = 0, ni = 0;
+    int status = 1;
+    std::vector<sccg_region> regs(bed.size());
+    int64_t total = 0, out_len = 0, seq_len = -1;
+    for (size_t i = 0; i < bed.size(); ++i) { regs[i].start = bed[i].start; regs[i].end = bed[i].end; total += bed[i].end - bed[i].start; }
+    std::vector<char> seq((size_t)total + 1);
+    if (!sccg_host::read_file_pinned(job.b, w.in0, &nf)) std::cerr << "Greska pri otvaranju reference: " << job.b << "\n";
+    else if (!sccg_host::read_file_pinned(inter_path, w.in1, &ni)) std::cerr << "Greska pri otvaranju datoteke: " << inter_path << "\n";
+    else {
+        const int rc = sccg_extract_fasta(w.ctx, w.in0.p, nf, w.in1.p, ni, regs.data(), (int64_t)regs.size(), seq.data(), total, &out_len, &seq_len);
+        if (rc != SCCG_OK && seq_len >= 0 && rc == SCCG_E_ARG) std::cerr << "Error: a region ends past the end of the sequence (" << seq_len << " bp)\n";
+        else if (rc != SCCG_OK) std::cerr << (rc == SCCG_E_BOUNDS ? "" : "Error during reconstruction: ") << sccg_last_error() << "\n";
+        else status = 0;
+    }
+    sccg_destroy(w.ctx);
+    if (status) return status;
+    // ">name:start-end" and the sequence in lines of 50, written next to the target and renamed: no partial regions.fa
+    const std::string out_path = job.out + "/regions.fa", tmp_path = out_path + ".part";
+    std::string text;
+    text.reserve((size_t)total + (size_t)total / 50 + bed.size() * 32);
+    int64_t at = 0;
+    for (const BedRegion& r : bed) {
+        text += ">" + r.name + ":" + std::to_string(r.start) + "-" + std::to_string(r.end) + "\n";
+        for (int64_t p = r.start; p < r.end; p += 50) {
+            const int64_t n = r.end - p < 50 ? r.end - p : 50;
+            text.append(seq.data() + at, (size_t)n); text += '\n';
+            at += n;
+        }
+    }
+    const int fd = open(tmp_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    const bool ok = fd >= 0 && sccg_host::write_all(fd, text.data(), text.size());
+    if (fd >= 0) close(fd);
+    if (!ok || rename(tmp_path.c_str(), out_path.c_str()) != 0) { unlink(tmp_path.c_str()); std::cerr << "Error opening output file: " << job.out << "\n"; return 1; }
+    return 0;
+}
+
 int main(int argc, char* argv[]) {
     const bool batch = argc >= 3 && std::string(argv[1]) == "--batch";
-    if (argc != 4 && !batch) {                                              // decompression.cpp:283-286
+    const bool regions = argc == 6 && std::string(argv[1]) == "--regions";
+    if (argc != 4 && !batch && !regions) {                                  // decompression.cpp:283-286
         std::cerr << "Usage: " << argv[0] << " <compressed_file> <reference_file> <output_folder>\n"
-                  << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n";
+                  << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n"
+                  << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n";
         return 1;
     }
     try {
+        if (regions) {
+            Job job; job.a = argv[3]; job.b = argv[4]; job.out = argv[5];
+            return extract_regions(argv[2], job);
+        }
         if (!batch) {
             const double t0 = sccg_host::now_s();
             const char* dev = getenv("SCCG_DEVICE");
