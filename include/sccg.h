@@ -172,6 +172,38 @@ int sccg_extract_fasta(sccg_ctx* ctx, const char* ref_file, int64_t ref_file_len
 int sccg_extract_resident(sccg_ctx* ctx, const char* intermediate, int64_t inter_len,
                           const sccg_region* regions, int64_t n_regions, char* out, int64_t out_cap, int64_t* out_len, int64_t* seq_len);
 
+/* Archives: a record file opened once, then queried many times (what the index of `samtools faidx` does for a plain FASTA).
+ * sccg_archive_open runs the decoder's front end of one intermediate file against the RESIDENT reference (sccg_reference_set)
+ * and keeps the tables a gather reads (record bytes, segment tables, N runs, lowercase runs -- run lists out of order are
+ * normalised here, once) in device memory owned by the handle; no later call on the context touches them.  It fails with
+ * SCCG_E_FORMAT / SCCG_E_BOUNDS exactly when sccg_decompress_resident_into fails on the same file, and with SCCG_E_ARG without a
+ * resident reference.  The first open of a local-mode (global-mode) file after sccg_reference_set prepares the upper-cased
+ * (N-stripped and upper-cased) form of the resident reference, which then stays next to it.  Profile after an open:
+ * serialize_ms (front end), kernels_ms, h2d_ms (record file upload).
+ * sccg_archive_info: len(D) of the archive, its mode (0 local, 1 global) and the device memory it holds (any pointer may be NULL).
+ * sccg_archive_close releases one archive; sccg_destroy releases every archive still open on the context.
+ * An archive is bound to the resident reference it was opened against: after sccg_reference_set or sccg_reference_clear on
+ * its context, a query that names it fails with SCCG_E_ARG (open it again); it can still be closed. */
+typedef struct sccg_archive sccg_archive;
+int sccg_archive_open(sccg_ctx* ctx, const char* intermediate, int64_t inter_len, sccg_archive** out);
+int sccg_archive_info(const sccg_archive* a, int64_t* seq_len, int* mode, int64_t* device_bytes);
+int sccg_archive_close(sccg_ctx* ctx, sccg_archive* a);
+
+/* Pieces of any number of open archives in one call: query i is D_a[start:end] of archive archives[archive] (D as for
+ * sccg_extract) when strand is 0, and its reverse complement when strand is 1 (`bedtools getfasta -s`, `samtools faidx -i`).
+ * out receives the pieces in the order given, with no separators; *out_len is the total.  Complement, case kept: A<->T,
+ * C<->G, R<->Y, K<->M, B<->V, D<->H; every other byte (S, W, N, anything else) maps to itself.
+ * Errors, all SCCG_E_ARG and all before any device work, in this order: a NULL pointer with a non-zero count or a negative
+ * count (2^31 or more archives or queries); then for each query in turn: an archive index out of range, a NULL archive, an
+ * archive opened on another context, an archive whose resident reference has since been replaced or cleared, start < 0 or
+ * start > end, end past len(D) of that archive, a strand other than 0 or 1; then a total of 2^31 bytes or more, and out_cap
+ * smaller than the total (*out_len then holds the required size).
+ * One host -> device copy (the query table), one launch, one device -> host copy.  Profile: h2d_ms, gather_ms, kernels_ms,
+ * d2h_ms, launches. */
+typedef struct { int64_t archive, start, end, strand; } sccg_query;
+int sccg_archive_extract(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_query* queries, int64_t n_queries,
+                         char* out, int64_t out_cap, int64_t* out_len);
+
 /* FASTA file images in: read_genomes_from_files (compression.cpp:181-220) and the reference reader of decompress_genome
  * (decompression.cpp:47-58) run on the device -- header lines skipped ('>' at a line start; in the target only the first one,
  * which becomes the header line of the output), isspace() bytes removed -- followed by sccg_compress / sccg_decompress.

@@ -136,6 +136,10 @@ def load_library(path: str | os.PathLike | None = None) -> C.CDLL:
     lib.sccg_extract.argtypes = [vp, cp, i64, cp, i64, vp, i64, vp, i64, i64p, i64p]
     lib.sccg_extract_fasta.argtypes = [vp, cp, i64, cp, i64, vp, i64, vp, i64, i64p, i64p]
     lib.sccg_extract_resident.argtypes = [vp, cp, i64, vp, i64, vp, i64, i64p, i64p]
+    lib.sccg_archive_open.argtypes = [vp, cp, i64, C.POINTER(vp)]
+    lib.sccg_archive_info.argtypes = [vp, i64p, C.POINTER(C.c_int), i64p]
+    lib.sccg_archive_close.argtypes = [vp, vp]
+    lib.sccg_archive_extract.argtypes = [vp, vp, i64, vp, i64, vp, i64, i64p]
     lib.sccg_mgpu_unique_id.argtypes = [C.c_char_p]
     lib.sccg_mgpu_init.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.POINTER(vp)]
     lib.sccg_mgpu_destroy.argtypes = [vp]
@@ -258,17 +262,45 @@ class Mgpu:
         return off.value, n.value, total.value
 
 
+class Archive:
+    """An intermediate file opened on the device (sccg_archive_open, include/sccg.h): its decoder tables stay in device memory
+    until close(), and Context.query extracts pieces of it.  Usable as a context manager."""
+
+    def __init__(self, ctx: "Context", handle: int):
+        self.ctx, self.handle = ctx, handle
+        n = C.c_int64(); mode = C.c_int(); nbytes = C.c_int64()
+        ctx._check(ctx.lib.sccg_archive_info(handle, C.byref(n), C.byref(mode), C.byref(nbytes)))
+        self.seq_len, self.mode, self.device_bytes = n.value, mode.value, nbytes.value
+
+    def close(self):
+        if self.handle:
+            h, self.handle = self.handle, None
+            self.ctx._archives.discard(self)
+            if self.ctx.handle:
+                self.ctx._check(self.ctx.lib.sccg_archive_close(self.ctx.handle, h))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+
 class Context:
     """One sccg_ctx (one GPU).  Method names follow the reference's free functions."""
 
     def __init__(self, device: int = 0, lib_path: str | os.PathLike | None = None):
         self.lib = load_library(lib_path)
+        self._archives: set[Archive] = set()
         self.handle = self.lib.sccg_create(device)
         if not self.handle:
             raise SccgError(SCCG_E_CUDA, self.lib.sccg_last_error().decode())
 
     def close(self):
         if getattr(self, "handle", None):
+            for a in list(self._archives):          # sccg_destroy releases them
+                a.handle = None
+            self._archives.clear()
             self.lib.sccg_destroy(self.handle)
             self.handle = None
 
@@ -512,6 +544,40 @@ class Context:
     def extract_resident(self, intermediate: bytes, regions, out_ptr: int = 0, out_cap: int = 0):
         """extract against the resident reference (set_reference)"""
         return self._extract(lambda *t: self.lib.sccg_extract_resident(self.handle, intermediate, len(intermediate), *t), regions, out_ptr, out_cap)
+
+    # archives (include/sccg.h): record files decoded once, then queried with pieces of any of them in one call
+    def open_archive(self, intermediate: bytes) -> Archive:
+        """open an intermediate file against the resident reference (set_reference)"""
+        h = C.c_void_p()
+        self._check(self.lib.sccg_archive_open(self.handle, intermediate, len(intermediate), C.byref(h)))
+        a = Archive(self, h.value)
+        self._archives.add(a)
+        return a
+
+    def query(self, archives, queries, out_ptr: int = 0, out_cap: int = 0):
+        """archives: a sequence of Archive; queries: an (n, 4) int64 array (or a sequence of rows) of [archive index, start, end,
+        strand], strand 1 being the reverse complement -> the concatenated pieces (bytes), or their total length when written
+        into the caller's buffer (out_ptr / out_cap).  A too-small buffer raises SccgError with out_len = the required size."""
+        import numpy as np
+        q = np.ascontiguousarray(np.asarray(queries, dtype=np.int64).reshape(-1, 4))     # sccg_query[] layout
+        arr = (C.c_void_p * max(len(archives), 1))(*[a.handle for a in archives])
+        n = C.c_int64(-1)
+        qp = q.ctypes.data if len(q) else None
+
+        def run(ptr, cap):
+            rc = self.lib.sccg_archive_extract(self.handle, arr if len(archives) else None, len(archives), qp, len(q), ptr, cap, C.byref(n))
+            if rc != SCCG_OK:
+                err = SccgError(rc, self.lib.sccg_last_error().decode())
+                err.out_len = n.value
+                raise err
+        if out_ptr:
+            run(out_ptr, out_cap)
+            return n.value
+        lens = q[:, 2] - q[:, 1]
+        cap = max(int(lens.sum()), 0) if len(q) and bool((lens >= 0).all()) else 0
+        buf = C.create_string_buffer(max(cap, 1))
+        run(C.cast(buf, C.c_void_p), cap)
+        return buf.raw[:n.value]
 
     # decompress_genome (in-memory part) + reconstruct_genome + header line (decompression.cpp:66-110, :117-279, :322)
     def decompress(self, ref_raw: bytes, intermediate: bytes) -> bytes:

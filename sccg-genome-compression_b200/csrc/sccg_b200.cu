@@ -91,6 +91,8 @@ void sccg_destroy(sccg_ctx* c) {
     for (int i = 0; i < B_NSLOTS; ++i) if (c->bufs[i].p) cudaFree(c->bufs[i].p);
     if (c->h_pinned) cudaFreeHost(c->h_pinned);
     if (c->res_ref) cudaFree(c->res_ref);
+    while (c->archives) { sccg_archive* a = c->archives; archive_unlink(c, a); archive_free(a); }
+    for (int f = 0; f < 2; ++f) if (c->res_form[f]) cudaFree(c->res_form[f]);
     for (int i = 0; i < 8; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
     for (int i = 0; i < 4; ++i) if (c->ev_x[i]) cudaEventDestroy(c->ev_x[i]);
     if (c->main_stream) cudaStreamDestroy(c->main_stream);
@@ -186,6 +188,7 @@ int sccg_reference_set(sccg_ctx* c, const char* ref, int64_t ref_len) {
     if (!c || ref_len < 0 || (ref_len > 0 && !ref)) return set_error(SCCG_E_ARG, "null argument");
     SCCG_TRY(check_sizes(ref_len, 0));
     SCCG_CK(cudaSetDevice(c->device));
+    reference_changed(c);
     const size_t need = (size_t)ref_len + 128;
     if (need > c->res_ref_cap) {
         if (c->res_ref) { SCCG_CK(cudaStreamSynchronize(c->main_stream)); cudaFree(c->res_ref); c->res_ref = nullptr; c->res_ref_cap = 0; }
@@ -206,6 +209,7 @@ int sccg_reference_set(sccg_ctx* c, const char* ref, int64_t ref_len) {
 int sccg_reference_clear(sccg_ctx* c) {
     if (!c) return set_error(SCCG_E_ARG, "null argument");
     SCCG_CK(cudaSetDevice(c->device));
+    reference_changed(c);
     if (c->res_ref) { SCCG_CK(cudaStreamSynchronize(c->main_stream)); cudaFree(c->res_ref); }
     c->res_ref = nullptr; c->res_ref_cap = 0; c->res_ref_len = 0; c->res_ref_set = 0;
     return SCCG_OK;
@@ -537,6 +541,44 @@ int sccg_extract_resident(sccg_ctx* c, const char* inter, int64_t inter_len, con
     SCCG_CK(cudaSetDevice(c->device));
     prof_reset(c);
     return extract_host(c, nullptr, c->res_ref_len, c->res_ref, inter, inter_len, regions, n_regions, out, out_cap, out_len, seq_len);
+}
+
+// ---- archives: record files decoded once and kept open on the device (csrc/sccg_extract.cuh) --------------------------------
+int sccg_archive_open(sccg_ctx* c, const char* inter, int64_t inter_len, sccg_archive** out) {
+    if (!c || !out || (inter_len > 0 && !inter)) return set_error(SCCG_E_ARG, "null argument");
+    if (!c->res_ref_set) return set_error(SCCG_E_ARG, "no resident reference (call sccg_reference_set first)");
+    SCCG_TRY(check_sizes(c->res_ref_len, inter_len));
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    return archive_open(c, inter, inter_len, out);
+}
+
+int sccg_archive_info(const sccg_archive* a, int64_t* seq_len, int* mode, int64_t* device_bytes) {
+    if (!a) return set_error(SCCG_E_ARG, "null argument");
+    if (seq_len) *seq_len = a->g.Lm;
+    if (mode) *mode = a->mode;
+    if (device_bytes) *device_bytes = a->device_bytes;
+    return SCCG_OK;
+}
+
+int sccg_archive_close(sccg_ctx* c, sccg_archive* a) {
+    if (!c || !a) return set_error(SCCG_E_ARG, "null argument");
+    if (a->ctx != c) return set_error(SCCG_E_ARG, "the archive was opened on another context");
+    SCCG_CK(cudaSetDevice(c->device));
+    SCCG_CK(cudaStreamSynchronize(c->main_stream));
+    archive_unlink(c, a);
+    archive_free(a);
+    return SCCG_OK;
+}
+
+int sccg_archive_extract(sccg_ctx* c, sccg_archive* const* archives, int64_t n_archives, const sccg_query* queries, int64_t n_queries,
+                         char* out, int64_t out_cap, int64_t* out_len) {
+    if (!c) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    const int rc = archive_extract_impl(c, archives, n_archives, queries, n_queries, out, out_cap, out_len);
+    if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
+    return rc;
 }
 
 void* sccg_pinned_alloc(int64_t bytes) {

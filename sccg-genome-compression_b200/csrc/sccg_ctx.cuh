@@ -67,7 +67,11 @@ struct sccg_ctx {
     void* h_stream[2]; size_t h_stream_cap;      // page-locked double buffer of the streaming decompressor (sccg_decompress*_stream)
     int pipe_ready;
     sccg::ShardState shard;
-    void* h_ext; size_t h_ext_cap;   // page-locked staging of the region tables (sccg_extract*), grow-only
+    void* h_ext; size_t h_ext_cap;   // page-locked staging of the region tables (sccg_extract*, sccg_archive_extract), grow-only
+    unsigned res_gen;                // resident reference generation: sccg_reference_set / _clear advance it (archives opened before go stale)
+    unsigned char* res_form[2]; long long res_form_len[2];   // the resident reference as archives read it: [0] upper-cased (local-mode
+                                                              // files), [1] N-stripped and upper-cased (global mode); built at first need
+    sccg_archive* archives;          // open archives (sccg_destroy releases them)
 };
 
 namespace sccg {

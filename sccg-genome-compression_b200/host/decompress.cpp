@@ -10,11 +10,19 @@
 // Additive: `decompress --regions <regions.bed> <compressed_file> <reference_file> <output_folder>` writes only the BED regions
 // (name, 0-based start, exclusive end) to <output_folder>/regions.fa, one record per region labelled ">name:start-end" as
 // `bedtools getfasta` does, 50 columns per line; the whole image is never produced (sccg_extract_fasta).
+//
+// Additive: `decompress --regions <regions.bed> --archives <list> <reference_file> <output_folder>` extracts every BED region from
+// every archive of <list> (one .7z per line) in one call: the reference is read once and made resident, each archive is
+// unpacked as the 3-argument form does and opened on the device (sccg_archive_open), and sccg_archive_extract gathers all pieces.
+// <output_folder>/regions.fa holds, archive by archive in list order and region by region in BED order, records
+// ">archive_stem::name:start-end" (with "(-)" appended for the minus strand, `bedtools getfasta -s` style); BED column 6 ("+",
+// "-" or "."; absent means "+") sets the strand, and a minus-strand record holds the reverse complement.
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
 
 #include "batch.hpp"
+#include "fasta_io.hpp"
 #include "sccg.h"
 
 namespace fs = std::filesystem;
@@ -73,8 +81,9 @@ static int decompress_one(Worker& w, const Job& job, Timing& tm, bool verbose) {
 
 // BED lines: "name start end [more columns]", separated by tabs or spaces; blank lines and "#", "track", "browser" lines are
 // skipped.  false (with a message) on anything else.
-struct BedRegion { std::string name; int64_t start, end; };
-static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std::string* err) {
+// with_strand: column 6, when present, must be "+", "-" or "." (strand 1 for "-")
+struct BedRegion { std::string name; int64_t start, end; int strand = 0; };
+static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std::string* err, bool with_strand = false) {
     std::istringstream in(text);
     std::string line;
     for (int64_t no = 1; std::getline(in, line); ++no) {
@@ -98,9 +107,23 @@ static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std:
             *err = "malformed BED line " + std::to_string(no) + ": " + line;
             return false;
         }
+        if (with_strand && f.size() >= 6) {
+            if (f[5] != "+" && f[5] != "-" && f[5] != ".") { *err = "malformed BED line " + std::to_string(no) + " (strand): " + line; return false; }
+            r.strand = f[5] == "-";
+        }
         r.name = f[0];
         out->push_back(r);
     }
+    return true;
+}
+
+// the records of regions.fa: header line, then the piece in lines of 50; written next to the target and renamed (no partial file)
+static bool write_records(const std::string& out_dir, const std::string& text) {
+    const std::string out_path = out_dir + "/regions.fa", tmp_path = out_path + ".part";
+    const int fd = open(tmp_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    const bool ok = fd >= 0 && sccg_host::write_all(fd, text.data(), text.size());
+    if (fd >= 0) close(fd);
+    if (!ok || rename(tmp_path.c_str(), out_path.c_str()) != 0) { unlink(tmp_path.c_str()); return false; }
     return true;
 }
 
@@ -136,8 +159,7 @@ static int extract_regions(const char* bed_path, const Job& job) {
     }
     sccg_destroy(w.ctx);
     if (status) return status;
-    // ">name:start-end" and the sequence in lines of 50, written next to the target and renamed: no partial regions.fa
-    const std::string out_path = job.out + "/regions.fa", tmp_path = out_path + ".part";
+    // ">name:start-end" and the sequence in lines of 50
     std::string text;
     text.reserve((size_t)total + (size_t)total / 50 + bed.size() * 32);
     int64_t at = 0;
@@ -149,23 +171,98 @@ static int extract_regions(const char* bed_path, const Job& job) {
             at += n;
         }
     }
-    const int fd = open(tmp_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
-    const bool ok = fd >= 0 && sccg_host::write_all(fd, text.data(), text.size());
-    if (fd >= 0) close(fd);
-    if (!ok || rename(tmp_path.c_str(), out_path.c_str()) != 0) { unlink(tmp_path.c_str()); std::cerr << "Error opening output file: " << job.out << "\n"; return 1; }
+    if (!write_records(job.out, text)) { std::cerr << "Error opening output file: " << job.out << "\n"; return 1; }
+    return 0;
+}
+
+static int extract_archives(const char* bed_path, const char* list_path, const std::string& ref_path, const std::string& out_dir) {
+    std::string bed_text, list_text, ref_file;
+    std::vector<BedRegion> bed;
+    std::string err;
+    if (!sccg_host::read_file(bed_path, bed_text)) { std::cerr << "Error opening BED file: " << bed_path << "\n"; return 1; }
+    if (!parse_bed(bed_text, &bed, &err, true)) { std::cerr << "Error: " << err << "\n"; return 1; }
+    if (!sccg_host::read_file(list_path, list_text)) { std::cerr << "Error opening list file: " << list_path << "\n"; return 1; }
+    std::vector<std::string> arcs;
+    {
+        std::istringstream in(list_text);
+        std::string line;
+        while (std::getline(in, line)) {
+            const size_t a = line.find_first_not_of(" \t\r"), b = line.find_last_not_of(" \t\r");
+            if (a != std::string::npos) arcs.push_back(line.substr(a, b - a + 1));
+        }
+    }
+    if (arcs.empty()) { std::cerr << "Error: the archive list " << list_path << " names no archive\n"; return 1; }
+    if (!sccg_host::read_file(ref_path, ref_file)) { std::cerr << "Greska pri otvaranju reference: " << ref_path << "\n"; return 1; }
+    std::string ref;
+    sccg_host::parse_fasta(ref_file, false, ref, nullptr);                  // decompression.cpp:47-58
+    std::error_code ec;
+    if (!fs::exists(out_dir)) fs::create_directory(out_dir, ec);
+    const char* dev = getenv("SCCG_DEVICE");
+    sccg_ctx* ctx = sccg_create(dev ? atoi(dev) : 0);
+    if (!ctx) { std::cerr << "Error: " << sccg_last_error() << "\n"; return 1; }
+    int status = 1;
+    std::vector<sccg_archive*> open;
+    std::vector<sccg_query> qs;
+    std::string text;
+    [&] {
+        if (sccg_reference_set(ctx, ref.data(), (int64_t)ref.size()) != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
+        for (const std::string& arc : arcs) {                               // unpacked one at a time: archives may share a file name
+            const std::string cmd = "7z e \"" + arc + "\" -o\"" + out_dir + "\" -y > /dev/null";
+            if (system(cmd.c_str()) != 0) { std::cerr << "Greska pri dekompresiji: " << arc << "\n"; return; }
+            std::string inter;
+            const std::string inter_path = out_dir + "/" + fs::path(arc).stem().string();
+            if (!sccg_host::read_file(inter_path, inter)) { std::cerr << "Greska pri otvaranju datoteke: " << inter_path << "\n"; return; }
+            sccg_archive* a = nullptr;
+            const int rc = sccg_archive_open(ctx, inter.data(), (int64_t)inter.size(), &a);
+            if (rc != SCCG_OK) { std::cerr << arc << ": " << (rc == SCCG_E_BOUNDS ? "" : "Error during reconstruction: ") << sccg_last_error() << "\n"; return; }
+            open.push_back(a);
+            int64_t seq_len = 0;
+            sccg_archive_info(a, &seq_len, nullptr, nullptr);
+            for (const BedRegion& r : bed) {
+                if (r.end > seq_len) { std::cerr << "Error: region " << r.name << ":" << r.start << "-" << r.end << " ends past the end of " << arc << " (" << seq_len << " bp)\n"; return; }
+                qs.push_back(sccg_query{(int64_t)open.size() - 1, r.start, r.end, r.strand});
+            }
+        }
+        int64_t total = 0, out_len = 0;
+        for (const sccg_query& q : qs) total += q.end - q.start;
+        std::vector<char> seq((size_t)total + 1);
+        if (sccg_archive_extract(ctx, open.data(), (int64_t)open.size(), qs.data(), (int64_t)qs.size(), seq.data(), total, &out_len) != SCCG_OK) {
+            std::cerr << "Error: " << sccg_last_error() << "\n";
+            return;
+        }
+        text.reserve((size_t)total + (size_t)total / 50 + qs.size() * 48);
+        int64_t at = 0;
+        for (size_t i = 0; i < qs.size(); ++i) {
+            const BedRegion& r = bed[i % bed.size()];
+            text += ">" + fs::path(arcs[i / bed.size()]).stem().string() + "::" + r.name + ":" + std::to_string(r.start) + "-" + std::to_string(r.end) +
+                    (r.strand ? "(-)" : "") + "\n";
+            for (int64_t p = r.start; p < r.end; p += 50) {
+                const int64_t n = r.end - p < 50 ? r.end - p : 50;
+                text.append(seq.data() + at, (size_t)n); text += '\n';
+                at += n;
+            }
+        }
+        status = 0;
+    }();
+    sccg_destroy(ctx);                                                      // (releases the archives)
+    if (status) return status;
+    if (!write_records(out_dir, text)) { std::cerr << "Error opening output file: " << out_dir << "\n"; return 1; }
     return 0;
 }
 
 int main(int argc, char* argv[]) {
     const bool batch = argc >= 3 && std::string(argv[1]) == "--batch";
     const bool regions = argc == 6 && std::string(argv[1]) == "--regions";
-    if (argc != 4 && !batch && !regions) {                                  // decompression.cpp:283-286
+    const bool archives = argc == 7 && std::string(argv[1]) == "--regions" && std::string(argv[3]) == "--archives";
+    if (argc != 4 && !batch && !regions && !archives) {                     // decompression.cpp:283-286
         std::cerr << "Usage: " << argv[0] << " <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n"
-                  << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n";
+                  << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n"
+                  << "       " << argv[0] << " --regions <regions.bed> --archives <list of .7z files, one per line> <reference_file> <output_folder>\n";
         return 1;
     }
     try {
+        if (archives) return extract_archives(argv[2], argv[4], argv[5], argv[6]);
         if (regions) {
             Job job; job.a = argv[3]; job.b = argv[4]; job.out = argv[5];
             return extract_regions(argv[2], job);
