@@ -47,6 +47,25 @@ __device__ __forceinline__ u32 movemask8(u64 flags) { return (u32)(((flags >> 7)
 __device__ __forceinline__ u8 upper1(u8 c) { return (c >= 'a' && c <= 'z') ? (u8)(c - 32) : c; }
 __device__ __forceinline__ u8 lower1(u8 c) { return (c >= 'A' && c <= 'Z') ? (u8)(c + 32) : c; }
 
+// std::stoi(s[a..b)) as the reference calls it (compression.cpp:279, decompression.cpp:218-219): leading isspace skipped,
+// optional sign, >= 1 digit, stops at the first non-digit, value must fit in int.  Returns false where stoi throws.
+__device__ __forceinline__ bool dt_stoi(const u8* __restrict__ s, u32 a, u32 b, int* out) {
+    while (a < b && (s[a] == ' ' || (s[a] >= 9 && s[a] <= 13))) ++a;
+    bool neg = false;
+    if (a < b && (s[a] == '-' || s[a] == '+')) { neg = s[a] == '-'; ++a; }
+    if (a >= b || s[a] < '0' || s[a] > '9') return false;                     // invalid_argument
+    i64 v = 0;
+    while (a < b && s[a] >= '0' && s[a] <= '9') {
+        v = v * 10 + (s[a] - '0');
+        if (v > 2147483648LL) return false;                                    // out_of_range
+        ++a;
+    }
+    if (neg) v = -v;
+    if (v > 2147483647LL || v < -2147483648LL) return false;
+    *out = (int)v;
+    return true;
+}
+
 // number of characters operator<<(int) / std::to_string(int) prints
 __device__ __forceinline__ int dec_len_u32(u32 v) {
     int n = 1;

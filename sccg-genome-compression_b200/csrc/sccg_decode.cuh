@@ -9,9 +9,13 @@
 //                                   produces 16 bytes of the final text straight from the reference /
 //                                   the literal bytes (no intermediate "stripped" sequence in HBM)
 //
-// Input grammar: exactly what the compressor emits (N1 in SURVEY.md) plus the optional ',' after a
-// tuple that the reference parser tolerates.  Anything else returns SCCG_E_FORMAT where the reference
-// would throw from stoi (exit 1) or run into undefined behaviour (unsorted / overlapping run lists).
+// Input grammar.  Body tokens are read as the reference reads them: the token ends at the first ')', its two numbers go
+// through std::stoi (leading isspace, '+' or '-', any number of leading zeros, whatever follows the digits is ignored).
+// SCCG_E_FORMAT where that stoi throws, and for three pinned divergences (INTEGRATION.md section 5): a negative token
+// length, a token whose ')' lies more than TOK_MAX bytes after its '(', and a token without ',' before its ')'.  Run
+// lists: exactly what the compressor emits (N1 in SURVEY.md) plus the optional ',' after a tuple that the reference
+// tolerates; other run-list text is SCCG_E_FORMAT (pinned too).  Run lists that are out of order or overlap are put in
+// order first (reconstruct_normalize), as the reference's sort does.
 #pragma once
 #include "sccg_compress.cuh"
 #include "sccg_strip.cuh"
@@ -74,6 +78,26 @@ __device__ __forceinline__ int parse_tuple(const u8* __restrict__ s, i64 i, i64 
     w += k;
     if (i + w >= n || s[i + w] != ')') return 0;
     return w + 1;
+}
+
+// a body token at s[i] == '(' (decompression.cpp:215-219): the token ends at the first ')' (where dec_chunk ends it), the
+// delta is stoi from the byte after '(', the length is stoi from the byte after the first ',' inside the token.  Canonical
+// tokens, all the writers emit, pass parse_tuple; anything else takes the stoi parse.  false -> SCCG_E_FORMAT: stoi throws,
+// or one of two pinned classes.  A ')' more than TOK_MAX bytes after the '(' lies beyond the look-back that decides a
+// chunk's entry state (dec_chunk would have classified the token's tail as literals), and a token without ',' before
+// its ')' takes its length from the next ',' anywhere in the body in the reference (or from the body's first byte).
+// The run lists keep parse_tuple / parse_int alone.
+__device__ __forceinline__ bool parse_body_token(const u8* __restrict__ s, i64 i, i64 n, int* d, int* l) {
+    if (parse_tuple(s, i, n, d, l)) return true;
+    const u8* t = s + i;
+    const int m = n - i - 1 < TOK_MAX ? (int)(n - i - 1) : TOK_MAX;      // bytes after the '(' the token may use
+    int comma = 0, close = 0;
+    for (int k = 1; k <= m; ++k) {
+        if (t[k] == ')') { close = k; break; }
+        if (t[k] == ',' && !comma) comma = k;
+    }
+    if (!close || !comma) return false;
+    return dt_stoi(t, 1u, (u32)comma, d) && dt_stoi(t, (u32)comma + 1u, (u32)close, l);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -144,7 +168,7 @@ __global__ void __launch_bounds__(DEC_T) dec_count_k(const u8* __restrict__ enc,
     u32 sym = (u32)__popc(c.lit);
     for (u32 m = c.tok; m; m &= m - 1) {
         int d = 0, l = 0;
-        if (!parse_tuple(enc, i0 + __ffs((int)m) - 1, ne, &d, &l) || l < 0) atomicOr(&sc[D_ERR], (u32)DE_FORMAT);
+        if (!parse_body_token(enc, i0 + __ffs((int)m) - 1, ne, &d, &l) || l < 0) atomicOr(&sc[D_ERR], (u32)DE_FORMAT);
         else sym += (u32)l;
     }
     th_sym[t] = sym; th_seg[t] = (u32)__popc(c.tok | c.segl); th_tok[t] = (u32)__popc(c.tok);
@@ -167,7 +191,7 @@ __global__ void __launch_bounds__(DEC_T) dec_emit_k(const u8* __restrict__ enc, 
         seg_dst[nseg] = at;
         if ((c.tok >> b) & 1u) {
             int d = 0, l = 0;
-            parse_tuple(enc, i0 + b, ne, &d, &l);                      // validated by dec_count_k
+            parse_body_token(enc, i0 + b, ne, &d, &l);                 // validated by dec_count_k
             seg_src[nseg] = (i64)ntok; tok_delta[ntok] = d; tok_len[ntok] = l;
             tok_syms += (u32)l; ++ntok;
         } else {

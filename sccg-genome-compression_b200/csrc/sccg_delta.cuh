@@ -66,25 +66,6 @@ __device__ __forceinline__ void warp_copy_bytes(u8* __restrict__ dst, const u8* 
     if (done + (u32)lane < len) dst[done + lane] = src[done + lane];   // < 8 tail bytes
 }
 
-// std::stoi(s[a..b)) as the reference calls it (:279): leading isspace skipped, optional sign, >= 1 digit, stops at the
-// first non-digit, value must fit in int.  Returns false where stoi throws.  Uniform (every lane runs it).
-__device__ __forceinline__ bool dt_stoi(const u8* __restrict__ s, u32 a, u32 b, int* out) {
-    while (a < b && (s[a] == ' ' || (s[a] >= 9 && s[a] <= 13))) ++a;
-    bool neg = false;
-    if (a < b && (s[a] == '-' || s[a] == '+')) { neg = s[a] == '-'; ++a; }
-    if (a >= b || s[a] < '0' || s[a] > '9') return false;                     // invalid_argument
-    i64 v = 0;
-    while (a < b && s[a] >= '0' && s[a] <= '9') {
-        v = v * 10 + (s[a] - '0');
-        if (v > 2147483648LL) return false;                                    // out_of_range
-        ++a;
-    }
-    if (neg) v = -v;
-    if (v > 2147483647LL || v < -2147483648LL) return false;
-    *out = (int)v;
-    return true;
-}
-
 // in[start..end) -> out (written from out[0]); res[DT_LEN] = bytes written, res[DT_ERR] != 0 iff stoi would have thrown
 // (then the reference leaves the file un-rewritten and exits 1).  `in` is the 8-byte aligned file image, offsets are
 // absolute.  One warp.
