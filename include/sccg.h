@@ -204,6 +204,33 @@ typedef struct { int64_t archive, start, end, strand; } sccg_query;
 int sccg_archive_extract(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_query* queries, int64_t n_queries,
                          char* out, int64_t out_cap, int64_t* out_len);
 
+/* Pattern search in windows of open archives: window w is D_a[start:end] of archives[archive] (D as for sccg_archive_extract:
+ * N runs re-inserted, lowercase restored).  Pattern i is patterns[pattern_off[i] .. pattern_off[i+1]); 1 to 1024 patterns of
+ * 1 to 64 bytes.  strands: 1 forward, 2 reverse complement, 3 both.
+ * Match rule, per byte, after ASCII upper-casing both sides: pattern byte p matches D byte d when up(d) == up(p), or when p is
+ * an IUPAC code (R Y S W K M B D H V N) and up(d) is one of A/C/G/T in its set.  So N in a pattern matches any base and N, an
+ * N gap in D matches only pattern N, and any other byte matches only itself.
+ * A hit (window w, pos, pattern i, strand s, mismatches k): D[pos, pos + len_i) lies inside window w and differs in exactly
+ * k <= max_mismatches positions from pattern i (s = 0) or from its reverse complement (s = 1; the complement of
+ * sccg_archive_extract, which maps the IUPAC codes).  pos is an absolute D coordinate, the leftmost base on either strand (BED).
+ * Every hit is reported (overlapping occurrences, both strands of a palindrome, an occurrence once per window that holds it),
+ * in (window, pos, pattern, strand) order.  Windows shorter than a pattern give no hits for it.
+ * *n_hits always receives the total.  hits == NULL counts only.  When hits is given and the total exceeds hits_cap, the call
+ * returns SCCG_E_ARG with the required count in *n_hits (hits then holds an unspecified prefix).
+ * Errors, all SCCG_E_ARG and all before any device work, in this order: a NULL pointer with a non-zero count or a negative
+ * count (2^31 or more archives, windows or patterns); a pattern count outside 1..1024, pattern_off not non-decreasing from 0
+ * or a pattern length outside 1..64, max_mismatches < 0 or >= the shortest pattern's length, strands not in 1..3; then the
+ * query checks of sccg_archive_extract over the windows (archive index out of range, NULL archive, another context, a
+ * replaced or cleared resident reference, start < 0 or start > end, end past len(D)).
+ * Windows may add up to any size: the call splits them into launches (SCCG_SEARCH_SPLIT: candidate positions per launch) and
+ * copies the hits out after each.  Cost grows linearly with the number of patterns.  Profile: h2d_ms (window and pattern
+ * tables), gather_ms (search kernels), kernels_ms, d2h_ms (hits), launches. */
+typedef struct { int64_t archive, start, end; } sccg_window;
+typedef struct { int64_t window, pos; int32_t pattern, strand, mismatches, reserved; } sccg_hit;
+int sccg_archive_search(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
+                        const char* patterns, const int64_t* pattern_off, int64_t n_patterns, int max_mismatches, int strands,
+                        sccg_hit* hits, int64_t hits_cap, int64_t* n_hits);
+
 /* FASTA file images in: read_genomes_from_files (compression.cpp:181-220) and the reference reader of decompress_genome
  * (decompression.cpp:47-58) run on the device -- header lines skipped ('>' at a line start; in the target only the first one,
  * which becomes the header line of the output), isspace() bytes removed -- followed by sccg_compress / sccg_decompress.

@@ -4,6 +4,7 @@
 #include "sccg_global.cuh"
 #include "sccg_decode.cuh"
 #include "sccg_extract.cuh"
+#include "sccg_search.cuh"
 #include "sccg_fasta.cuh"
 #include "sccg_shard.cuh"
 #include "sccg_mgpu.cuh"
@@ -577,6 +578,18 @@ int sccg_archive_extract(sccg_ctx* c, sccg_archive* const* archives, int64_t n_a
     SCCG_CK(cudaSetDevice(c->device));
     prof_reset(c);
     const int rc = archive_extract_impl(c, archives, n_archives, queries, n_queries, out, out_cap, out_len);
+    if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
+    return rc;
+}
+
+int sccg_archive_search(sccg_ctx* c, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
+                        const char* patterns, const int64_t* pattern_off, int64_t n_patterns, int max_mismatches, int strands,
+                        sccg_hit* hits, int64_t hits_cap, int64_t* n_hits) {
+    if (!c) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    const int rc = archive_search_impl(c, archives, n_archives, windows, n_windows, patterns, pattern_off, n_patterns, max_mismatches,
+                                       strands, hits, hits_cap, n_hits);
     if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
     return rc;
 }

@@ -32,7 +32,7 @@ enum Slot {
     B_ENC, B_NIDX, B_LOW, B_TOK_FLAG, B_TOK_POS, B_ITEM_OFF, B_ITEM_SRC, B_NUM0, B_NUM1, B_NUM2, B_NUM3, B_NUM4, B_NUM5,
     B_LRUN_S, B_LRUN_E, B_NRUNS_S, B_NRUNS_E, B_NRUNS_CUM, B_TILE0, B_TILE1, B_TILE2, B_TILE3, B_SEG_PTR, B_TILE_WIN, B_FILE_R, B_FILE_T, B_FA_TMP, B_FA_RNG, B_NEED,
     B_GREF, B_GTGT, B_GKEYS, B_GVALS, B_GKEYS2, B_GVALS2, B_GHIST, B_GOFFS, B_GBUCKET, B_GREC, B_GLIT, B_GTMP0, B_GTMP1, B_GTMP2, B_GTMP3, B_GFIRST, B_SHARD,
-    B_EXT_REG, B_EXT_IV,
+    B_EXT_REG, B_EXT_IV, B_SRCH_TAB, B_SRCH_REG, B_SRCH_TILE, B_SRCH_HITS,
     B_NSLOTS
 };
 
@@ -67,7 +67,7 @@ struct sccg_ctx {
     void* h_stream[2]; size_t h_stream_cap;      // page-locked double buffer of the streaming decompressor (sccg_decompress*_stream)
     int pipe_ready;
     sccg::ShardState shard;
-    void* h_ext; size_t h_ext_cap;   // page-locked staging of the region tables (sccg_extract*, sccg_archive_extract), grow-only
+    void* h_ext; size_t h_ext_cap;   // page-locked staging of the region tables (sccg_extract*, sccg_archive_extract, sccg_archive_search), grow-only
     unsigned res_gen;                // resident reference generation: sccg_reference_set / _clear advance it (archives opened before go stale)
     unsigned char* res_form[2]; long long res_form_len[2];   // the resident reference as archives read it: [0] upper-cased (local-mode
                                                               // files), [1] N-stripped and upper-cased (global mode); built at first need

@@ -639,6 +639,20 @@ static void archive_unlink(sccg_ctx* c, sccg_archive* a) {
     if (a->next) a->next->prev = a->prev;
 }
 
+// the checks of one query (sccg_archive_extract) or window (sccg_archive_search) in the order of include/sccg.h: the index of
+// the first that fails, ARCHIVE_QUERY_OK when none does
+static const char* const archive_query_why[] = {"a query names an archive index out of range", "null argument",
+                                                "a query names an archive opened on another context",
+                                                "a query names an archive opened against a resident reference that has since been replaced or cleared",
+                                                "a query must have 0 <= start <= end", "a query ends past the end of its archive's decoded sequence",
+                                                "a query's strand must be 0 or 1"};
+static const int ARCHIVE_QUERY_OK = 6;
+static int archive_query_fault(const sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, i64 archive, i64 start, i64 end) {
+    const sccg_archive* a = archive >= 0 && archive < n_archives ? archives[archive] : nullptr;
+    return (archive < 0 || archive >= n_archives) ? 0 : !a ? 1 : a->ctx != c ? 2 : a->gen != c->res_gen ? 3
+         : (start < 0 || start > end) ? 4 : end > a->g.Lm ? 5 : ARCHIVE_QUERY_OK;
+}
+
 // sccg_archive_extract: argument checks (include/sccg.h, in that order), then one copy of the query table, one gather, one copy back
 static int archive_extract_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, const sccg_query* queries, i64 n_queries,
                                 char* out, i64 out_cap, int64_t* out_len) {
@@ -646,22 +660,16 @@ static int archive_extract_impl(sccg_ctx* c, sccg_archive* const* archives, i64 
         return set_error(SCCG_E_ARG, "null argument");
     if (n_archives >= 0x80000000LL || n_queries >= 0x80000000LL) return set_error(SCCG_E_ARG, "at most 2^31 - 1 archives and queries per call");
     // one pass; the error reported is the first of the list in include/sccg.h that any query commits
-    static const char* const why[] = {"a query names an archive index out of range", "null argument",
-                                      "a query names an archive opened on another context",
-                                      "a query names an archive opened against a resident reference that has since been replaced or cleared",
-                                      "a query must have 0 <= start <= end", "a query ends past the end of its archive's decoded sequence",
-                                      "a query's strand must be 0 or 1"};
     int first = 7;
     i64 total = 0;
     for (i64 i = 0; i < n_queries && first > 0; ++i) {
         const sccg_query& q = queries[i];
-        const sccg_archive* a = q.archive >= 0 && q.archive < n_archives ? archives[q.archive] : nullptr;
-        const int bad = (q.archive < 0 || q.archive >= n_archives) ? 0 : !a ? 1 : a->ctx != c ? 2 : a->gen != c->res_gen ? 3
-                      : (q.start < 0 || q.start > q.end) ? 4 : q.end > a->g.Lm ? 5 : (q.strand != 0 && q.strand != 1) ? 6 : 7;
+        const int f = archive_query_fault(c, archives, n_archives, q.archive, q.start, q.end);
+        const int bad = f < ARCHIVE_QUERY_OK ? f : (q.strand != 0 && q.strand != 1) ? 6 : 7;
         if (bad < first) first = bad;
         if (bad == 7) total += q.end - q.start;                              // (< 2^31 each, < 2^31 queries: no overflow)
     }
-    if (first < 7) return set_error(SCCG_E_ARG, why[first]);
+    if (first < 7) return set_error(SCCG_E_ARG, archive_query_why[first]);
     if (total >= 0x80000000LL) return set_error(SCCG_E_ARG, "the queries add up to 2^31 bytes or more");
     *out_len = total;
     if (total > 0 && !out) return set_error(SCCG_E_ARG, "null argument");

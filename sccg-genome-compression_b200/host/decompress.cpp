@@ -17,6 +17,13 @@
 // <output_folder>/regions.fa holds, archive by archive in list order and region by region in BED order, records
 // ">archive_stem::name:start-end" (with "(-)" appended for the minus strand, `bedtools getfasta -s` style); BED column 6 ("+",
 // "-" or "."; absent means "+") sets the strand, and a minus-strand record holds the reverse complement.
+//
+// Additive: `decompress --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K] [--strand both|+|-]
+// <reference_file> <output_folder>` finds every occurrence of the FASTA patterns (name: the header up to the first whitespace;
+// 1 to 64 bytes each) with at most K mismatches (default 0) in every BED region of every archive, or in each archive's whole
+// sequence without --regions (sccg_archive_search; archives unpacked and opened as above).  <output_folder>/hits.bed holds one
+// line per hit, "archive_stem<TAB>start<TAB>end<TAB>pattern_name<TAB>mismatches<TAB>+|-", archive by archive in list order and
+// in the library's (window, position, pattern, strand) order.
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
@@ -118,14 +125,8 @@ static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std:
 }
 
 // the records of regions.fa: header line, then the piece in lines of 50; written next to the target and renamed (no partial file)
-static bool write_records(const std::string& out_dir, const std::string& text) {
-    const std::string out_path = out_dir + "/regions.fa", tmp_path = out_path + ".part";
-    const int fd = open(tmp_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
-    const bool ok = fd >= 0 && sccg_host::write_all(fd, text.data(), text.size());
-    if (fd >= 0) close(fd);
-    if (!ok || rename(tmp_path.c_str(), out_path.c_str()) != 0) { unlink(tmp_path.c_str()); return false; }
-    return true;
-}
+static bool write_output(const std::string& out_path, const std::string& text);
+static bool write_records(const std::string& out_dir, const std::string& text) { return write_output(out_dir + "/regions.fa", text); }
 
 static int extract_regions(const char* bed_path, const Job& job) {
     std::ifstream bf(bed_path, std::ios::binary);
@@ -175,46 +176,75 @@ static int extract_regions(const char* bed_path, const Job& job) {
     return 0;
 }
 
+// the archive list: one path per line, blank lines skipped; false (with a message) when it cannot be read or names none
+static bool read_archive_list(const char* list_path, std::vector<std::string>* arcs) {
+    std::string list_text;
+    if (!sccg_host::read_file(list_path, list_text)) { std::cerr << "Error opening list file: " << list_path << "\n"; return false; }
+    std::istringstream in(list_text);
+    std::string line;
+    while (std::getline(in, line)) {
+        const size_t a = line.find_first_not_of(" \t\r"), b = line.find_last_not_of(" \t\r");
+        if (a != std::string::npos) arcs->push_back(line.substr(a, b - a + 1));
+    }
+    if (arcs->empty()) { std::cerr << "Error: the archive list " << list_path << " names no archive\n"; return false; }
+    return true;
+}
+
+// the reference FASTA read once and made resident on a new context; NULL (with a message) on failure
+static sccg_ctx* resident_context(const std::string& ref_path) {
+    std::string ref_file, ref;
+    if (!sccg_host::read_file(ref_path, ref_file)) { std::cerr << "Greska pri otvaranju reference: " << ref_path << "\n"; return nullptr; }
+    sccg_host::parse_fasta(ref_file, false, ref, nullptr);                  // decompression.cpp:47-58
+    const char* dev = getenv("SCCG_DEVICE");
+    sccg_ctx* ctx = sccg_create(dev ? atoi(dev) : 0);
+    if (!ctx) { std::cerr << "Error: " << sccg_last_error() << "\n"; return nullptr; }
+    if (sccg_reference_set(ctx, ref.data(), (int64_t)ref.size()) != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; sccg_destroy(ctx); return nullptr; }
+    return ctx;
+}
+
+// one archive unpacked as the 3-argument form does and opened on the device; NULL (with a message) on failure
+static sccg_archive* open_archive_file(sccg_ctx* ctx, const std::string& arc, const std::string& out_dir) {
+    const std::string cmd = "7z e \"" + arc + "\" -o\"" + out_dir + "\" -y > /dev/null";
+    if (system(cmd.c_str()) != 0) { std::cerr << "Greska pri dekompresiji: " << arc << "\n"; return nullptr; }
+    std::string inter;
+    const std::string inter_path = out_dir + "/" + fs::path(arc).stem().string();
+    if (!sccg_host::read_file(inter_path, inter)) { std::cerr << "Greska pri otvaranju datoteke: " << inter_path << "\n"; return nullptr; }
+    sccg_archive* a = nullptr;
+    const int rc = sccg_archive_open(ctx, inter.data(), (int64_t)inter.size(), &a);
+    if (rc != SCCG_OK) { std::cerr << arc << ": " << (rc == SCCG_E_BOUNDS ? "" : "Error during reconstruction: ") << sccg_last_error() << "\n"; return nullptr; }
+    return a;
+}
+
+// an output file written next to its target and renamed (no partial file)
+static bool write_output(const std::string& out_path, const std::string& text) {
+    const std::string tmp_path = out_path + ".part";
+    const int fd = open(tmp_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    const bool ok = fd >= 0 && sccg_host::write_all(fd, text.data(), text.size());
+    if (fd >= 0) close(fd);
+    if (!ok || rename(tmp_path.c_str(), out_path.c_str()) != 0) { unlink(tmp_path.c_str()); return false; }
+    return true;
+}
+
 static int extract_archives(const char* bed_path, const char* list_path, const std::string& ref_path, const std::string& out_dir) {
-    std::string bed_text, list_text, ref_file;
+    std::string bed_text;
     std::vector<BedRegion> bed;
     std::string err;
     if (!sccg_host::read_file(bed_path, bed_text)) { std::cerr << "Error opening BED file: " << bed_path << "\n"; return 1; }
     if (!parse_bed(bed_text, &bed, &err, true)) { std::cerr << "Error: " << err << "\n"; return 1; }
-    if (!sccg_host::read_file(list_path, list_text)) { std::cerr << "Error opening list file: " << list_path << "\n"; return 1; }
     std::vector<std::string> arcs;
-    {
-        std::istringstream in(list_text);
-        std::string line;
-        while (std::getline(in, line)) {
-            const size_t a = line.find_first_not_of(" \t\r"), b = line.find_last_not_of(" \t\r");
-            if (a != std::string::npos) arcs.push_back(line.substr(a, b - a + 1));
-        }
-    }
-    if (arcs.empty()) { std::cerr << "Error: the archive list " << list_path << " names no archive\n"; return 1; }
-    if (!sccg_host::read_file(ref_path, ref_file)) { std::cerr << "Greska pri otvaranju reference: " << ref_path << "\n"; return 1; }
-    std::string ref;
-    sccg_host::parse_fasta(ref_file, false, ref, nullptr);                  // decompression.cpp:47-58
+    if (!read_archive_list(list_path, &arcs)) return 1;
+    sccg_ctx* ctx = resident_context(ref_path);
+    if (!ctx) return 1;
     std::error_code ec;
     if (!fs::exists(out_dir)) fs::create_directory(out_dir, ec);
-    const char* dev = getenv("SCCG_DEVICE");
-    sccg_ctx* ctx = sccg_create(dev ? atoi(dev) : 0);
-    if (!ctx) { std::cerr << "Error: " << sccg_last_error() << "\n"; return 1; }
     int status = 1;
     std::vector<sccg_archive*> open;
     std::vector<sccg_query> qs;
     std::string text;
     [&] {
-        if (sccg_reference_set(ctx, ref.data(), (int64_t)ref.size()) != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
         for (const std::string& arc : arcs) {                               // unpacked one at a time: archives may share a file name
-            const std::string cmd = "7z e \"" + arc + "\" -o\"" + out_dir + "\" -y > /dev/null";
-            if (system(cmd.c_str()) != 0) { std::cerr << "Greska pri dekompresiji: " << arc << "\n"; return; }
-            std::string inter;
-            const std::string inter_path = out_dir + "/" + fs::path(arc).stem().string();
-            if (!sccg_host::read_file(inter_path, inter)) { std::cerr << "Greska pri otvaranju datoteke: " << inter_path << "\n"; return; }
-            sccg_archive* a = nullptr;
-            const int rc = sccg_archive_open(ctx, inter.data(), (int64_t)inter.size(), &a);
-            if (rc != SCCG_OK) { std::cerr << arc << ": " << (rc == SCCG_E_BOUNDS ? "" : "Error during reconstruction: ") << sccg_last_error() << "\n"; return; }
+            sccg_archive* a = open_archive_file(ctx, arc, out_dir);
+            if (!a) return;
             open.push_back(a);
             int64_t seq_len = 0;
             sccg_archive_info(a, &seq_len, nullptr, nullptr);
@@ -250,19 +280,130 @@ static int extract_archives(const char* bed_path, const char* list_path, const s
     return 0;
 }
 
+// FASTA patterns: the name is the header up to the first whitespace, the sequence lines are joined (line-end whitespace
+// dropped); false (with a message) for text before the first header, a record without sequence, or none at all
+struct Pattern { std::string name, seq; };
+static bool parse_patterns(const std::string& text, std::vector<Pattern>* out, std::string* err) {
+    std::istringstream in(text);
+    std::string line;
+    for (int64_t no = 1; std::getline(in, line); ++no) {
+        while (!line.empty() && isspace((unsigned char)line.back())) line.pop_back();
+        if (!line.empty() && line[0] == '>') {
+            if (!out->empty() && out->back().seq.empty()) { *err = "pattern " + out->back().name + " has no sequence"; return false; }
+            const size_t e = line.find_first_of(" \t", 1);
+            out->push_back(Pattern{line.substr(1, e == std::string::npos ? std::string::npos : e - 1), ""});
+            continue;
+        }
+        if (line.empty()) continue;
+        if (out->empty()) { *err = "line " + std::to_string(no) + " comes before the first '>' header"; return false; }
+        out->back().seq += line;
+    }
+    if (out->empty()) { *err = "the pattern file holds no pattern"; return false; }
+    if (out->back().seq.empty()) { *err = "pattern " + out->back().name + " has no sequence"; return false; }
+    for (const Pattern& p : *out)
+        if (p.seq.size() > 64) { *err = "pattern " + p.name + " is longer than 64 bytes"; return false; }
+    return true;
+}
+
+static int search_archives(int argc, char* argv[]) {
+    const char *pat_path = argv[2], *list_path = nullptr, *bed_path = nullptr;
+    int k = 0, strands = 3;
+    int i = 3;
+    for (; i + 1 < argc - 2; i += 2) {
+        const std::string opt = argv[i], v = argv[i + 1];
+        if (opt == "--archives") list_path = argv[i + 1];
+        else if (opt == "--regions") bed_path = argv[i + 1];
+        else if (opt == "--mismatches") {
+            if (v.empty() || v.size() > 2 || v.find_first_not_of("0123456789") != std::string::npos) { std::cerr << "Error: bad mismatch count " << v << "\n"; return 1; }
+            k = std::stoi(v);
+        } else if (opt == "--strand") {
+            if (v != "both" && v != "+" && v != "-") { std::cerr << "Error: --strand takes both, + or -\n"; return 1; }
+            strands = v == "both" ? 3 : v == "+" ? 1 : 2;
+        } else { std::cerr << "Error: unknown option " << opt << "\n"; return 1; }
+    }
+    if (i != argc - 2 || !list_path) { std::cerr << "Error: --search needs --archives <list>, then <reference_file> <output_folder>\n"; return 1; }
+    const std::string ref_path = argv[argc - 2], out_dir = argv[argc - 1];
+    std::string pat_text, err;
+    std::vector<Pattern> pats;
+    if (!sccg_host::read_file(pat_path, pat_text)) { std::cerr << "Error opening pattern file: " << pat_path << "\n"; return 1; }
+    if (!parse_patterns(pat_text, &pats, &err)) { std::cerr << "Error: " << err << "\n"; return 1; }
+    int64_t minlen = 64;
+    for (const Pattern& p : pats) minlen = (int64_t)p.seq.size() < minlen ? (int64_t)p.seq.size() : minlen;
+    if (k >= minlen) { std::cerr << "Error: the mismatch count must be below the shortest pattern's length (" << minlen << ")\n"; return 1; }
+    std::vector<BedRegion> bed;
+    if (bed_path) {
+        std::string bed_text;
+        if (!sccg_host::read_file(bed_path, bed_text)) { std::cerr << "Error opening BED file: " << bed_path << "\n"; return 1; }
+        if (!parse_bed(bed_text, &bed, &err)) { std::cerr << "Error: " << err << "\n"; return 1; }
+    }
+    std::vector<std::string> arcs;
+    if (!read_archive_list(list_path, &arcs)) return 1;
+    sccg_ctx* ctx = resident_context(ref_path);
+    if (!ctx) return 1;
+    std::error_code ec;
+    if (!fs::exists(out_dir)) fs::create_directory(out_dir, ec);
+    int status = 1;
+    std::vector<sccg_archive*> open;
+    std::vector<sccg_window> wins;
+    std::vector<size_t> win_arc;
+    std::string text;
+    [&] {
+        for (const std::string& arc : arcs) {                               // unpacked one at a time: archives may share a file name
+            sccg_archive* a = open_archive_file(ctx, arc, out_dir);
+            if (!a) return;
+            open.push_back(a);
+            int64_t seq_len = 0;
+            sccg_archive_info(a, &seq_len, nullptr, nullptr);
+            const int64_t ai = (int64_t)open.size() - 1;
+            if (!bed_path) { wins.push_back(sccg_window{ai, 0, seq_len}); win_arc.push_back((size_t)ai); }
+            for (const BedRegion& r : bed) {
+                if (r.end > seq_len) { std::cerr << "Error: region " << r.name << ":" << r.start << "-" << r.end << " ends past the end of " << arc << " (" << seq_len << " bp)\n"; return; }
+                wins.push_back(sccg_window{ai, r.start, r.end}); win_arc.push_back((size_t)ai);
+            }
+        }
+        std::string blob;
+        std::vector<int64_t> off(1, 0);
+        for (const Pattern& p : pats) { blob += p.seq; off.push_back((int64_t)blob.size()); }
+        int64_t n = 0;
+        std::vector<sccg_hit> hits;
+        int rc = sccg_archive_search(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), blob.data(), off.data(), (int64_t)pats.size(),
+                                     k, strands, nullptr, 0, &n);
+        if (rc == SCCG_OK && n > 0) {
+            hits.resize((size_t)n);
+            rc = sccg_archive_search(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), blob.data(), off.data(), (int64_t)pats.size(),
+                                     k, strands, hits.data(), n, &n);
+        }
+        if (rc != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
+        std::vector<std::string> stems;
+        for (const std::string& arc : arcs) stems.push_back(fs::path(arc).stem().string());
+        for (const sccg_hit& h : hits) {
+            text += stems[win_arc[(size_t)h.window]] + "\t" + std::to_string(h.pos) + "\t" + std::to_string(h.pos + (int64_t)pats[(size_t)h.pattern].seq.size()) +
+                    "\t" + pats[(size_t)h.pattern].name + "\t" + std::to_string(h.mismatches) + (h.strand ? "\t-\n" : "\t+\n");
+        }
+        status = 0;
+    }();
+    sccg_destroy(ctx);                                                      // (releases the archives)
+    if (status) return status;
+    if (!write_output(out_dir + "/hits.bed", text)) { std::cerr << "Error opening output file: " << out_dir << "\n"; return 1; }
+    return 0;
+}
+
 int main(int argc, char* argv[]) {
     const bool batch = argc >= 3 && std::string(argv[1]) == "--batch";
     const bool regions = argc == 6 && std::string(argv[1]) == "--regions";
     const bool archives = argc == 7 && std::string(argv[1]) == "--regions" && std::string(argv[3]) == "--archives";
-    if (argc != 4 && !batch && !regions && !archives) {                     // decompression.cpp:283-286
+    const bool search = argc >= 7 && std::string(argv[1]) == "--search";
+    if (argc != 4 && !batch && !regions && !archives && !search) {          // decompression.cpp:283-286
         std::cerr << "Usage: " << argv[0] << " <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n"
                   << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n"
-                  << "       " << argv[0] << " --regions <regions.bed> --archives <list of .7z files, one per line> <reference_file> <output_folder>\n";
+                  << "       " << argv[0] << " --regions <regions.bed> --archives <list of .7z files, one per line> <reference_file> <output_folder>\n"
+                  << "       " << argv[0] << " --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K] [--strand both|+|-] <reference_file> <output_folder>\n";
         return 1;
     }
     try {
         if (archives) return extract_archives(argv[2], argv[4], argv[5], argv[6]);
+        if (search) return search_archives(argc, argv);
         if (regions) {
             Job job; job.a = argv[3]; job.b = argv[4]; job.out = argv[5];
             return extract_regions(argv[2], job);
