@@ -419,19 +419,20 @@ __device__ __forceinline__ int lm_parse(LmWarpSmem& S, const u32 (&wm)[4], int L
 //     shorter interval        : every position of it is a looked-up window that contains m_i -> literals
 //     every m_i               : a looked-up window that starts with a mismatch -> literal
 // (windows must start at j <= L - k, :64).  So the warp works lane-parallel, no serial walk:
-//   1. mismatching symbols from the diagonal XOR words it still holds in registers (one packed warp scan orders them),
+//   1. mismatching symbols from the word ballots of the diagonal compare: the warp visits the (usually one or two) differing
+//      8-byte words in position order, lanes 0-7 test one symbol of the word each, a ballot gives each mismatch its slot,
 //   2. lane i owns interval i: its looked-up windows (<= 32 in total, else the generic path runs) and its match,
 //   3. PROOF of the hypothesis.  An occurrence of a looked-up k-mer t[j..j+k) at r[p..p+k) implies that the 8-byte chunk
 //      of r at the next multiple of 4, a = ceil4(p), equals the 8 bytes of t at u = j + (a - p), u in {j .. j+3}
-//      (u + 8 <= j + k needs k >= 11).  So the <= 4 * 32 chunks t[u..u+8) go into a hash table keyed by content and every
-//      lane probes the 250 four-aligned chunks of r (8 per lane, straight from two 16-byte shared-memory loads): 8
+//      (u + 8 <= j + k needs k >= 11).  So the <= 4 * 32 chunks t[u..u+8) go into a hash table keyed by content (entry e on
+//      lane e % 32: a segment with <= 8 looked-up windows stores one entry per lane) and every lane probes the 250 four-aligned chunks of r (8 per lane, straight from two 16-byte shared-memory loads): 8
 //      instructions per chunk and no per-position work at all.  A table entry carries u: a hit with a == u is the
 //      diagonal itself (the expected occurrence of a clean window, no occurrence at all for a window with a mismatch) and is
 //      ignored by construction (the XOR below is 0); any other hit is checked symbol by symbol, and a real occurrence --
 //      a repeat in r, an off-diagonal occurrence of a mutated k-mer -- rejects the hypothesis.
 // Rejection falls back to the exact generic path (index + parse), so the result is always the reference's.
 // ------------------------------------------------------------------------------------------------
-static const int DV_MAX_MISWORDS = 16;        // mismatching 8-byte words (<= 128 symbols: the packed scan below cannot overflow)
+static const int DV_MAX_MISWORDS = 16;        // mismatching 8-byte words (one warp-uniform round each in step 1)
 static const int DV_MAX_MIS = 30;             // mismatching symbols (+ sentinel <= 32 intervals, one per lane)
 static const int DV_TAB = 1024;               // table slots: S.head and S.next together (4 KiB)
 
@@ -439,46 +440,52 @@ __device__ __forceinline__ u32 dv_hash(u32 lo, u32 hi) { return (lo * 0x9E3779B1
 // table entry / probe value: hash bits 11..31, bit 10 set (an empty slot is 0), symbol position in bits 0..9
 __device__ __forceinline__ u32 dv_slot(u32 e, u32 alt_shift) { return (e >> alt_shift) & (u32)(DV_TAB - 1); }   // alt_shift: 22, or 12 on the retry
 
+// table entry e of the proof: the chunk t[u .. u+8), u = (position of looked-up window e / 4) + e % 4
+__device__ __forceinline__ u32 dv_entry(const LmWarpSmem& S, int e) {
+    const int u = (int)(S.qv[e >> 2] & 0x3ffu) + (e & 3);
+    const u32* t32 = reinterpret_cast<const u32*>(S.t);
+    const int w = u >> 2;
+    const u32 sh = (u32)(u & 3) * 8u;
+    const u32 b0 = t32[w], b1 = t32[w + 1], b2 = t32[w + 2];
+    return (dv_hash(__funnelshift_r(b0, b1, sh), __funnelshift_r(b1, b2, sh)) & ~1023u) | 1024u | (u32)u;
+}
+enum { DV_STORE = 0, DV_CHECK = 1, DV_CLEAR = 2 };
+__device__ __forceinline__ void dv_tab_one(u32* tab, u32 x, u32 alt, int op, bool& coll) {
+    u32& s = tab[dv_slot(x, alt)];
+    if (op == DV_STORE) s = x;
+    else if (op == DV_CHECK) coll |= s != x;
+    else s = 0u;
+}
+// one pass over the ne = 4 * nq entries, entry e on lane e % 32.  en0: this lane's entry `lane` (0: none); the later rounds
+// (more than 8 looked-up windows) are recomputed.  DV_CHECK returns true if another entry holds one of this lane's slots.
+__device__ __forceinline__ bool dv_tab_pass(const LmWarpSmem& S, u32* tab, u32 en0, int ne, u32 alt, int op) {
+    bool coll = false;
+    if (en0) dv_tab_one(tab, en0, alt, op, coll);
+#pragma unroll 1
+    for (int e = 32 + lane_of(); e < ne; e += 32) dv_tab_one(tab, dv_entry(S, e), alt, op, coll);
+    return coll;
+}
+
 // returns the number of matches (written to gmatches, their summed length in covered), or 0 when the hypothesis was
 // rejected / not applicable.  tab_clean (in/out): the 4 KiB table region is all zero.
-__device__ __forceinline__ int lm_diag_parse(LmWarpSmem& S, const u64 (&rw)[4], const u64 (&tw)[4], const u32 (&wm)[4], int L, int k, bool& tab_clean,
+__device__ __forceinline__ int lm_diag_parse(LmWarpSmem& S, const u32 (&wm)[4], int L, int k, bool& tab_clean,
                                              u32* __restrict__ gmatches, int& covered) {
     const int lane = lane_of();
     if (__popc(wm[0]) + __popc(wm[1]) + __popc(wm[2]) + __popc(wm[3]) > DV_MAX_MISWORDS) return 0;
-    // ---- 1. mismatching symbols.  Lane holds the words q = lane + 32 * it; symbol order is it-major.
-    u32 bm[4];
-    u32 cntp = 0u;                                                  // four 8-bit counters, one per `it`
+    // ---- 1. mismatching symbols, ascending: bit `lane` of wm[it] is word 32 * it + lane (S.r / S.t hold the upper-cased pair)
+    int c = 0;
 #pragma unroll
     for (int it = 0; it < 4; ++it) {
-        bm[it] = 0u;
-        if (wm[it]) {                                               // uniform
-            const u64 d = rw[it] ^ tw[it];
-            if (d) {
-                const int q = lane + 32 * it;
-                u32 m = movemask8(nonzero_flags8(d));
-                if (8 * q + 8 > L) m = 8 * q < L ? (m & ((1u << (L - 8 * q)) - 1u)) : 0u;
-                bm[it] = m;
-                cntp |= (u32)__popc(m) << (8 * it);
-            }
+        for (u32 m = wm[it]; m; m &= m - 1) {                      // uniform
+            const int pos = 8 * (32 * it + __ffs((int)m) - 1) + lane;
+            const bool mis = lane < 8 && pos < L && S.r[pos] != S.t[pos];
+            const u32 bal = __ballot_sync(SCCG_FULL_MASK, mis);
+            const int slot = c + __popc(bal & ((1u << lane) - 1u));
+            if (mis && slot < DV_MAX_MIS) S.mis[slot] = (u16)pos;
+            c += __popc(bal);
         }
     }
-    const u32 incl = warp_scan_incl(cntp);
-    const u32 tot = __shfl_sync(SCCG_FULL_MASK, incl, 31);
-    const int c = (int)((tot & 0xffu) + ((tot >> 8) & 0xffu) + ((tot >> 16) & 0xffu) + (tot >> 24));
     if (c > DV_MAX_MIS) return 0;
-    {
-        const u32 excl = incl - cntp;
-        u32 base = 0u;
-#pragma unroll
-        for (int it = 0; it < 4; ++it) {
-            if (bm[it]) {
-                u32 off = base + ((excl >> (8 * it)) & 0xffu);
-                const int q = lane + 32 * it;
-                for (u32 m = bm[it]; m; m &= m - 1) S.mis[off++] = (u16)(8 * q + __ffs((int)m) - 1);
-            }
-            base += (tot >> (8 * it)) & 0xffu;
-        }
-    }
     if (lane == 0) S.mis[c] = (u16)L;                               // sentinel
     __syncwarp();
     // ---- 2. lane i owns the mismatch-free interval [a, b) before mismatch i (i == c: the tail up to L)
@@ -514,40 +521,17 @@ __device__ __forceinline__ int lm_diag_parse(LmWarpSmem& S, const u64 (&rw)[4], 
         tab_clean = true;
     }
     __syncwarp();
-    // ---- 3a. the chunks t[u .. u+8), u = j .. j+3, of this lane's looked-up window
-    const bool isq = lane < nq;
-    const int myj = isq ? (int)(S.qv[lane] & 0x3ffu) : 0;
-    u32 e[4];
-    {
-        const u32* t32 = reinterpret_cast<const u32*>(S.t);
-        const int w = myj >> 2;
-        const u32 sh = (u32)(myj & 3) * 8u;
-        const u32 a0 = t32[w], a1 = t32[w + 1], a2 = t32[w + 2], a3 = t32[w + 3];
-        const u32 w0 = __funnelshift_r(a0, a1, sh), w1 = __funnelshift_r(a1, a2, sh), w2 = __funnelshift_r(a2, a3, sh);
-#pragma unroll
-        for (int o = 0; o < 4; ++o) {
-            const u32 lo = o ? __funnelshift_r(w0, w1, 8u * o) : w0, hi = o ? __funnelshift_r(w1, w2, 8u * o) : w1;
-            e[o] = (dv_hash(lo, hi) & ~1023u) | 1024u | (u32)(myj + o);
-        }
-    }
+    // ---- 3a. the chunks t[u .. u+8), u = j .. j+3, of the looked-up windows j
+    const int ne = 4 * nq;
+    const u32 en0 = lane < ne ? dv_entry(S, lane) : 0u;
     u32 alt = 22u;
     for (;;) {
-        if (isq) {
-#pragma unroll
-            for (int o = 0; o < 4; ++o) tab[dv_slot(e[o], alt)] = e[o];
-        }
+        dv_tab_pass(S, tab, en0, ne, alt, DV_STORE);
         __syncwarp();
-        bool coll = false;                                          // two different chunks in one slot (equal chunks of neighbouring windows coincide)
-        if (isq) {
-#pragma unroll
-            for (int o = 0; o < 4; ++o) coll |= tab[dv_slot(e[o], alt)] != e[o];
-        }
+        const bool coll = dv_tab_pass(S, tab, en0, ne, alt, DV_CHECK);   // two different chunks in one slot (equal chunks of neighbouring windows coincide)
         if (!__any_sync(SCCG_FULL_MASK, coll)) break;
         __syncwarp();
-        if (isq) {
-#pragma unroll
-            for (int o = 0; o < 4; ++o) tab[dv_slot(e[o], alt)] = 0u;
-        }
+        dv_tab_pass(S, tab, en0, ne, alt, DV_CLEAR);
         __syncwarp();
         if (alt == 12u) return 0;                                   // collides under both slot functions (or equal chunks at different positions): generic path
         alt = 12u;
@@ -599,10 +583,7 @@ __device__ __forceinline__ int lm_diag_parse(LmWarpSmem& S, const u64 (&rw)[4], 
         }
     }
     __syncwarp();
-    if (isq) {                                                      // leave the table clean for the next segment
-#pragma unroll
-        for (int o = 0; o < 4; ++o) tab[dv_slot(e[o], alt)] = 0u;
-    }
+    dv_tab_pass(S, tab, en0, ne, alt, DV_CLEAR);                    // leave the table clean for the next segment
     __syncwarp();
     return __any_sync(SCCG_FULL_MASK, bad) ? 0 : nmatch;
 }
@@ -775,7 +756,7 @@ __device__ __forceinline__ void seg_match_body(const u8* __restrict__ ref, i64 n
             __syncwarp();
             SEG_PHASE(0);
             if (use_diag && Lr == Lt && Lt >= k1 && k1 >= 11 &&
-                (nmatch = lm_diag_parse(S, nrw, ntw, wm, Lt, k1, tab_clean, matches + (i64)seg * LM_SLOT, covered)) > 0) {
+                (nmatch = lm_diag_parse(S, wm, Lt, k1, tab_clean, matches + (i64)seg * LM_SLOT, covered)) > 0) {
                 // near-identical segment: parse determined by the mismatch positions, hypothesis proven against all of r
                 direct = true;
                 SEG_STAT(1);

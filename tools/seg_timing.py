@@ -33,8 +33,17 @@ ph = call[1:]
 gen = ph[1] > 0
 print("generic segments", int(gen.sum()), "mean cycles: staged %.0f diagonal attempt %.0f runs %.0f index %.0f parse %.0f epilogue %.0f" % tuple(ph[i][gen].mean() for i in range(6)), " total mean", c[gen].mean())
 print("segments", nseg, "sum cycles", c.sum(), "mean", c.mean(), "median", np.median(c), "p99", np.percentile(c, 99), "max", c.max())
-top = np.argsort(-c)[:15]
 tu = np.where((tgt >= 97) & (tgt <= 122), tgt - 32, tgt).astype(np.uint8)
+ru = np.where((ref >= 97) & (ref <= 122), ref - 32, ref).astype(np.uint8)
+# path of each segment: identical pairs are decided in registers, generic segments record their phases, the rest took the
+# diagonal-hypothesis path (the same split for any build of the library, so two builds can be compared)
+m = min(ru.size, tu.size) // 1000 * 1000
+ident = np.zeros(nseg, dtype=bool)
+ident[:m // 1000] = (ru[:m] == tu[:m]).reshape(-1, 1000).all(axis=1)
+diag = ~ident & ~gen
+for name, sel in (("identical", ident), ("diagonal", diag), ("generic", gen)):
+    print(f"path {name}: {int(sel.sum())} segments, mean cycles {c[sel].mean() if sel.any() else 0.0:.0f}, sum {int(c[sel].sum())}")
+top = np.argsort(-c)[:15]
 for i in top:
     r = ref[i * 1000:(i + 1) * 1000]; t = tu[i * 1000:(i + 1) * 1000]
     m = min(r.size, t.size)
