@@ -231,6 +231,31 @@ int sccg_archive_search(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_
                         const char* patterns, const int64_t* pattern_off, int64_t n_patterns, int max_mismatches, int strands,
                         sccg_hit* hits, int64_t hits_cap, int64_t* n_hits);
 
+/* Pattern search with insertions and deletions: the inputs of sccg_archive_search (windows, archives, 1 to 1024 patterns of 1
+ * to 64 bytes, strands 1/2/3, the per-byte match rule), with unit-cost Levenshtein distance ed(P, X) instead of mismatches: a
+ * substitution is a pair of bytes that does not match under the rule, an insertion an extra D byte, a deletion a missing
+ * pattern byte.  Strand 1 searches the reverse complement of the pattern (the same complement) on forward D.
+ * A hit (window w, start, end, pattern i, strand s, edits): for window w = D_a[ws:we], pattern i (its reverse complement for
+ * s = 1) and an end e with ws < e <= we, let d(e) = min over ws <= x <= e of ed(P, D[x:e]).  There is a hit iff
+ * d(e) <= max_edits, with end = e, edits = d(e) and start = the largest x reaching d(e) (the shortest text).  start and end
+ * are absolute D coordinates: [start, end) is a BED interval.  At most one hit per (w, e, i, s), in (window, end, pattern,
+ * strand) order.  Hits are not clustered: every qualifying end is reported, so with max_edits >= 1 an exact occurrence
+ * ending at e also gives 1-edit hits ending at e - 1 and e + 1.  Windows shorter than len_i - max_edits give no hits for i.
+ * With max_edits = 0 the hits are exactly the sccg_archive_search hits with max_mismatches = 0 (start = pos,
+ * end = pos + len_i).  For every sccg_archive_search hit (w, pos, i, s, m) there is a hit here at end = pos + len_i with
+ * edits <= m.
+ * *n_hits always receives the total.  hits == NULL counts only.  When hits is given and the total exceeds hits_cap, the call
+ * returns SCCG_E_ARG with the required count in *n_hits (hits then holds an unspecified prefix).
+ * Errors: those of sccg_archive_search, in the same order and all before any device work, with max_edits in place of
+ * max_mismatches (>= 0 and below the shortest pattern's length).
+ * Windows may add up to any size: the call splits them into launches (SCCG_SEARCH_SPLIT: candidate end positions per launch).
+ * Cost grows linearly with the number of patterns.  Profile: h2d_ms (window and pattern tables), gather_ms (search kernels),
+ * kernels_ms, d2h_ms (hits), launches. */
+typedef struct { int64_t window, start, end; int32_t pattern, strand, edits, reserved; } sccg_edit_hit;
+int sccg_archive_search_edits(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
+                              const char* patterns, const int64_t* pattern_off, int64_t n_patterns, int max_edits, int strands,
+                              sccg_edit_hit* hits, int64_t hits_cap, int64_t* n_hits);
+
 /* FASTA file images in: read_genomes_from_files (compression.cpp:181-220) and the reference reader of decompress_genome
  * (decompression.cpp:47-58) run on the device -- header lines skipped ('>' at a line start; in the target only the first one,
  * which becomes the header line of the output), isspace() bytes removed -- followed by sccg_compress / sccg_decompress.

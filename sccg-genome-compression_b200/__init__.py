@@ -141,6 +141,7 @@ def load_library(path: str | os.PathLike | None = None) -> C.CDLL:
     lib.sccg_archive_close.argtypes = [vp, vp]
     lib.sccg_archive_extract.argtypes = [vp, vp, i64, vp, i64, vp, i64, i64p]
     lib.sccg_archive_search.argtypes = [vp, vp, i64, vp, i64, cp, vp, i64, C.c_int, C.c_int, vp, i64, i64p]
+    lib.sccg_archive_search_edits.argtypes = [vp, vp, i64, vp, i64, cp, vp, i64, C.c_int, C.c_int, vp, i64, i64p]
     lib.sccg_mgpu_unique_id.argtypes = [C.c_char_p]
     lib.sccg_mgpu_init.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.POINTER(vp)]
     lib.sccg_mgpu_destroy.argtypes = [vp]
@@ -619,6 +620,44 @@ class Context:
         h = buf[:n.value]
         return np.stack([h["window"], h["pos"], h["pattern"].astype(np.int64), h["strand"].astype(np.int64),
                          h["mismatches"].astype(np.int64)], axis=1).reshape(-1, 5)
+
+    _EDIT_HIT = [("window", "<i8"), ("start", "<i8"), ("end", "<i8"), ("pattern", "<i4"), ("strand", "<i4"), ("edits", "<i4"),
+                 ("reserved", "<i4")]
+
+    def search_edits(self, archives, patterns, windows=None, max_edits: int = 0, strands="both", count_only: bool = False):
+        """every end of an alignment of the patterns within max_edits edits (substitutions, insertions, deletions) in windows of
+        open archives (sccg_archive_search_edits, include/sccg.h); windows and strands as for search.  -> an (n, 6) int64 array
+        of [window, start, end, pattern, strand, edits] in (window, end, pattern, strand) order, or the number of hits when
+        count_only.  Hits are not clustered: every end within max_edits is reported.  Same buffer scheme as search."""
+        import numpy as np
+        if strands not in self._STRANDS:
+            raise ValueError("strands must be 'both', '+' or '-'")
+        if windows is None:
+            windows = [(k, 0, a.seq_len) for k, a in enumerate(archives)]
+        w = np.ascontiguousarray(np.asarray(windows, dtype=np.int64).reshape(-1, 3))      # sccg_window[] layout
+        pats = [bytes(p) for p in patterns]
+        off = np.zeros(len(pats) + 1, dtype=np.int64)
+        off[1:] = np.cumsum([len(p) for p in pats]) if pats else []
+        blob = b"".join(pats)
+        arr = (C.c_void_p * max(len(archives), 1))(*[a.handle for a in archives])
+        n = C.c_int64(-1)
+
+        def run(out, cap):
+            return self.lib.sccg_archive_search_edits(self.handle, arr if len(archives) else None, len(archives), w.ctypes.data if len(w) else None,
+                                                      len(w), blob, off.ctypes.data if pats else None, len(pats), max_edits,
+                                                      self._STRANDS[strands], out, cap, C.byref(n))
+        if count_only:
+            self._check(run(None, 0))
+            return n.value
+        for cap in (65536, None):
+            buf = np.zeros(n.value if cap is None else cap, dtype=self._EDIT_HIT)
+            rc = run(buf.ctypes.data if len(buf) else None, len(buf))
+            if rc == SCCG_OK or not (cap is not None and rc == SCCG_E_ARG and n.value > cap):
+                break
+        self._check(rc)
+        h = buf[:n.value]
+        return np.stack([h["window"], h["start"], h["end"], h["pattern"].astype(np.int64), h["strand"].astype(np.int64),
+                         h["edits"].astype(np.int64)], axis=1).reshape(-1, 6)
 
     # decompress_genome (in-memory part) + reconstruct_genome + header line (decompression.cpp:66-110, :117-279, :322)
     def decompress(self, ref_raw: bytes, intermediate: bytes) -> bytes:

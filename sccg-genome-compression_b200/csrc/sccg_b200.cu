@@ -5,6 +5,7 @@
 #include "sccg_decode.cuh"
 #include "sccg_extract.cuh"
 #include "sccg_search.cuh"
+#include "sccg_search_edit.cuh"
 #include "sccg_fasta.cuh"
 #include "sccg_shard.cuh"
 #include "sccg_mgpu.cuh"
@@ -590,6 +591,18 @@ int sccg_archive_search(sccg_ctx* c, sccg_archive* const* archives, int64_t n_ar
     prof_reset(c);
     const int rc = archive_search_impl(c, archives, n_archives, windows, n_windows, patterns, pattern_off, n_patterns, max_mismatches,
                                        strands, hits, hits_cap, n_hits);
+    if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
+    return rc;
+}
+
+int sccg_archive_search_edits(sccg_ctx* c, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
+                              const char* patterns, const int64_t* pattern_off, int64_t n_patterns, int max_edits, int strands,
+                              sccg_edit_hit* hits, int64_t hits_cap, int64_t* n_hits) {
+    if (!c) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    const int rc = archive_search_edits_impl(c, archives, n_archives, windows, n_windows, patterns, pattern_off, n_patterns, max_edits,
+                                             strands, hits, hits_cap, n_hits);
     if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
     return rc;
 }

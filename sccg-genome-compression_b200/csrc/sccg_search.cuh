@@ -33,6 +33,7 @@ struct SrchArgs {
     ExtArgs x;               // the launch's image: r_start, r_off, r_tag (archive << 1), n_reg, total (image bytes), g, lane_min
     const u32* r_win;        // window index of region i (a window cut over launches makes several regions)
     const u32* r_cend;       // candidate positions of region i: image [r_off[i], r_cend[i]); bytes past it are look-ahead
+    const u32* r_cbeg;       // (= r_off: no look-behind; the edit-distance engine's table has it)
     const u16* desc;         // pattern byte descriptors, both strands (the minus strand: the reverse complement)
     const u8* plen;
     int n_pat, strands, kmax;
@@ -59,7 +60,7 @@ __device__ __forceinline__ u32 srch_eq4(u32 x, u32 rep) {
 }
 
 // the match rule of one pattern byte descriptor against one byte of D
-__device__ __forceinline__ bool srch_match(u32 d, u32 b) {
+__host__ __device__ __forceinline__ bool srch_match(u32 d, u32 b) {
     const u32 l = b | 0x20u;
     if (((d & 1u) && l == 'a') || ((d & 2u) && l == 'c') || ((d & 4u) && l == 'g') || ((d & 8u) && l == 't') || ((d & SD_N) && l == 'n')) return true;
     if (!(d & SD_OTHER)) return false;
@@ -70,8 +71,10 @@ __device__ __forceinline__ bool srch_match(u32 d, u32 b) {
 // image bytes [Q0, Qe) -> s.O: every piece that reaches into them, without the lowercase pass (the match is case-blind; the
 // lane path's ext_sym still lowers, which changes nothing here).  Tiles of lane_min pieces or more: a thread per piece, as in
 // ext_gather_k, searching each archive's whole tables.  Others: warp w builds the pieces that meet the w-th quarter of the
-// bytes, clipped to it, so a tile made of one long piece keeps every warp busy.
-__device__ __forceinline__ void srch_build(const ExtArgs& e, u32 Q0, u32 Qe, SrchSmem& s) {
+// bytes, clipped to it, so a tile made of one long piece keeps every warp busy.  Q0 is a multiple of 16; s.O is zero past
+// the last byte.  (S: SrchSmem, or the shared memory of the edit-distance engine, sccg_search_edit.cuh)
+template <class S>
+__device__ __forceinline__ void srch_build(const ExtArgs& e, u32 Q0, u32 Qe, S& s) {
     const int warp = (int)(threadIdx.x >> 5), lane = lane_of();
     if (threadIdx.x == 0) mbar_init(&s.bar, 1u);
     if (warp < 2) {
@@ -101,7 +104,7 @@ __device__ __forceinline__ void srch_build(const ExtArgs& e, u32 Q0, u32 Qe, Src
     __syncthreads();                                                  // every copy has been issued ...
     if (threadIdx.x == 0) mbar_arrive(&s.bar);
     mbar_wait(&s.bar, 0u);                                            // ... and has landed
-    for (u32 i = Qe - Q0 + threadIdx.x; i < (u32)SRCH_BYTES; i += SRCH_T) s.O[i] = 0;
+    for (u32 i = Qe - Q0 + threadIdx.x; i < (u32)sizeof(s.O); i += SRCH_T) s.O[i] = 0;
     __syncthreads();
 }
 
@@ -273,12 +276,11 @@ static u16 search_desc(u8 p) {
     return (u16)(SD_OTHER | ((P >= 'A' && P <= 'Z') ? SD_FOLD : 0u) | (P << 8));
 }
 
-// sccg_archive_search: argument checks (include/sccg.h, in that order), the pattern tables once, then per launch one copy of the
-// region table, the count pass, the scan and one round trip for the total, and (while the hits fit hits_cap) the emit pass and
-// one copy of its hits
-static int archive_search_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, const sccg_window* windows, i64 n_windows,
-                               const char* patterns, const int64_t* pattern_off, i64 n_patterns, int max_mismatches, int strands,
-                               sccg_hit* hits, i64 hits_cap, int64_t* n_hits) {
+// the argument checks of sccg_archive_search and sccg_archive_search_edits (include/sccg.h, in that order; k_why: the message
+// for k out of range) -> the shortest and the longest pattern
+static int search_check(sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, const sccg_window* windows, i64 n_windows,
+                        const char* patterns, const int64_t* pattern_off, i64 n_patterns, int k, const char* k_why, int strands,
+                        i64 hits_cap, int64_t* n_hits, i64* minlen_out, i64* maxlen_out) {
     if (!n_hits || n_archives < 0 || n_windows < 0 || n_patterns < 0 || hits_cap < 0 || (n_archives > 0 && !archives) ||
         (n_windows > 0 && !windows) || (n_patterns > 0 && (!pattern_off || !patterns)))
         return set_error(SCCG_E_ARG, "null argument");
@@ -295,7 +297,7 @@ static int archive_search_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n
         minlen = len < minlen ? len : minlen;
         maxlen = len > maxlen ? len : maxlen;
     }
-    if (max_mismatches < 0 || max_mismatches >= minlen) return set_error(SCCG_E_ARG, "max_mismatches must be >= 0 and below the shortest pattern's length");
+    if (k < 0 || k >= minlen) return set_error(SCCG_E_ARG, k_why);
     if (strands < 1 || strands > 3) return set_error(SCCG_E_ARG, "strands must be 1 (forward), 2 (reverse complement) or 3 (both)");
     // ---- windows: the query checks of sccg_archive_extract
     int first = ARCHIVE_QUERY_OK;
@@ -304,90 +306,77 @@ static int archive_search_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n
         if (bad < first) first = bad;
     }
     if (first < ARCHIVE_QUERY_OK) return set_error(SCCG_E_ARG, archive_query_why[first]);
-    if (n_windows == 0) return SCCG_OK;
-    // ---- regions of the launches: window pieces of at most `lim` candidate positions per launch, each with maxlen - 1 bytes
-    //      of look-ahead where it is cut short of its window's end
-    const int ns = (strands & 1) + (strands >> 1);
-    i64 lim = search_split();
-    const i64 hit_lim = 0xffffffffLL / (n_patterns * ns);             // a launch's hits fit 32 bits
-    lim = lim < hit_lim ? lim : hit_lim;
-    std::vector<u32> rs, rlen, rcand, rwin, rarch;
-    std::vector<size_t> launch_end;
+    *minlen_out = minlen; *maxlen_out = maxlen;
+    return SCCG_OK;
+}
+
+// the regions of a search's launches: the windows of at least min_win bytes, cut into pieces of at most `lim` candidate positions
+// per launch.  Region i is D[rs[i], rs[i] + rlen[i]) of archive rarch[i]; its candidates are bytes [rlo[i], rhi[i]) of it; the
+// bytes before them (at most `behind`) and past them (at most `ahead`) are those of its window that a cut left out of the piece.
+struct SearchCut {
+    std::vector<u32> rs, rlen, rlo, rhi, rwin, rarch;
+    std::vector<size_t> launch_end;                                   // regions [launch_end[k - 1], launch_end[k]) make launch k
+    size_t max_reg = 0;
+};
+
+static void search_cut(const sccg_window* windows, i64 n_windows, i64 min_win, i64 ahead, i64 behind, i64 lim, SearchCut& o) {
     i64 left = lim;
     for (i64 w = 0; w < n_windows; ++w) {
         const sccg_window& W = windows[w];
-        if (W.end - W.start < minlen) continue;                         // no pattern fits
+        if (W.end - W.start < min_win) continue;                        // no pattern fits
         for (i64 s = W.start; s < W.end;) {
             const i64 take = W.end - s < left ? W.end - s : left;
-            const i64 ce = s + take, be = ce + maxlen - 1 < W.end ? ce + maxlen - 1 : W.end;
-            rs.push_back((u32)s); rlen.push_back((u32)(be - s)); rcand.push_back((u32)take); rwin.push_back((u32)w); rarch.push_back((u32)W.archive);
+            const i64 ce = s + take, be = ce + ahead < W.end ? ce + ahead : W.end, bs = s - behind > W.start ? s - behind : W.start;
+            o.rs.push_back((u32)bs); o.rlen.push_back((u32)(be - bs)); o.rlo.push_back((u32)(s - bs)); o.rhi.push_back((u32)(ce - bs));
+            o.rwin.push_back((u32)w); o.rarch.push_back((u32)W.archive);
             left -= take;
             s = ce;
-            if (left == 0) { launch_end.push_back(rs.size()); left = lim; }
+            if (left == 0) { o.launch_end.push_back(o.rs.size()); left = lim; }
         }
     }
-    if (launch_end.empty() || launch_end.back() != rs.size()) launch_end.push_back(rs.size());
-    size_t max_reg = 0;
-    for (size_t k = 0, b = 0; k < launch_end.size(); b = launch_end[k++]) max_reg = launch_end[k] - b > max_reg ? launch_end[k] - b : max_reg;
-    // ---- staging: [GatherArgs of every archive | descriptors | lengths] once, then [r_start | r_off | r_tag | r_win | r_cend] per launch
-    const size_t ga_bytes = sizeof(GatherArgs) * (size_t)n_archives;
-    const size_t desc_off = align_up(ga_bytes, 16), desc_bytes = sizeof(u16) * (size_t)n_patterns * 2 * SRCH_MAXLEN;
-    const size_t tab_bytes = align_up(desc_off + desc_bytes + (size_t)n_patterns, 16);
-    const size_t reg_bytes = sizeof(u32) * (5 * max_reg + 1);
-    SCCG_TRY(ext_staging(c, tab_bytes + reg_bytes));
-    u8* h = (u8*)c->h_ext;
-    GatherArgs* h_g = (GatherArgs*)h;
-    for (i64 k = 0; k < n_archives; ++k) {
-        const sccg_archive* a = archives[k];
-        if (a && a->ctx == c && a->gen == c->res_gen) h_g[k] = a->g;
-        else memset(&h_g[k], 0, sizeof(GatherArgs));                      // (named by no window)
-    }
-    u16* h_desc = (u16*)(h + desc_off);
-    u8* h_len = h + desc_off + desc_bytes;
-    for (i64 i = 0; i < n_patterns; ++i) {
-        const u8* p = (const u8*)patterns + pattern_off[i];
-        const i64 len = pattern_off[i + 1] - pattern_off[i];
-        h_len[i] = (u8)len;
-        for (i64 j = 0; j < SRCH_MAXLEN; ++j) {
-            h_desc[(i * 2) * SRCH_MAXLEN + j] = j < len ? search_desc(p[j]) : 0;
-            h_desc[(i * 2 + 1) * SRCH_MAXLEN + j] = j < len ? search_desc(comp_byte(p[len - 1 - j])) : 0;
-        }
-    }
-    u8* d_tab = nullptr; u32* d_reg = nullptr; u32* d_tile = nullptr;
-    SCCG_TRY(buf(c, B_SRCH_TAB, tab_bytes, &d_tab));
-    SCCG_TRY(buf(c, B_SRCH_REG, 5 * max_reg + 1, &d_reg));
+    if (o.launch_end.empty() || o.launch_end.back() != o.rs.size()) o.launch_end.push_back(o.rs.size());
+    for (size_t k = 0, b = 0; k < o.launch_end.size(); b = o.launch_end[k++]) o.max_reg = o.launch_end[k] - b > o.max_reg ? o.launch_end[k] - b : o.max_reg;
+}
+
+static void search_launch(sccg_ctx* c, unsigned ntiles, const SrchArgs& sa, bool emit) {
+    if (emit) LAUNCH(c, srch_emit_k, dim3(ntiles), dim3(SRCH_T), 0, sa);
+    else LAUNCH(c, srch_count_k, dim3(ntiles), dim3(SRCH_T), 0, sa);
+}
+
+// the launches of either engine (Args: SrchArgs or EditArgs, with their search_launch): per launch one copy of the region table
+// [r_start | r_off | r_tag | r_win | r_cend | r_cbeg] from h_reg to d_reg, the count pass, the scan and one round trip for the
+// total, and (while the hits fit hits_cap) the emit pass and one copy of its hits.  The table copy of the call is timed from
+// c->ev[4] on.
+template <class Args, class Hit>
+static int search_launches(sccg_ctx* c, const SearchCut& cut, u32* h_reg, u32* d_reg, Args& sa, Hit* hits, i64 hits_cap, int64_t* n_hits) {
     float h2d = 0.f, gat = 0.f, ker = 0.f, d2h = 0.f, ms = 0.f;
-    SCCG_CK(cudaEventRecord(c->ev[4], c->stream));
-    SCCG_CK(cudaMemcpyAsync(d_tab, h, tab_bytes, cudaMemcpyHostToDevice, c->stream));
-    SCCG_CK(cudaEventRecord(c->ev[5], c->stream));
-    u32* h_reg = (u32*)(h + tab_bytes);
     u32* h_total = (u32*)((char*)c->h_pinned + 8192);
-    SrchArgs sa;
-    sa.x.g = (const GatherArgs*)d_tab; sa.x.out = nullptr; sa.x.lane_min = ext_lane_min(); sa.x.err = nullptr;
-    sa.desc = (const u16*)(d_tab + desc_off); sa.plen = d_tab + desc_off + desc_bytes;
-    sa.n_pat = (int)n_patterns; sa.strands = strands; sa.kmax = max_mismatches; sa.maxlen = (u32)maxlen;
+    u32* d_tile = nullptr;
     i64 found = 0;
     bool over = false;
-    for (size_t k = 0, b = 0; k < launch_end.size(); b = launch_end[k++]) {
-        const size_t n = launch_end[k] - b;
+    for (size_t k = 0, b = 0; k < cut.launch_end.size(); b = cut.launch_end[k++]) {
+        const size_t n = cut.launch_end[k] - b;
         if (n == 0) continue;
         if (k > 0) { SCCG_CK(cudaEventRecord(c->ev[4], c->stream)); }
         u32* r_start = h_reg; u32* r_off = r_start + n; u32* r_tag = r_off + n + 1; u32* r_win = r_tag + n; u32* r_cend = r_win + n;
+        u32* r_cbeg = r_cend + n;
         u32 off = 0;
         for (size_t i = 0; i < n; ++i) {
-            r_start[i] = rs[b + i]; r_off[i] = off; r_tag[i] = rarch[b + i] << 1; r_win[i] = rwin[b + i]; r_cend[i] = off + rcand[b + i];
-            off += rlen[b + i];
+            r_start[i] = cut.rs[b + i]; r_off[i] = off; r_tag[i] = cut.rarch[b + i] << 1; r_win[i] = cut.rwin[b + i];
+            r_cend[i] = off + cut.rhi[b + i]; r_cbeg[i] = off + cut.rlo[b + i];
+            off += cut.rlen[b + i];
         }
         r_off[n] = off;
         const unsigned ntiles = div_up(off, SRCH_TILE);
         SCCG_TRY(buf(c, B_SRCH_TILE, 2 * (size_t)ntiles + 1, &d_tile));
-        SCCG_CK(cudaMemcpyAsync(d_reg, h_reg, sizeof(u32) * (5 * n + 1), cudaMemcpyHostToDevice, c->stream));
+        SCCG_CK(cudaMemcpyAsync(d_reg, h_reg, sizeof(u32) * (6 * n + 1), cudaMemcpyHostToDevice, c->stream));
         SCCG_CK(cudaEventRecord(c->ev[5], c->stream));
         sa.x.r_start = d_reg; sa.x.r_off = d_reg + n; sa.x.r_tag = d_reg + 2 * n + 1; sa.r_win = d_reg + 3 * n + 1; sa.r_cend = d_reg + 4 * n + 1;
+        sa.r_cbeg = d_reg + 5 * n + 1;
         sa.x.n_reg = (int)n; sa.x.total = off;
         sa.tile_cnt = d_tile; sa.tile_off = d_tile + ntiles; sa.hits = nullptr;
         SCCG_CK(cudaEventRecord(c->ev[3], c->stream));
-        LAUNCH(c, srch_count_k, dim3(ntiles), dim3(SRCH_T), 0, sa);
+        search_launch(c, ntiles, sa, false);
         SCCG_CK(cudaEventRecord(c->ev[2], c->stream));
         SCCG_TRY(scan_exclusive_u32(c, d_tile, d_tile + ntiles, (i64)ntiles, d_tile + 2 * ntiles));
         SCCG_CK(cudaEventRecord(c->ev[1], c->stream));
@@ -400,13 +389,13 @@ static int archive_search_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n
         found += t;
         if (!hits || over || t == 0) continue;
         if (found > hits_cap) { over = true; continue; }                  // the remaining launches are only counted
-        sccg_hit* d_hits = nullptr;
+        Hit* d_hits = nullptr;
         SCCG_TRY(buf(c, B_SRCH_HITS, (size_t)t, &d_hits));
         sa.hits = d_hits;
         SCCG_CK(cudaEventRecord(c->ev[3], c->stream));
-        LAUNCH(c, srch_emit_k, dim3(ntiles), dim3(SRCH_T), 0, sa);
+        search_launch(c, ntiles, sa, true);
         SCCG_CK(cudaEventRecord(c->ev[2], c->stream));
-        SCCG_CK(cudaMemcpyAsync(hits + (found - t), d_hits, sizeof(sccg_hit) * (size_t)t, cudaMemcpyDeviceToHost, c->stream));
+        SCCG_CK(cudaMemcpyAsync(hits + (found - t), d_hits, sizeof(Hit) * (size_t)t, cudaMemcpyDeviceToHost, c->stream));
         SCCG_CK(cudaEventRecord(c->ev[7], c->stream));
         SCCG_CK(cudaStreamSynchronize(c->stream));
         cudaEventElapsedTime(&ms, c->ev[3], c->ev[2]); gat += ms; ker += ms;
@@ -416,6 +405,64 @@ static int archive_search_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n
     *n_hits = found;
     if (over) return set_error(SCCG_E_ARG, "hit buffer too small (required count returned in *n_hits)");
     return SCCG_OK;
+}
+
+// the GatherArgs of every archive a window may name (a stale or foreign one is named by no window: zeros)
+static void search_stage_archives(const sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, GatherArgs* h_g) {
+    for (i64 k = 0; k < n_archives; ++k) {
+        const sccg_archive* a = archives[k];
+        if (a && a->ctx == c && a->gen == c->res_gen) h_g[k] = a->g;
+        else memset(&h_g[k], 0, sizeof(GatherArgs));
+    }
+}
+
+// the byte descriptors of pattern i (len bytes at p), both strands (the minus strand: the reverse complement), zero past len
+static void search_stage_desc(const u8* p, i64 len, u16* d) {
+    for (i64 j = 0; j < SRCH_MAXLEN; ++j) {
+        d[j] = j < len ? search_desc(p[j]) : 0;
+        d[SRCH_MAXLEN + j] = j < len ? search_desc(comp_byte(p[len - 1 - j])) : 0;
+    }
+}
+
+// sccg_archive_search: argument checks, the pattern tables once, then the launches (windows cut with maxlen - 1 bytes of
+// look-ahead)
+static int archive_search_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, const sccg_window* windows, i64 n_windows,
+                               const char* patterns, const int64_t* pattern_off, i64 n_patterns, int max_mismatches, int strands,
+                               sccg_hit* hits, i64 hits_cap, int64_t* n_hits) {
+    i64 minlen = 0, maxlen = 0;
+    SCCG_TRY(search_check(c, archives, n_archives, windows, n_windows, patterns, pattern_off, n_patterns, max_mismatches,
+                          "max_mismatches must be >= 0 and below the shortest pattern's length", strands, hits_cap, n_hits, &minlen, &maxlen));
+    if (n_windows == 0) return SCCG_OK;
+    const int ns = (strands & 1) + (strands >> 1);
+    i64 lim = search_split();
+    const i64 hit_lim = 0xffffffffLL / (n_patterns * ns);             // a launch's hits fit 32 bits
+    lim = lim < hit_lim ? lim : hit_lim;
+    SearchCut cut;
+    search_cut(windows, n_windows, minlen, maxlen - 1, 0, lim, cut);
+    // ---- staging: [GatherArgs of every archive | descriptors | lengths] once, then the region table per launch
+    const size_t ga_bytes = sizeof(GatherArgs) * (size_t)n_archives;
+    const size_t desc_off = align_up(ga_bytes, 16), desc_bytes = sizeof(u16) * (size_t)n_patterns * 2 * SRCH_MAXLEN;
+    const size_t tab_bytes = align_up(desc_off + desc_bytes + (size_t)n_patterns, 16);
+    const size_t reg_bytes = sizeof(u32) * (6 * cut.max_reg + 1);
+    SCCG_TRY(ext_staging(c, tab_bytes + reg_bytes));
+    u8* h = (u8*)c->h_ext;
+    search_stage_archives(c, archives, n_archives, (GatherArgs*)h);
+    u16* h_desc = (u16*)(h + desc_off);
+    u8* h_len = h + desc_off + desc_bytes;
+    for (i64 i = 0; i < n_patterns; ++i) {
+        h_len[i] = (u8)(pattern_off[i + 1] - pattern_off[i]);
+        search_stage_desc((const u8*)patterns + pattern_off[i], h_len[i], h_desc + i * 2 * SRCH_MAXLEN);
+    }
+    u8* d_tab = nullptr; u32* d_reg = nullptr;
+    SCCG_TRY(buf(c, B_SRCH_TAB, tab_bytes, &d_tab));
+    SCCG_TRY(buf(c, B_SRCH_REG, 6 * cut.max_reg + 1, &d_reg));
+    SCCG_CK(cudaEventRecord(c->ev[4], c->stream));
+    SCCG_CK(cudaMemcpyAsync(d_tab, h, tab_bytes, cudaMemcpyHostToDevice, c->stream));
+    SrchArgs sa;
+    sa.x.g = (const GatherArgs*)d_tab; sa.x.out = nullptr; sa.x.lane_min = ext_lane_min(); sa.x.err = nullptr;
+    sa.desc = (const u16*)(d_tab + desc_off); sa.plen = d_tab + desc_off + desc_bytes;
+    sa.n_pat = (int)n_patterns; sa.strands = strands; sa.kmax = max_mismatches; sa.maxlen = (u32)maxlen;
+    return search_launches(c, cut, (u32*)(h + tab_bytes), d_reg, sa, hits, hits_cap, n_hits);
 }
 
 }  // namespace sccg

@@ -18,12 +18,14 @@
 // ">archive_stem::name:start-end" (with "(-)" appended for the minus strand, `bedtools getfasta -s` style); BED column 6 ("+",
 // "-" or "."; absent means "+") sets the strand, and a minus-strand record holds the reverse complement.
 //
-// Additive: `decompress --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K] [--strand both|+|-]
+// Additive: `decompress --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K | --edits K] [--strand both|+|-]
 // <reference_file> <output_folder>` finds every occurrence of the FASTA patterns (name: the header up to the first whitespace;
 // 1 to 64 bytes each) with at most K mismatches (default 0) in every BED region of every archive, or in each archive's whole
 // sequence without --regions (sccg_archive_search; archives unpacked and opened as above).  <output_folder>/hits.bed holds one
 // line per hit, "archive_stem<TAB>start<TAB>end<TAB>pattern_name<TAB>mismatches<TAB>+|-", archive by archive in list order and
-// in the library's (window, position, pattern, strand) order.
+// in the library's (window, position, pattern, strand) order.  With `--edits K` instead of --mismatches (not both) insertions
+// and deletions count too: every end of an alignment within K edits (sccg_archive_search_edits), one line per hit with its
+// start, end and edit count in the fifth column, in (window, end, pattern, strand) order.
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
@@ -308,13 +310,17 @@ static bool parse_patterns(const std::string& text, std::vector<Pattern>* out, s
 static int search_archives(int argc, char* argv[]) {
     const char *pat_path = argv[2], *list_path = nullptr, *bed_path = nullptr;
     int k = 0, strands = 3;
+    bool by_mm = false, by_edits = false;
     int i = 3;
     for (; i + 1 < argc - 2; i += 2) {
         const std::string opt = argv[i], v = argv[i + 1];
         if (opt == "--archives") list_path = argv[i + 1];
         else if (opt == "--regions") bed_path = argv[i + 1];
-        else if (opt == "--mismatches") {
-            if (v.empty() || v.size() > 2 || v.find_first_not_of("0123456789") != std::string::npos) { std::cerr << "Error: bad mismatch count " << v << "\n"; return 1; }
+        else if (opt == "--mismatches" || opt == "--edits") {
+            const bool edits = opt == "--edits";
+            if (v.empty() || v.size() > 2 || v.find_first_not_of("0123456789") != std::string::npos) { std::cerr << "Error: bad " << (edits ? "edit" : "mismatch") << " count " << v << "\n"; return 1; }
+            (edits ? by_edits : by_mm) = true;
+            if (by_edits && by_mm) { std::cerr << "Error: --edits and --mismatches exclude each other\n"; return 1; }
             k = std::stoi(v);
         } else if (opt == "--strand") {
             if (v != "both" && v != "+" && v != "-") { std::cerr << "Error: --strand takes both, + or -\n"; return 1; }
@@ -329,7 +335,7 @@ static int search_archives(int argc, char* argv[]) {
     if (!parse_patterns(pat_text, &pats, &err)) { std::cerr << "Error: " << err << "\n"; return 1; }
     int64_t minlen = 64;
     for (const Pattern& p : pats) minlen = (int64_t)p.seq.size() < minlen ? (int64_t)p.seq.size() : minlen;
-    if (k >= minlen) { std::cerr << "Error: the mismatch count must be below the shortest pattern's length (" << minlen << ")\n"; return 1; }
+    if (k >= minlen) { std::cerr << "Error: the " << (by_edits ? "edit" : "mismatch") << " count must be below the shortest pattern's length (" << minlen << ")\n"; return 1; }
     std::vector<BedRegion> bed;
     if (bed_path) {
         std::string bed_text;
@@ -364,7 +370,27 @@ static int search_archives(int argc, char* argv[]) {
         std::string blob;
         std::vector<int64_t> off(1, 0);
         for (const Pattern& p : pats) { blob += p.seq; off.push_back((int64_t)blob.size()); }
+        std::vector<std::string> stems;
+        for (const std::string& arc : arcs) stems.push_back(fs::path(arc).stem().string());
+        auto line = [&](int64_t w, int64_t start, int64_t end, int32_t i, int32_t d, int32_t strand) {
+            text += stems[win_arc[(size_t)w]] + "\t" + std::to_string(start) + "\t" + std::to_string(end) + "\t" + pats[(size_t)i].name + "\t" +
+                    std::to_string(d) + (strand ? "\t-\n" : "\t+\n");
+        };
         int64_t n = 0;
+        if (by_edits) {
+            std::vector<sccg_edit_hit> hits;
+            int rc = sccg_archive_search_edits(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), blob.data(), off.data(),
+                                               (int64_t)pats.size(), k, strands, nullptr, 0, &n);
+            if (rc == SCCG_OK && n > 0) {
+                hits.resize((size_t)n);
+                rc = sccg_archive_search_edits(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), blob.data(), off.data(),
+                                               (int64_t)pats.size(), k, strands, hits.data(), n, &n);
+            }
+            if (rc != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
+            for (const sccg_edit_hit& h : hits) line(h.window, h.start, h.end, h.pattern, h.edits, h.strand);
+            status = 0;
+            return;
+        }
         std::vector<sccg_hit> hits;
         int rc = sccg_archive_search(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), blob.data(), off.data(), (int64_t)pats.size(),
                                      k, strands, nullptr, 0, &n);
@@ -374,12 +400,7 @@ static int search_archives(int argc, char* argv[]) {
                                      k, strands, hits.data(), n, &n);
         }
         if (rc != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
-        std::vector<std::string> stems;
-        for (const std::string& arc : arcs) stems.push_back(fs::path(arc).stem().string());
-        for (const sccg_hit& h : hits) {
-            text += stems[win_arc[(size_t)h.window]] + "\t" + std::to_string(h.pos) + "\t" + std::to_string(h.pos + (int64_t)pats[(size_t)h.pattern].seq.size()) +
-                    "\t" + pats[(size_t)h.pattern].name + "\t" + std::to_string(h.mismatches) + (h.strand ? "\t-\n" : "\t+\n");
-        }
+        for (const sccg_hit& h : hits) line(h.window, h.pos, h.pos + (int64_t)pats[(size_t)h.pattern].seq.size(), h.pattern, h.mismatches, h.strand);
         status = 0;
     }();
     sccg_destroy(ctx);                                                      // (releases the archives)
@@ -398,7 +419,7 @@ int main(int argc, char* argv[]) {
                   << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n"
                   << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --regions <regions.bed> --archives <list of .7z files, one per line> <reference_file> <output_folder>\n"
-                  << "       " << argv[0] << " --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K] [--strand both|+|-] <reference_file> <output_folder>\n";
+                  << "       " << argv[0] << " --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K | --edits K] [--strand both|+|-] <reference_file> <output_folder>\n";
         return 1;
     }
     try {
