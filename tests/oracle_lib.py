@@ -138,12 +138,16 @@ def orc_parse_target_fasta(data: bytes) -> tuple[bytes, bytes]:
     return _take(lib.orc_free, out, n.value), _take(lib.orc_free, h, nh.value)
 
 
-def split_intermediate(data: bytes) -> tuple[bytes, bytes, bytes, bytes]:
-    """decompress_genome's line split (decompression.cpp:66-101): -> (header, lowercase, nline, body)."""
+def split_intermediate(data: bytes) -> tuple[bytes, bytes, bytes, bytes] | None:
+    """decompress_genome's line split (decompression.cpp:66-101): -> (header, lowercase, nline, body), or None when a
+    getline fails.  getline extracts a line while input remains, so a final '\n' ends the last line without starting
+    another: '>x\\n(3,12)\\n,\\n' has no body line."""
     lines = data.split(b"\n")
+    if data.endswith(b"\n") or not data:
+        lines.pop()
     if data.startswith(b">"):
-        return lines[0], lines[1], lines[2], lines[3]
-    return b"", lines[0], lines[1], lines[2]
+        return (lines[0], lines[1], lines[2], lines[3]) if len(lines) >= 4 else None
+    return (b"", lines[0], lines[1], lines[2]) if len(lines) >= 3 else None
 
 
 def prepare_reference(ref_raw: bytes, nline: bytes) -> bytes:
@@ -154,8 +158,12 @@ def prepare_reference(ref_raw: bytes, nline: bytes) -> bytes:
 
 
 def orc_decompress(ref_raw: bytes, intermediate: bytes) -> tuple[int, bytes]:
-    """reference `decompress` minus 7z and file I/O: -> (rc, reconstructed_genome.fa bytes)."""
-    header, low, nline, body = split_intermediate(intermediate)
+    """reference `decompress` minus 7z and file I/O: -> (rc, reconstructed_genome.fa bytes).  A file getline cannot split
+    fails with rc 1, as a malformed record stream does."""
+    lines = split_intermediate(intermediate)
+    if lines is None:
+        return 1, b""
+    header, low, nline, body = lines
     rc, text = orc_reconstruct(prepare_reference(ref_raw, nline), body, b"" if nline == b"," else nline, low)
     return rc, header + b"\n" + text
 

@@ -265,9 +265,9 @@ def check_argument_errors(ctx, ctx2):
     ctx.clear_reference()
 
 
-def check_complement_table(ctx):
-    """every byte value D can hold through the minus strand: the reference holds every byte but '\n' (which D cannot hold;
-    tokens copy them, upper-cased), literals add IUPAC codes and other bytes in both cases, a lowercase run lowers a stretch"""
+def every_byte_archive():
+    """the reference holds every byte but '\n' (which D cannot hold; tokens copy them, upper-cased), literals add IUPAC
+    codes and other bytes in both cases, a lowercase run lowers a stretch -> (ref, intermediate, D)"""
     ref = bytes(b for b in range(256) if b != 10) * 8
     lits = bytes(b for b in range(256) if b not in b"()\n,-0123456789")
     body = b"(0,2040)" + lits + b"(500,300)acgtrykmbvdhswnACGTRYKMBVDHSWN"
@@ -276,11 +276,40 @@ def check_complement_table(ctx):
     assert rc == 0
     D = seq_of(image)
     assert set(D) == set(range(256)) - {10}
+    return ref, inter, D
+
+
+def check_complement_table(ctx):
+    """every byte value D can hold through the minus strand (every_byte_archive)"""
+    ref, inter, D = every_byte_archive()
     ctx.set_reference(ref)
     with ctx.open_archive(inter) as a:
         assert a.seq_len == len(D)
         for path in PATHS:
             check_query(ctx, [a], [D], [(0, 0, len(D), 1), (0, 0, len(D), 0)] + [(0, i, i + 1, 1) for i in range(len(D))], path)
+    ctx.clear_reference()
+
+
+def check_no_body_line(ctx):
+    """a file whose last line is the N line (the compressor writes one when the record body is empty; the last '\n' ends a
+    line and starts none) has no body line for getline: the oracle, decompress, decompress_resident and open_archive all
+    refuse it with the same code"""
+    ref = b"GGGACGTACGTACGTTT"
+    files = [b">x\n(3,12)\n,\n", b"(3,12)\n,\n", b">x\n\n,"]
+    rc, inter, mode = ol.orc_compress(ref, b"ACGTNNNNACGTACG", b">x")
+    assert rc == 0 and ol.split_intermediate(inter) is None
+    assert ctx.compress(ref, b"ACGTNNNNACGTACG", b">x") == (inter, mode)
+    files.append(inter)
+    ctx.set_reference(ref)
+    for f in files:
+        assert ol.split_intermediate(f) is None and ol.orc_decompress(ref, f)[0] != 0, f
+        for call in (lambda: ctx.decompress(ref, f), lambda: ctx.decompress_resident(f), lambda: ctx.open_archive(f)):
+            with pytest.raises(sccg_b200.SccgError) as e:
+                call()
+            assert e.value.code == sccg_b200.SCCG_E_FORMAT, (f, str(e.value))
+    # one more '\n' gives an empty body line: an empty D
+    rc, image = ol.orc_decompress(ref, b">x\n\n,\n\n")
+    assert rc == 0 and seq_of(image) == b"" and ctx.decompress(ref, b">x\n\n,\n\n") == image
     ctx.clear_reference()
 
 
@@ -315,3 +344,7 @@ def test_argument_errors(ctx):
 
 def test_complement_table(ctx):
     check_complement_table(ctx)
+
+
+def test_no_body_line(ctx):
+    check_no_body_line(ctx)

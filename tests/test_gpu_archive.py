@@ -6,7 +6,7 @@ import pytest
 
 import sccg_b200
 from test_emu_archive import (COMP, check_argument_errors, check_complement_table, check_golden_archives, check_lifetime,
-                              check_many_archives, check_reference_generation, expect)
+                              check_many_archives, check_no_body_line, check_reference_generation, expect)
 
 pytestmark = pytest.mark.gpu
 
@@ -46,6 +46,10 @@ def test_argument_errors(ctx):
 
 def test_complement_table(ctx):
     check_complement_table(ctx)
+
+
+def test_no_body_line(ctx):
+    check_no_body_line(ctx)
 
 
 def expect_np(Ds, q):
