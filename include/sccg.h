@@ -256,6 +256,43 @@ int sccg_archive_search_edits(sccg_ctx* ctx, sccg_archive* const* archives, int6
                               const char* patterns, const int64_t* pattern_off, int64_t n_patterns, int max_edits, int strands,
                               sccg_edit_hit* hits, int64_t hits_cap, int64_t* n_hits);
 
+/* Differences of open archives from the resident reference, as normalised variant records.  R is the raw resident reference
+ * (the bytes given to sccg_reference_set), D an archive's decoded sequence (as for sccg_archive_extract), up() ASCII
+ * upper-casing of a-z; every comparison is on up() bytes, so lowercase is never a difference.  A record says that
+ * up(R[pos:end]) is replaced by up(D[d_start:d_end]); its ALT bytes, exactly up(D[d_start:d_end]), are at alt + alt_off.
+ * The records of an archive are a function of its record file and R alone:
+ *  1. copy pieces: the decoder's token segments in D order, each (x, p, l) with up(D[x:x+l]) == up(R[p:p+l]) in raw
+ *     coordinates (global mode: split wherever D skips a target N run or R skips a reference N run); literal runs and
+ *     pieces with l = 0 are not pieces;
+ *  2. anchors: with M = the maximum of p + l over all earlier pieces (0 at the start), piece (x, p, l) clipped at its start
+ *     by s = max(0, M - p) is the anchor (x + s, p + s, l - s) when s < l.  Anchors increase strictly in D and in R;
+ *  3. gaps: between consecutive anchors, before the first (from (0, 0)) and after the last (to (len(D), len(R))), the
+ *     reference gap G_R and the D gap G_D.  Equal lengths: one substitution record per maximal run of differing positions.
+ *     Different lengths: trim the longest common suffix, then the longest common prefix of what is left; both sides still
+ *     non-empty make one complex record, otherwise one insertion (end == pos) or deletion (d_end == d_start);
+ *  4. left-alignment: each insertion and deletion moves left one base at a time (pos, end, d_start and d_end decrease by
+ *     1) while pos is greater than the end the previous record had at step 3 (0 for the first) and up(R[pos - 1]) equals
+ *     the last byte of the allele (R[end - 1] for a deletion, the last ALT byte for an insertion): bcftools norm's
+ *     left-alignment, bounded by the previous record, so records never overlap;
+ *  5. windows: window w = {archive, start, end} is in REFERENCE coordinates (0 <= start <= end <= len(R)) and returns the
+ *     records of its archive whose pos lies in [start, end) (a window that ends at len(R) also takes the insertions at
+ *     pos = len(R)), each with window = w.  A window filters the records of the
+ *     whole archive and never changes one; overlapping and repeated windows each report theirs.
+ * Records come in (window, pos, d_start) order.  Per archive: pos_j >= end_{j-1} and d_start_j >= d_end_{j-1}, the stretches
+ * between records are equally long and equal under up(), a substitution differs at every position, other records differ
+ * in their first and in their last byte unless a side is empty, and splicing the ALTs into up(R) gives up(D).
+ * Not done: realignment (the records are a faithful account of the encoding: permuted blocks appear as large complex
+ * records), splitting complex records or MNPs (bcftools norm -a), genotypes or phasing, liftover of coordinates.
+ * *n_vars and *alt_len always receive the totals.  vars == NULL counts only.  When either cap is too small the call returns
+ * SCCG_E_ARG with both totals set.  Errors, all SCCG_E_ARG and all before any device work, in this order: a NULL pointer with
+ * a non-zero count or a negative count (2^31 or more archives or windows, a negative cap); then for each window the archive
+ * checks of sccg_archive_extract (index out of range, NULL archive, another context, a replaced or cleared resident
+ * reference), start < 0 or start > end, end > len(R); then the caps.  Profile: h2d_ms (archive and window tables), gather_ms
+ * (variant kernels), kernels_ms, d2h_ms (records and ALT bytes), launches. */
+typedef struct { int64_t window, pos, end, d_start, d_end, alt_off; } sccg_variant;
+int sccg_archive_variants(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
+                          sccg_variant* vars, int64_t vars_cap, int64_t* n_vars, char* alt, int64_t alt_cap, int64_t* alt_len);
+
 /* FASTA file images in: read_genomes_from_files (compression.cpp:181-220) and the reference reader of decompress_genome
  * (decompression.cpp:47-58) run on the device -- header lines skipped ('>' at a line start; in the target only the first one,
  * which becomes the header line of the output), isspace() bytes removed -- followed by sccg_compress / sccg_decompress.

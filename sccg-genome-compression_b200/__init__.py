@@ -142,6 +142,7 @@ def load_library(path: str | os.PathLike | None = None) -> C.CDLL:
     lib.sccg_archive_extract.argtypes = [vp, vp, i64, vp, i64, vp, i64, i64p]
     lib.sccg_archive_search.argtypes = [vp, vp, i64, vp, i64, cp, vp, i64, C.c_int, C.c_int, vp, i64, i64p]
     lib.sccg_archive_search_edits.argtypes = [vp, vp, i64, vp, i64, cp, vp, i64, C.c_int, C.c_int, vp, i64, i64p]
+    lib.sccg_archive_variants.argtypes = [vp, vp, i64, vp, i64, vp, i64, i64p, vp, i64, i64p]
     lib.sccg_mgpu_unique_id.argtypes = [C.c_char_p]
     lib.sccg_mgpu_init.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.POINTER(vp)]
     lib.sccg_mgpu_destroy.argtypes = [vp]
@@ -294,6 +295,7 @@ class Context:
     def __init__(self, device: int = 0, lib_path: str | os.PathLike | None = None):
         self.lib = load_library(lib_path)
         self._archives: set[Archive] = set()
+        self.ref_len = 0                            # len(R) of the resident reference (set_reference)
         self.handle = self.lib.sccg_create(device)
         if not self.handle:
             raise SccgError(SCCG_E_CUDA, self.lib.sccg_last_error().decode())
@@ -415,9 +417,11 @@ class Context:
     def set_reference(self, ref) -> None:
         """ref: bytes or a C-contiguous uint8 numpy array (raw symbols, as read_genomes_from_files yields them)"""
         self._check(self.lib.sccg_reference_set(self.handle, _as_char_p(ref), len(ref)))
+        self.ref_len = len(ref)
 
     def clear_reference(self) -> None:
         self._check(self.lib.sccg_reference_clear(self.handle))
+        self.ref_len = 0
 
     def compress_resident(self, tgt, header: bytes = b"", out_ptr: int = 0, out_cap: int = 0):
         """compress against the resident reference -> (file image, mode); with out_ptr / out_cap the image is written into
@@ -658,6 +662,41 @@ class Context:
         h = buf[:n.value]
         return np.stack([h["window"], h["start"], h["end"], h["pattern"].astype(np.int64), h["strand"].astype(np.int64),
                          h["edits"].astype(np.int64)], axis=1).reshape(-1, 6)
+
+    _VARIANT = [("window", "<i8"), ("pos", "<i8"), ("end", "<i8"), ("d_start", "<i8"), ("d_end", "<i8"), ("alt_off", "<i8")]
+
+    def variants(self, archives, windows=None, count_only: bool = False):
+        """differences of open archives from the resident reference as normalised variant records (sccg_archive_variants,
+        include/sccg.h).  windows: an (n, 3) int64 array of [archive index, start, end] in REFERENCE coordinates, passed
+        straight through; None takes the whole reference for each archive, in order.  -> (records, alt): records an (n, 6)
+        int64 array of [window, pos, end, d_start, d_end, alt_off] in (window, pos, d_start) order, alt the ALT bytes (record
+        i's are alt[alt_off:alt_off + d_end - d_start]); or (number of records, ALT bytes) when count_only.  The buffers start
+        at 65,536 records and 1 MiB; a call that needs more runs once more with the exact sizes it reported."""
+        import numpy as np
+        if windows is None:
+            windows = [(k, 0, self.ref_len) for k in range(len(archives))]
+        w = np.ascontiguousarray(np.asarray(windows, dtype=np.int64).reshape(-1, 3))      # sccg_window[] layout
+        arr = (C.c_void_p * max(len(archives), 1))(*[a.handle for a in archives])
+        n = C.c_int64(-1); na = C.c_int64(-1)
+
+        def run(out, cap, alt, alt_cap):
+            return self.lib.sccg_archive_variants(self.handle, arr if len(archives) else None, len(archives), w.ctypes.data if len(w) else None,
+                                                  len(w), out, cap, C.byref(n), alt, alt_cap, C.byref(na))
+        if count_only:
+            self._check(run(None, 0, None, 0))
+            return n.value, na.value
+        caps = (65536, 1 << 20)
+        for _ in range(2):
+            buf = np.zeros(caps[0], dtype=self._VARIANT)
+            alt = C.create_string_buffer(max(caps[1], 1))
+            rc = run(buf.ctypes.data if len(buf) else None, len(buf), C.cast(alt, C.c_void_p), caps[1])
+            if rc == SCCG_OK or not (rc == SCCG_E_ARG and (n.value > caps[0] or na.value > caps[1])):
+                break
+            caps = (n.value, na.value)
+        self._check(rc)
+        v = buf[:n.value]
+        rec = np.stack([v[f] for f, _ in self._VARIANT], axis=1).reshape(-1, 6).astype(np.int64)
+        return rec, alt.raw[:na.value]
 
     # decompress_genome (in-memory part) + reconstruct_genome + header line (decompression.cpp:66-110, :117-279, :322)
     def decompress(self, ref_raw: bytes, intermediate: bytes) -> bytes:

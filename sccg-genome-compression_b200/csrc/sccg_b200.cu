@@ -6,6 +6,7 @@
 #include "sccg_extract.cuh"
 #include "sccg_search.cuh"
 #include "sccg_search_edit.cuh"
+#include "sccg_variants.cuh"
 #include "sccg_fasta.cuh"
 #include "sccg_shard.cuh"
 #include "sccg_mgpu.cuh"
@@ -95,6 +96,7 @@ void sccg_destroy(sccg_ctx* c) {
     if (c->res_ref) cudaFree(c->res_ref);
     while (c->archives) { sccg_archive* a = c->archives; archive_unlink(c, a); archive_free(a); }
     for (int f = 0; f < 2; ++f) if (c->res_form[f]) cudaFree(c->res_form[f]);
+    if (c->res_nrun) cudaFree(c->res_nrun);
     for (int i = 0; i < 8; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
     for (int i = 0; i < 4; ++i) if (c->ev_x[i]) cudaEventDestroy(c->ev_x[i]);
     if (c->main_stream) cudaStreamDestroy(c->main_stream);
@@ -604,6 +606,16 @@ int sccg_archive_search_edits(sccg_ctx* c, sccg_archive* const* archives, int64_
     const int rc = archive_search_edits_impl(c, archives, n_archives, windows, n_windows, patterns, pattern_off, n_patterns, max_edits,
                                              strands, hits, hits_cap, n_hits);
     if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
+    return rc;
+}
+
+int sccg_archive_variants(sccg_ctx* c, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
+                          sccg_variant* vars, int64_t vars_cap, int64_t* n_vars, char* alt, int64_t alt_cap, int64_t* alt_len) {
+    if (!c) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    const int rc = archive_variants_impl(c, archives, n_archives, windows, n_windows, vars, vars_cap, n_vars, alt, alt_cap, alt_len);
+    if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffers stays in flight
     return rc;
 }
 

@@ -33,6 +33,7 @@ enum Slot {
     B_LRUN_S, B_LRUN_E, B_NRUNS_S, B_NRUNS_E, B_NRUNS_CUM, B_TILE0, B_TILE1, B_TILE2, B_TILE3, B_SEG_PTR, B_TILE_WIN, B_FILE_R, B_FILE_T, B_FA_TMP, B_FA_RNG, B_NEED,
     B_GREF, B_GTGT, B_GKEYS, B_GVALS, B_GKEYS2, B_GVALS2, B_GHIST, B_GOFFS, B_GBUCKET, B_GREC, B_GLIT, B_GTMP0, B_GTMP1, B_GTMP2, B_GTMP3, B_GFIRST, B_SHARD,
     B_EXT_REG, B_EXT_IV, B_SRCH_TAB, B_SRCH_REG, B_SRCH_TILE, B_SRCH_HITS,
+    B_VR_AGG, B_VR_SC, B_VR_TAB, B_VR_KEY, B_VR_CNT, B_VR_ANC, B_VR_GAP, B_VR_TILE, B_VR_REC3, B_VR_P, B_VR_WIN, B_VR_OUT,
     B_NSLOTS
 };
 
@@ -72,6 +73,7 @@ struct sccg_ctx {
     unsigned char* res_form[2]; long long res_form_len[2];   // the resident reference as archives read it: [0] upper-cased (local-mode
                                                               // files), [1] N-stripped and upper-cased (global mode); built at first need
     sccg_archive* archives;          // open archives (sccg_destroy releases them)
+    void* res_nrun; long long res_nrun_k;   // the resident reference's N runs for sccg_archive_variants (sccg_variants.cuh), built at first need
 };
 
 namespace sccg {

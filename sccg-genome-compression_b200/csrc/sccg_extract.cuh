@@ -567,6 +567,8 @@ static void reference_changed(sccg_ctx* c) {
         if (c->res_form[f]) { cudaStreamSynchronize(c->main_stream); cudaFree(c->res_form[f]); }
         c->res_form[f] = nullptr; c->res_form_len[f] = 0;
     }
+    if (c->res_nrun) { cudaStreamSynchronize(c->main_stream); cudaFree(c->res_nrun); }
+    c->res_nrun = nullptr; c->res_nrun_k = 0;
 }
 
 static void archive_free(sccg_archive* a) {

@@ -26,9 +26,22 @@
 // in the library's (window, position, pattern, strand) order.  With `--edits K` instead of --mismatches (not both) insertions
 // and deletions count too: every end of an alignment within K edits (sccg_archive_search_edits), one line per hit with its
 // start, end and edit count in the fifth column, in (window, end, pattern, strand) order.
+//
+// Additive: `decompress --variants --archives <list> [--regions <bed>] <reference_file> <output_folder>` reports how every
+// archive of <list> differs from the reference (sccg_archive_variants; archives unpacked and opened as above), in the whole
+// reference or in the BED regions (reference coordinates).  <output_folder>/variants.vcf is VCF 4.2:
+//   ##fileformat=VCFv4.2, ##contig=<ID=CHROM,length=len(R)>, a GT ##FORMAT line, then the header line
+//   #CHROM POS ID REF ALT QUAL FILTER INFO FORMAT <one haploid sample column per archive: its stem, as in hits.bed>.
+// CHROM is the first word of the reference FASTA's first header line (the file stem when there is none).  One row per
+// distinct (POS, REF, ALT) over all archives, GT 1 for the archives that carry it and 0 for the others, sorted by POS, then
+// by the REF and ALT bytes; a record in several regions appears once.  REF is up(R[pos:end]) and ALT the record's ALT bytes
+// at POS = pos + 1; an insertion or deletion is padded with the preceding reference base (POS = pos), or at pos = 0 with the
+// following one (N if neither exists); substitutions and complex records are not padded.  ID, QUAL, FILTER and INFO are '.'.
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
+#include <map>
+#include <tuple>
 
 #include "batch.hpp"
 #include "fasta_io.hpp"
@@ -409,22 +422,117 @@ static int search_archives(int argc, char* argv[]) {
     return 0;
 }
 
+// the VCF of `--variants` (format in the header comment)
+static int variants_archives(int argc, char* argv[]) {
+    const char *list_path = nullptr, *bed_path = nullptr;
+    int i = 2;
+    for (; i + 1 < argc - 2; i += 2) {
+        const std::string opt = argv[i];
+        if (opt == "--archives") list_path = argv[i + 1];
+        else if (opt == "--regions") bed_path = argv[i + 1];
+        else { std::cerr << "Error: unknown option " << opt << "\n"; return 1; }
+    }
+    if (i != argc - 2 || !list_path) { std::cerr << "Error: --variants needs --archives <list>, then <reference_file> <output_folder>\n"; return 1; }
+    const std::string ref_path = argv[argc - 2], out_dir = argv[argc - 1];
+    std::string err;
+    std::vector<BedRegion> bed;
+    if (bed_path) {
+        std::string bed_text;
+        if (!sccg_host::read_file(bed_path, bed_text)) { std::cerr << "Error opening BED file: " << bed_path << "\n"; return 1; }
+        if (!parse_bed(bed_text, &bed, &err)) { std::cerr << "Error: " << err << "\n"; return 1; }
+    }
+    std::vector<std::string> arcs;
+    if (!read_archive_list(list_path, &arcs)) return 1;
+    std::string ref_file, ref, chrom;
+    if (!sccg_host::read_file(ref_path, ref_file)) { std::cerr << "Greska pri otvaranju reference: " << ref_path << "\n"; return 1; }
+    sccg_host::parse_fasta(ref_file, false, ref, nullptr);
+    for (size_t p = 0; p < ref_file.size();) {                              // the first header line's first word
+        const size_t e = ref_file.find('\n', p);
+        const std::string line = ref_file.substr(p, e == std::string::npos ? std::string::npos : e - p);
+        if (!line.empty() && line[0] == '>') {
+            const size_t w = line.find_first_of(" \t\r", 1);
+            chrom = line.substr(1, w == std::string::npos ? std::string::npos : w - 1);
+            break;
+        }
+        if (e == std::string::npos) break;
+        p = e + 1;
+    }
+    if (chrom.empty()) chrom = fs::path(ref_path).stem().string();
+    for (const BedRegion& r : bed)
+        if (r.end > (int64_t)ref.size()) { std::cerr << "Error: region " << r.name << ":" << r.start << "-" << r.end << " ends past the end of the reference (" << ref.size() << " bp)\n"; return 1; }
+    sccg_ctx* ctx = resident_context(ref_path);
+    if (!ctx) return 1;
+    std::error_code ec;
+    if (!fs::exists(out_dir)) fs::create_directory(out_dir, ec);
+    int status = 1;
+    std::vector<sccg_archive*> open;
+    std::vector<sccg_window> wins;
+    std::string text;
+    [&] {
+        for (const std::string& arc : arcs) {                               // unpacked one at a time: archives may share a file name
+            sccg_archive* a = open_archive_file(ctx, arc, out_dir);
+            if (!a) return;
+            open.push_back(a);
+            const int64_t ai = (int64_t)open.size() - 1;
+            if (!bed_path) wins.push_back(sccg_window{ai, 0, (int64_t)ref.size()});
+            for (const BedRegion& r : bed) wins.push_back(sccg_window{ai, r.start, r.end});
+        }
+        int64_t n = 0, na = 0;
+        int rc = sccg_archive_variants(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), nullptr, 0, &n, nullptr, 0, &na);
+        std::vector<sccg_variant> vars((size_t)n);
+        std::vector<char> alt((size_t)na + 1);
+        if (rc == SCCG_OK && n > 0) rc = sccg_archive_variants(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), vars.data(), n, &n, alt.data(), na, &na);
+        if (rc != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
+        auto up = [](char ch) { return (ch >= 'a' && ch <= 'z') ? (char)(ch - 32) : ch; };
+        std::map<std::tuple<int64_t, std::string, std::string>, std::vector<char>> rows;
+        for (const sccg_variant& v : vars) {
+            std::string r, a(alt.data() + v.alt_off, (size_t)(v.d_end - v.d_start));
+            for (int64_t q = v.pos; q < v.end; ++q) r += up(ref[(size_t)q]);
+            int64_t pos = v.pos + 1;
+            if (r.empty() || a.empty()) {
+                if (v.pos > 0) { const char b = up(ref[(size_t)v.pos - 1]); r = b + r; a = b + a; pos = v.pos; }
+                else { const char b = v.end < (int64_t)ref.size() ? up(ref[(size_t)v.end]) : 'N'; r += b; a += b; }
+            }
+            std::vector<char>& gt = rows[std::make_tuple(pos, r, a)];
+            gt.resize(open.size(), 0);
+            gt[(size_t)wins[(size_t)v.window].archive] = 1;
+        }
+        text = "##fileformat=VCFv4.2\n##contig=<ID=" + chrom + ",length=" + std::to_string(ref.size()) + ">\n"
+               "##FORMAT=<ID=GT,Number=1,Type=String,Description=\"Genotype\">\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT";
+        for (const std::string& arc : arcs) text += "\t" + fs::path(arc).stem().string();
+        text += "\n";
+        for (const auto& row : rows) {
+            text += chrom + "\t" + std::to_string(std::get<0>(row.first)) + "\t.\t" + std::get<1>(row.first) + "\t" + std::get<2>(row.first) + "\t.\t.\t.\tGT";
+            for (char g : row.second) text += g ? "\t1" : "\t0";
+            text += "\n";
+        }
+        status = 0;
+    }();
+    sccg_destroy(ctx);                                                      // (releases the archives)
+    if (status) return status;
+    if (!write_output(out_dir + "/variants.vcf", text)) { std::cerr << "Error opening output file: " << out_dir << "\n"; return 1; }
+    return 0;
+}
+
 int main(int argc, char* argv[]) {
     const bool batch = argc >= 3 && std::string(argv[1]) == "--batch";
     const bool regions = argc == 6 && std::string(argv[1]) == "--regions";
     const bool archives = argc == 7 && std::string(argv[1]) == "--regions" && std::string(argv[3]) == "--archives";
     const bool search = argc >= 7 && std::string(argv[1]) == "--search";
-    if (argc != 4 && !batch && !regions && !archives && !search) {          // decompression.cpp:283-286
+    const bool variants = argc >= 6 && std::string(argv[1]) == "--variants";
+    if (argc != 4 && !batch && !regions && !archives && !search && !variants) {          // decompression.cpp:283-286
         std::cerr << "Usage: " << argv[0] << " <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n"
                   << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --regions <regions.bed> --archives <list of .7z files, one per line> <reference_file> <output_folder>\n"
-                  << "       " << argv[0] << " --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K | --edits K] [--strand both|+|-] <reference_file> <output_folder>\n";
+                  << "       " << argv[0] << " --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K | --edits K] [--strand both|+|-] <reference_file> <output_folder>\n"
+                  << "       " << argv[0] << " --variants --archives <list> [--regions <bed>] <reference_file> <output_folder>\n";
         return 1;
     }
     try {
         if (archives) return extract_archives(argv[2], argv[4], argv[5], argv[6]);
         if (search) return search_archives(argc, argv);
+        if (variants) return variants_archives(argc, argv);
         if (regions) {
             Job job; job.a = argv[3]; job.b = argv[4]; job.out = argv[5];
             return extract_regions(argv[2], job);
