@@ -37,6 +37,8 @@
 // by the REF and ALT bytes; a record in several regions appears once.  REF is up(R[pos:end]) and ALT the record's ALT bytes
 // at POS = pos + 1; an insertion or deletion is padded with the preceding reference base (POS = pos), or at pos = 0 with the
 // following one (N if neither exists); substitutions and complex records are not padded.  ID, QUAL, FILTER and INFO are '.'.
+// REF and ALT hold ASCII letters only (IUPAC codes included): when a record's REF or ALT would hold any other byte (D and R
+// may hold any byte but '\n'), the command names the record's position, exits 1 and writes no variants.vcf.
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
@@ -484,6 +486,10 @@ static int variants_archives(int argc, char* argv[]) {
         if (rc == SCCG_OK && n > 0) rc = sccg_archive_variants(ctx, open.data(), (int64_t)open.size(), wins.data(), (int64_t)wins.size(), vars.data(), n, &n, alt.data(), na, &na);
         if (rc != SCCG_OK) { std::cerr << "Error: " << sccg_last_error() << "\n"; return; }
         auto up = [](char ch) { return (ch >= 'a' && ch <= 'z') ? (char)(ch - 32) : ch; };
+        auto letters = [](const std::string& s) {
+            for (char ch : s) if (!((ch >= 'A' && ch <= 'Z') || (ch >= 'a' && ch <= 'z'))) return false;
+            return true;
+        };
         std::map<std::tuple<int64_t, std::string, std::string>, std::vector<char>> rows;
         for (const sccg_variant& v : vars) {
             std::string r, a(alt.data() + v.alt_off, (size_t)(v.d_end - v.d_start));
@@ -492,6 +498,11 @@ static int variants_archives(int argc, char* argv[]) {
             if (r.empty() || a.empty()) {
                 if (v.pos > 0) { const char b = up(ref[(size_t)v.pos - 1]); r = b + r; a = b + a; pos = v.pos; }
                 else { const char b = v.end < (int64_t)ref.size() ? up(ref[(size_t)v.end]) : 'N'; r += b; a += b; }
+            }
+            if (!letters(r) || !letters(a)) {                                 // a tab, ',' or control byte would corrupt the row
+                std::cerr << "Error: the record at reference position " << v.pos + 1 << " of " << fs::path(arcs[(size_t)wins[(size_t)v.window].archive]).stem().string()
+                          << " has REF or ALT bytes that are not ASCII letters; VCF cannot hold them\n";
+                return;
             }
             std::vector<char>& gt = rows[std::make_tuple(pos, r, a)];
             gt.resize(open.size(), 0);

@@ -88,3 +88,70 @@ def test_variants_archives(env, tmp_path):  # noqa: F811
     out = tmp_path / "errref"
     r = run(env, BIN / "decompress", "--variants", *good, tmp_path / "nope.fa", out)
     assert r.returncode == 1 and not (out / "variants.vcf").exists()
+
+
+def hand_archive(env, d, name: str, inter: bytes):  # noqa: F811
+    """a record file written by hand, packed as <name>.txt.7z"""
+    d.mkdir(exist_ok=True)
+    (d / f"{name}.txt").write_bytes(inter)
+    r = run(env, "7z", "a", "-mx=9", d / f"{name}.txt.7z", d / f"{name}.txt")
+    assert r.returncode == 0, r.stderr
+    return d / f"{name}.txt.7z"
+
+
+def test_variants_edges(env, tmp_path):  # noqa: F811
+    """records at pos 0 (deletion, insertion, complex), an insertion at len(R), an empty target (all of R deleted), two
+    archives sharing a row, overlapping BED regions, an identical target alone (a header-only VCF); then a target whose
+    ALT bytes are not letters: exit 1 naming the position, no variants.vcf and no variants.vcf.part"""
+    from test_emu_search_space import odd_target_archive
+    from test_emu_variants import hand_file, tokens
+    from test_emu_variants_space import bases
+    R = bases(3000, 31)
+    L = len(R)
+    ol.write_fasta(tmp_path / "ref.fa", R, b">chr2 edges")
+    snp = b"T" if R[1200:1201] != b"T" else b"G"
+    files = {"del0": tokens((5, L - 5)), "ins0": b"GG" + tokens((0, L)), "cx0": b"TTTT" + tokens((2, L - 2)),
+             "insL": tokens((0, L)) + b"CC", "empty": b"", "snpA": tokens((0, 1200), snp, (1201, L - 1201)),
+             "snpB": tokens((0, 1200), snp, (1201, 1000), (2300, L - 2300))}
+    arcs, Ds, wholes = [], [], []
+    for name, body in files.items():
+        inter = hand_file(body)
+        arcs.append(hand_archive(env, tmp_path / "a", name, inter))
+        Ds.append(vl.decoded(R, inter))
+        wholes.append(vl.variants_whole(R, inter, Ds[-1]))
+    stems = [a.stem for a in arcs]
+    (tmp_path / "list.txt").write_text("".join(f"{a}\n" for a in arcs))
+    bed = [(0, 1500), (1000, L), (1100, 1300), (L - 10, L)]
+    (tmp_path / "r.bed").write_text("".join(f"chr2\t{a}\t{b}\n" for a, b in bed))
+    for j, (opts, regions) in enumerate((((), [(0, L)]), (("--regions", tmp_path / "r.bed"), bed))):
+        out = tmp_path / f"out{j}"
+        r = run(env, BIN / "decompress", "--variants", "--archives", tmp_path / "list.txt", *opts, tmp_path / "ref.fa", out)
+        assert r.returncode == 0, r.stderr
+        got = (out / "variants.vcf").read_bytes()
+        assert got == render_vcf("chr2", R, stems, Ds, wholes, regions), opts
+        rows = [l.split(b"\t") for l in got.splitlines() if not l.startswith(b"#")]
+        assert sum(1 for f in rows if f[1] == b"1") >= 3                   # three records at pos 0 (POS 1)
+        assert any(f[-2:] == [b"1", b"1"] for f in rows)                  # the SNP both snpA and snpB carry: one row
+        assert any(f[3] == vl.up(R[:L]) + b"N" for f in rows)             # the empty target: all of R deleted
+    # an identical target alone: a header-only VCF
+    (tmp_path / "same.txt").write_text(f"{hand_archive(env, tmp_path / 's', 'same', hand_file(tokens((0, L))))}\n")
+    r = run(env, BIN / "decompress", "--variants", "--archives", tmp_path / "same.txt", tmp_path / "ref.fa", tmp_path / "outs")
+    assert r.returncode == 0, r.stderr
+    got = (tmp_path / "outs" / "variants.vcf").read_bytes()
+    assert got == render_vcf("chr2", R, ["same.txt"], [R], [vl.variants_whole(R, hand_file(tokens((0, L))))], [(0, L)]) and got.count(b"\n") == 4
+    # ALT bytes that are not letters (tab, ',', control bytes, bytes >= 0x80): refused, nothing written
+    ref2, inter2, _, _, D2 = odd_target_archive()
+    ol.write_fasta(tmp_path / "ref2.fa", ref2, b">chrO")
+    (tmp_path / "odd.txt").write_text(f"{hand_archive(env, tmp_path / 'o', 'odd', inter2)}\n")
+    out = tmp_path / "outo"
+    r = run(env, BIN / "decompress", "--variants", "--archives", tmp_path / "odd.txt", tmp_path / "ref2.fa", out)
+    assert r.returncode == 1 and b"position" in r.stderr and b"letters" in r.stderr, r.stderr
+    assert not (out / "variants.vcf").exists() and not (out / "variants.vcf.part").exists()
+    # the same archive in a region of letter records only is written
+    W = vl.variants_whole(ref2, inter2, D2)
+    bad = [int(p) for p, e, s, t in W.tolist() if not all(65 <= c <= 90 for c in vl.up(D2[s:t]) + vl.up(ref2[p:e]))]
+    assert bad and bad[0] > 0
+    (tmp_path / "first.bed").write_text(f"chrO\t0\t{bad[0]}\n")
+    r = run(env, BIN / "decompress", "--variants", "--archives", tmp_path / "odd.txt", "--regions", tmp_path / "first.bed", tmp_path / "ref2.fa", out)
+    assert r.returncode == 0, r.stderr
+    assert (out / "variants.vcf").read_bytes() == render_vcf("chrO", ref2, ["odd.txt"], [D2], [W], [(0, bad[0])])

@@ -83,9 +83,8 @@ def variants_whole(ref_raw: bytes, intermediate: bytes, D: bytes | None = None) 
     return variants_from_pieces(ref_raw, D, copy_pieces(ref_raw, intermediate, D))
 
 
-def variants_from_pieces(R: bytes, D: bytes, P: np.ndarray) -> np.ndarray:
-    UR, UD = up(R), up(D)
-    # step 2: anchors
+def anchors(R: bytes, D: bytes, P: np.ndarray) -> list:
+    """step 2: the anchors [x, p, l] of the copy pieces P, then the sentinel [len(D), len(R), 0]"""
     if len(P):
         x, p, l = P[:, 0], P[:, 1], P[:, 2]
         M = np.concatenate([[0], np.maximum.accumulate(p + l)[:-1]])
@@ -94,7 +93,46 @@ def variants_from_pieces(R: bytes, D: bytes, P: np.ndarray) -> np.ndarray:
         anc = np.stack([x[a] + s[a], p[a] + s[a], l[a] - s[a]], axis=1)
     else:
         anc = np.zeros((0, 3), np.int64)
-    anc = np.concatenate([anc, [[len(D), len(R), 0]]]).tolist()
+    return np.concatenate([anc, [[len(D), len(R), 0]]]).astype(np.int64).tolist()
+
+
+def gap_layout(R: bytes, Ds: list[bytes], pieces: list[np.ndarray]) -> np.ndarray:
+    """the gap-byte space of one call over the archives with D = Ds[k] and copy pieces pieces[k], in that order: per gap
+    (goff, width, nd, nr), goff the exclusive prefix sum of width = max(nd, nr) over every gap of every archive (zero-width
+    gaps included) -> an (n, 4) int64 array"""
+    rows = []
+    for D, P in zip(Ds, pieces):
+        lx = lp = 0
+        for ax, ap, al in anchors(R, D, P):
+            rows.append((ax - lx, ap - lp))
+            lx, lp = ax + al, ap + al
+    nd = np.array([r[0] for r in rows], np.int64)
+    nr = np.array([r[1] for r in rows], np.int64)
+    w = np.maximum(nd, nr)
+    goff = np.concatenate([[0], np.cumsum(w)[:-1]]).astype(np.int64)
+    return np.stack([goff, w, nd, nr], axis=1).reshape(-1, 4)
+
+
+def record_gap_bytes(layout: np.ndarray, R: bytes, Ds: list[bytes], pieces: list[np.ndarray], whole: list[np.ndarray]):
+    """where the substitution records of whole[k] (variants_whole) fall in the gap-byte space of gap_layout, for the gaps of
+    equal length: -> (first byte, last byte) of each record's run of differences"""
+    first, last = [], []
+    g = 0
+    for D, P, W in zip(Ds, pieces, whole):
+        lx = lp = 0
+        for ax, ap, al in anchors(R, D, P):
+            if ax - lx == ap - lp:
+                for pos, end, ds, de in W[(W[:, 0] >= lp) & (W[:, 1] <= ap) & (W[:, 2] >= lx) & (W[:, 3] <= ax)].tolist():
+                    if pos - lp == ds - lx and end - pos == de - ds:
+                        first.append(int(layout[g, 0]) + pos - lp); last.append(int(layout[g, 0]) + end - lp - 1)
+            g += 1
+            lx, lp = ax + al, ap + al
+    return np.array(first, np.int64), np.array(last, np.int64)
+
+
+def variants_from_pieces(R: bytes, D: bytes, P: np.ndarray) -> np.ndarray:
+    UR, UD = up(R), up(D)
+    anc = anchors(R, D, P)                                                  # step 2
     # step 3: gaps
     recs = []
     lx = lp = 0
