@@ -282,7 +282,7 @@ int sccg_archive_search_edits(sccg_ctx* ctx, sccg_archive* const* archives, int6
  * between records are equally long and equal under up(), a substitution differs at every position, other records differ
  * in their first and in their last byte unless a side is empty, and splicing the ALTs into up(R) gives up(D).
  * Not done: realignment (the records are a faithful account of the encoding: permuted blocks appear as large complex
- * records), splitting complex records or MNPs (bcftools norm -a), genotypes or phasing, liftover of coordinates.
+ * records), splitting complex records or MNPs (bcftools norm -a), genotypes or phasing.
  * *n_vars and *alt_len always receive the totals.  vars == NULL counts only.  When either cap is too small the call returns
  * SCCG_E_ARG with both totals set.  Errors, all SCCG_E_ARG and all before any device work, in this order: a NULL pointer with
  * a non-zero count or a negative count (2^31 or more archives or windows, a negative cap); then for each window the archive
@@ -292,6 +292,46 @@ int sccg_archive_search_edits(sccg_ctx* ctx, sccg_archive* const* archives, int6
 typedef struct { int64_t window, pos, end, d_start, d_end, alt_off; } sccg_variant;
 int sccg_archive_variants(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_window* windows, int64_t n_windows,
                           sccg_variant* vars, int64_t vars_cap, int64_t* n_vars, char* alt, int64_t alt_cap, int64_t* alt_len);
+
+/* Coordinates lifted between the resident reference R and open archives D (R, D and up() as for sccg_archive_variants).
+ * The records of archive a are its whole-archive records of sccg_archive_variants after step 4, in (pos, d_start) order
+ * (windows play no part).  A record is a substitution when end - pos == d_end - d_start; otherwise it changes length.
+ * Ownership: every reference base outside all [pos, end) spans lies in a stretch and is aligned one to one with a D base;
+ * the D bases of a record, D[d_start:d_end], are owned by its pos (the rule by which a variants window reports a record).
+ * from = 0, reference -> archive: query [s, e) with 0 <= s <= e <= len(R) lifts to [F(s), F+(e)), where F(b) is the number
+ * of D bases whose owner or aligned reference base is < b, and F+(e) = F(e) except F+(len(R)) = len(D) (the end only: a
+ * window that ends at len(R) also owns the records at pos = len(R), so [len(R), len(R)) owns a trailing insertion).  In
+ * closed form, with j the last record with pos < b: F(b) = d_end_j + max(0, b - end_j), or b when there is none.
+ * from = 1, archive -> reference: the mirror image.  [x, y) with 0 <= x <= y <= len(D) lifts to [G(x), G+(y)), the roles of
+ * (pos, end) and (d_start, d_end) swapped: the reference bases of a record are owned by its d_start, and G+(len(D)) = len(R)
+ * (so deletions at the end of D belong to a window that ends there).
+ * Per query, in query order: start, end (the lifted interval; it may be empty, e.g. inside a deletion); same (source bases of
+ * the query in stretches, copied identically); subst (source bases of the query inside substitution records); records (the
+ * records the query owns: for from = 0 exactly what sccg_archive_variants reports for the window {archive, s, e}); flags:
+ * SCCG_LIFT_START_INSIDE a record that begins before s reaches past it (the lifted start skips its ALT),
+ * SCCG_LIFT_END_INSIDE an owned record reaches past e, SCCG_LIFT_LENGTH_CHANGE an owned record changes length; for from = 1
+ * the same on the D side.  The sum same + subst + (the query's source bases inside length-changing records) is e - s.
+ * Splice identity (from = 0): up(D[start:end]) equals up(R[s:e]) with each owned record's reference span replaced by its
+ * ALT (a span that reaches past e taken whole) and the reference bases of [s, e) inside a record that begins before s
+ * dropped.  For from = 1, the mirror: up(R[start:end]) equals up(D[x:y]) with each owned record's D span replaced by
+ * up(R[pos:end]) (taken whole past y) and the D bases of [x, y) inside a record that begins before x dropped.
+ * Lift tables: each archive's records are kept on the device as a compact sorted table (record bounds in both systems and
+ * prefix sums of record lengths), one exactly-sized allocation held by the archive.  A call builds the tables of all its
+ * archives that have none in one pipeline run; later calls only search.  sccg_archive_info's device_bytes includes the table
+ * once built; sccg_archive_close and sccg_destroy release it.  A failed build (e.g. SCCG_E_NOMEM) leaves every archive
+ * without a partial table and usable.  An archive whose resident reference was replaced fails the checks below, so a table
+ * is never stale.
+ * Errors, all SCCG_E_ARG and all before any device work, in this order: a NULL pointer with a non-zero count or a negative
+ * count (2^31 or more archives or queries); then, the first failing check over all queries: the archive checks of
+ * sccg_archive_extract (index out of range, NULL archive, another context, a replaced or cleared resident reference), from
+ * not 0 or 1, start < 0 or start > end, end past len(R) (from = 0) or len(D) (from = 1).
+ * Each query does two binary searches of its archive's table.  Profile: h2d_ms (query table), gather_ms (lift kernel),
+ * kernels_ms (every kernel, table builds included: the build costs kernels_ms - gather_ms), d2h_ms (results), launches. */
+typedef struct { int64_t archive, start, end; int32_t from, reserved; } sccg_lift_query;
+typedef struct { int64_t start, end, same, subst, records; int32_t flags, reserved; } sccg_lift;
+enum { SCCG_LIFT_START_INSIDE = 1, SCCG_LIFT_END_INSIDE = 2, SCCG_LIFT_LENGTH_CHANGE = 4 };
+int sccg_archive_liftover(sccg_ctx* ctx, sccg_archive* const* archives, int64_t n_archives, const sccg_lift_query* queries, int64_t n_queries,
+                          sccg_lift* out);
 
 /* FASTA file images in: read_genomes_from_files (compression.cpp:181-220) and the reference reader of decompress_genome
  * (decompression.cpp:47-58) run on the device -- header lines skipped ('>' at a line start; in the target only the first one,

@@ -143,6 +143,7 @@ def load_library(path: str | os.PathLike | None = None) -> C.CDLL:
     lib.sccg_archive_search.argtypes = [vp, vp, i64, vp, i64, cp, vp, i64, C.c_int, C.c_int, vp, i64, i64p]
     lib.sccg_archive_search_edits.argtypes = [vp, vp, i64, vp, i64, cp, vp, i64, C.c_int, C.c_int, vp, i64, i64p]
     lib.sccg_archive_variants.argtypes = [vp, vp, i64, vp, i64, vp, i64, i64p, vp, i64, i64p]
+    lib.sccg_archive_liftover.argtypes = [vp, vp, i64, vp, i64, vp]
     lib.sccg_mgpu_unique_id.argtypes = [C.c_char_p]
     lib.sccg_mgpu_init.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.POINTER(vp)]
     lib.sccg_mgpu_destroy.argtypes = [vp]
@@ -273,7 +274,16 @@ class Archive:
         self.ctx, self.handle = ctx, handle
         n = C.c_int64(); mode = C.c_int(); nbytes = C.c_int64()
         ctx._check(ctx.lib.sccg_archive_info(handle, C.byref(n), C.byref(mode), C.byref(nbytes)))
-        self.seq_len, self.mode, self.device_bytes = n.value, mode.value, nbytes.value
+        self.seq_len, self.mode, self._device_bytes = n.value, mode.value, nbytes.value
+
+    @property
+    def device_bytes(self) -> int:
+        """device memory the archive holds (sccg_archive_info): its tables, plus its lift table once a liftover call built it"""
+        if self.handle:
+            n = C.c_int64()
+            self.ctx._check(self.ctx.lib.sccg_archive_info(self.handle, None, None, C.byref(n)))
+            self._device_bytes = n.value
+        return self._device_bytes
 
     def close(self):
         if self.handle:
@@ -697,6 +707,25 @@ class Context:
         v = buf[:n.value]
         rec = np.stack([v[f] for f, _ in self._VARIANT], axis=1).reshape(-1, 6).astype(np.int64)
         return rec, alt.raw[:na.value]
+
+    _LIFT_QUERY = [("archive", "<i8"), ("start", "<i8"), ("end", "<i8"), ("from", "<i4"), ("reserved", "<i4")]
+    _LIFT = [("start", "<i8"), ("end", "<i8"), ("same", "<i8"), ("subst", "<i8"), ("records", "<i8"), ("flags", "<i4"), ("reserved", "<i4")]
+
+    def liftover(self, archives, queries):
+        """intervals lifted between the resident reference and open archives (sccg_archive_liftover, include/sccg.h).  queries:
+        an (n, 4) int64 array of [archive index, start, end, from], from 0 for a reference interval lifted into the archive
+        and 1 for an archive interval lifted onto the reference.  -> an (n, 6) int64 array of [start, end, same, subst,
+        records, flags], one row per query in order.  The first call that names an archive builds its lift table."""
+        import numpy as np
+        q = np.asarray(queries, dtype=np.int64).reshape(-1, 4)
+        t = np.zeros(len(q), dtype=self._LIFT_QUERY)                     # sccg_lift_query[] layout
+        t["archive"], t["start"], t["end"] = q[:, 0], q[:, 1], q[:, 2]
+        t["from"] = np.where((q[:, 3] < -2**31) | (q[:, 3] >= 2**31), -1, q[:, 3]).astype(np.int32)   # (out of range stays invalid)
+        out = np.zeros(len(q), dtype=self._LIFT)
+        arr = (C.c_void_p * max(len(archives), 1))(*[a.handle for a in archives])
+        self._check(self.lib.sccg_archive_liftover(self.handle, arr if len(archives) else None, len(archives), t.ctypes.data if len(t) else None,
+                                                   len(t), out.ctypes.data if len(out) else None))
+        return np.stack([out[f].astype(np.int64) for f, _ in self._LIFT[:6]], axis=1).reshape(-1, 6)
 
     # decompress_genome (in-memory part) + reconstruct_genome + header line (decompression.cpp:66-110, :117-279, :322)
     def decompress(self, ref_raw: bytes, intermediate: bytes) -> bytes:

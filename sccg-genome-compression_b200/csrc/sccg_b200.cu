@@ -7,6 +7,7 @@
 #include "sccg_search.cuh"
 #include "sccg_search_edit.cuh"
 #include "sccg_variants.cuh"
+#include "sccg_liftover.cuh"
 #include "sccg_fasta.cuh"
 #include "sccg_shard.cuh"
 #include "sccg_mgpu.cuh"
@@ -616,6 +617,16 @@ int sccg_archive_variants(sccg_ctx* c, sccg_archive* const* archives, int64_t n_
     prof_reset(c);
     const int rc = archive_variants_impl(c, archives, n_archives, windows, n_windows, vars, vars_cap, n_vars, alt, alt_cap, alt_len);
     if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffers stays in flight
+    return rc;
+}
+
+int sccg_archive_liftover(sccg_ctx* c, sccg_archive* const* archives, int64_t n_archives, const sccg_lift_query* queries, int64_t n_queries,
+                          sccg_lift* out) {
+    if (!c) return set_error(SCCG_E_ARG, "null argument");
+    SCCG_CK(cudaSetDevice(c->device));
+    prof_reset(c);
+    const int rc = archive_liftover_impl(c, archives, n_archives, queries, n_queries, out);
+    if (rc != SCCG_OK) cudaStreamSynchronize(c->main_stream);              // no copy into the caller's buffer stays in flight
     return rc;
 }
 

@@ -34,6 +34,7 @@ enum Slot {
     B_GREF, B_GTGT, B_GKEYS, B_GVALS, B_GKEYS2, B_GVALS2, B_GHIST, B_GOFFS, B_GBUCKET, B_GREC, B_GLIT, B_GTMP0, B_GTMP1, B_GTMP2, B_GTMP3, B_GFIRST, B_SHARD,
     B_EXT_REG, B_EXT_IV, B_SRCH_TAB, B_SRCH_REG, B_SRCH_TILE, B_SRCH_HITS,
     B_VR_AGG, B_VR_SC, B_VR_TAB, B_VR_KEY, B_VR_CNT, B_VR_ANC, B_VR_GAP, B_VR_TILE, B_VR_REC3, B_VR_P, B_VR_WIN, B_VR_OUT,
+    B_LT_LO, B_LT_X, B_LT_Q, B_LT_OUT,
     B_NSLOTS
 };
 

@@ -535,7 +535,9 @@ struct sccg_archive {
     int mode;                      // 0: local-mode file, 1: global mode
     sccg::GatherArgs g;            // the tables (in mem) and the reference form they read; seg_src, tok_abs, err, out unused
     void* mem;                     // one exactly-sized allocation: record bytes, seg_dst, seg_ptr, N runs, lowercase runs
-    long long device_bytes;
+    long long device_bytes;        // mem, plus lift once built
+    void* lift;                    // the lift table (sccg_liftover.cuh), one exactly-sized allocation built by the first liftover call
+    long long lift_n;              // its records
 };
 
 namespace sccg {
@@ -573,6 +575,7 @@ static void reference_changed(sccg_ctx* c) {
 
 static void archive_free(sccg_archive* a) {
     if (a->mem) cudaFree(a->mem);
+    if (a->lift) cudaFree(a->lift);
     delete a;
 }
 

@@ -486,33 +486,16 @@ __global__ void __launch_bounds__(VR_T) vr_alt_k(VrArgs a, const sccg_variant* o
     }
 }
 
-// sccg_archive_variants: argument checks (include/sccg.h, in that order), then the pipeline above
-static int archive_variants_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, const sccg_window* windows, i64 n_windows,
-                                 sccg_variant* vars, i64 vars_cap, int64_t* n_vars, char* alt, i64 alt_cap, int64_t* alt_len) {
-    if (!n_vars || !alt_len || n_archives < 0 || n_windows < 0 || vars_cap < 0 || alt_cap < 0 || (n_archives > 0 && !archives) ||
-        (n_windows > 0 && !windows))
-        return set_error(SCCG_E_ARG, "null argument");
-    *n_vars = 0; *alt_len = 0;
-    if (n_archives >= 0x80000000LL || n_windows >= 0x80000000LL) return set_error(SCCG_E_ARG, "at most 2^31 - 1 archives and windows per call");
-    int first = ARCHIVE_QUERY_OK;
-    for (i64 i = 0; i < n_windows && first > 0; ++i) {
-        const sccg_window& W = windows[i];
-        const int f = archive_query_fault(c, archives, n_archives, W.archive, W.start, W.end);
-        const int bad = f < 4 ? f : (W.start < 0 || W.start > W.end) ? 4 : W.end > c->res_ref_len ? 5 : ARCHIVE_QUERY_OK;
-        if (bad < first) first = bad;
-    }
-    if (first == 5) return set_error(SCCG_E_ARG, "a window ends past the end of the resident reference");
-    if (first < ARCHIVE_QUERY_OK) return set_error(SCCG_E_ARG, archive_query_why[first]);
-    if (n_windows == 0) return SCCG_OK;
-    // ---- the archives the windows name, in index order: their elements (segments + sentinel) and the bounds that size the tables
-    std::vector<int> ord((size_t)n_archives, -1);
-    for (i64 i = 0; i < n_windows; ++i) ord[(size_t)windows[i].archive] = 0;
-    int n_arch = 0, n_global = 0;
+// steps 1-4 of include/sccg.h for the archives arcs[0 .. n_arch) (a record's window is the archive's ordinal there): the
+// staging table [VrArch of each archive | tail_bytes that fill(tail) writes] goes over in one copy (ev[4] -> ev[5]), and *d_tail
+// is the device copy of the tail.  Runs the anchors, gaps and per-tile record counts (ev[3] -> ev[2], added to *ms) and reads
+// the record total once into *nr; rec3 / recf are then sized for it.  vr_records_emit writes the records into a->recf.
+template <class Fill>
+static int vr_records_count(sccg_ctx* c, sccg_archive* const* arcs, int n_arch, size_t tail_bytes, Fill fill, VrArgs* out, u8** d_tail, u64* nr, float* ms) {
+    int n_global = 0;
     u64 n_elem = 0, anc_bound = 0, byte_bound = 0;
-    for (i64 k = 0; k < n_archives; ++k) {
-        if (ord[(size_t)k] < 0) continue;
-        ord[(size_t)k] = n_arch++;
-        const sccg_archive* a = archives[k];
+    for (int k = 0; k < n_arch; ++k) {
+        const sccg_archive* a = arcs[k];
         n_elem += (u64)a->g.nseg + 1;
         anc_bound += (u64)a->g.nseg + 1 + (a->mode ? (u64)a->g.n_k : 0);
         byte_bound += (u64)a->g.Lm + (u64)c->res_ref_len;
@@ -523,25 +506,23 @@ static int archive_variants_impl(sccg_ctx* c, sccg_archive* const* archives, i64
         anc_bound += (u64)n_global * (u64)c->res_nrun_k;
     }
     const u64 tile_bound = byte_bound / VR_TILE + 1;
-    // ---- staging: [VrArch of each named archive | VrWin of each window], one copy
-    const size_t arch_bytes = align_up(sizeof(VrArch) * (size_t)n_arch, 16), win_bytes = sizeof(VrWin) * (size_t)n_windows;
-    SCCG_TRY(ext_staging(c, arch_bytes + win_bytes));
+    // ---- staging: [VrArch of each archive | the caller's tail], one copy
+    const size_t arch_bytes = align_up(sizeof(VrArch) * (size_t)n_arch, 16);
+    SCCG_TRY(ext_staging(c, arch_bytes + tail_bytes));
     VrArch* h_arch = (VrArch*)c->h_ext;
-    VrWin* h_win = (VrWin*)((char*)c->h_ext + arch_bytes);
     {
         i64 e0 = 0;
-        for (i64 k = 0; k < n_archives; ++k) {
-            if (ord[(size_t)k] < 0) continue;
-            const sccg_archive* a = archives[k];
-            VrArch& A = h_arch[ord[(size_t)k]];
+        for (int k = 0; k < n_arch; ++k) {
+            const sccg_archive* a = arcs[k];
+            VrArch& A = h_arch[k];
             memset(&A, 0, sizeof A);
             A.g = a->g; A.e0 = e0; A.dlen = a->g.Lm; A.mode = a->mode;
             e0 += a->g.nseg + 1;
         }
-        for (i64 i = 0; i < n_windows; ++i) h_win[i] = VrWin{windows[i].start, windows[i].end, ord[(size_t)windows[i].archive]};
+        fill((char*)c->h_ext + arch_bytes);
     }
     u8* d_tab = nullptr; u64* sc = nullptr;
-    SCCG_TRY(buf(c, B_VR_TAB, arch_bytes + win_bytes, &d_tab));
+    SCCG_TRY(buf(c, B_VR_TAB, arch_bytes + tail_bytes, &d_tab));
     SCCG_TRY(buf(c, B_VR_SC, SC_COUNT, &sc));
     VrArgs a;
     memset(&a, 0, sizeof a);
@@ -556,9 +537,9 @@ static int archive_variants_impl(sccg_ctx* c, sccg_archive* const* archives, i64
     SCCG_TRY(buf(c, B_VR_GAP, (size_t)anc_bound * 16, &gp));
     a.goff = (u64*)gp; a.suf = (u32*)(gp + 8 * anc_bound); a.pre = a.suf + anc_bound;
     SCCG_TRY(buf(c, B_VR_TILE, (size_t)tile_bound, &a.tcnt));
-    const VrWin* d_win = (const VrWin*)(d_tab + arch_bytes);
+    *d_tail = d_tab + arch_bytes;
     SCCG_CK(cudaEventRecord(c->ev[4], c->stream));
-    SCCG_CK(cudaMemcpyAsync(d_tab, c->h_ext, arch_bytes + win_bytes, cudaMemcpyHostToDevice, c->stream));
+    SCCG_CK(cudaMemcpyAsync(d_tab, c->h_ext, arch_bytes + tail_bytes, cudaMemcpyHostToDevice, c->stream));
     SCCG_CK(cudaEventRecord(c->ev[5], c->stream));
     // ---- anchors, gaps, records per tile
     const unsigned grid = (unsigned)(c->sm_count > 0 ? c->sm_count : 1) * 8u;
@@ -578,20 +559,70 @@ static int archive_variants_impl(sccg_ctx* c, sccg_archive* const* archives, i64
     u64* h = (u64*)c->h_pinned;
     SCCG_CK(cudaMemcpyAsync(h, sc + SC_NR, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
     SCCG_CK(cudaStreamSynchronize(c->stream));
+    float t = 0.f;
+    cudaEventElapsedTime(&t, c->ev[3], c->ev[2]); *ms += t;
+    *nr = h[0];
+    SCCG_TRY(buf(c, B_VR_REC3, (size_t)*nr * 2 + 2, &a.rec3));
+    a.recf = a.rec3 + *nr + 1;
+    *out = a;
+    return SCCG_OK;
+}
+
+// the nr records of step 3, then each insertion / deletion left-aligned (step 4), into a.recf
+static int vr_records_emit(sccg_ctx* c, const VrArgs& a, u64 nr) {
+    const unsigned grid = (unsigned)(c->sm_count > 0 ? c->sm_count : 1) * 8u;
+    const unsigned rg = nr ? (div_up((long long)nr, VR_T) < grid ? div_up((long long)nr, VR_T) : grid) : 1;
+    LAUNCH(c, vr_emit_k, dim3(grid), dim3(VR_T), 0, a);
+    LAUNCH(c, vr_align_k, dim3(rg), dim3(VR_T), 0, a, nr);
+    return SCCG_OK;
+}
+
+// sccg_archive_variants: argument checks (include/sccg.h, in that order), then the pipeline above
+static int archive_variants_impl(sccg_ctx* c, sccg_archive* const* archives, i64 n_archives, const sccg_window* windows, i64 n_windows,
+                                 sccg_variant* vars, i64 vars_cap, int64_t* n_vars, char* alt, i64 alt_cap, int64_t* alt_len) {
+    if (!n_vars || !alt_len || n_archives < 0 || n_windows < 0 || vars_cap < 0 || alt_cap < 0 || (n_archives > 0 && !archives) ||
+        (n_windows > 0 && !windows))
+        return set_error(SCCG_E_ARG, "null argument");
+    *n_vars = 0; *alt_len = 0;
+    if (n_archives >= 0x80000000LL || n_windows >= 0x80000000LL) return set_error(SCCG_E_ARG, "at most 2^31 - 1 archives and windows per call");
+    int first = ARCHIVE_QUERY_OK;
+    for (i64 i = 0; i < n_windows && first > 0; ++i) {
+        const sccg_window& W = windows[i];
+        const int f = archive_query_fault(c, archives, n_archives, W.archive, W.start, W.end);
+        const int bad = f < 4 ? f : (W.start < 0 || W.start > W.end) ? 4 : W.end > c->res_ref_len ? 5 : ARCHIVE_QUERY_OK;
+        if (bad < first) first = bad;
+    }
+    if (first == 5) return set_error(SCCG_E_ARG, "a window ends past the end of the resident reference");
+    if (first < ARCHIVE_QUERY_OK) return set_error(SCCG_E_ARG, archive_query_why[first]);
+    if (n_windows == 0) return SCCG_OK;
+    // ---- the archives the windows name, in index order, then the records of steps 1-4 with the window table in the same copy
+    std::vector<int> ord((size_t)n_archives, -1);
+    for (i64 i = 0; i < n_windows; ++i) ord[(size_t)windows[i].archive] = 0;
+    std::vector<sccg_archive*> named;
+    for (i64 k = 0; k < n_archives; ++k)
+        if (ord[(size_t)k] >= 0) { ord[(size_t)k] = (int)named.size(); named.push_back(archives[k]); }
+    const size_t win_bytes = sizeof(VrWin) * (size_t)n_windows;
+    auto fill = [&](void* tail) {
+        VrWin* h_win = (VrWin*)tail;
+        for (i64 i = 0; i < n_windows; ++i) h_win[i] = VrWin{windows[i].start, windows[i].end, ord[(size_t)windows[i].archive]};
+    };
+    VrArgs a;
+    u8* d_tail = nullptr;
+    u64 nr = 0;
     float ms = 0.f, gat = 0.f;
-    cudaEventElapsedTime(&ms, c->ev[3], c->ev[2]); gat += ms;
-    const u64 nr = h[0];
+    SCCG_TRY(vr_records_count(c, named.data(), (int)named.size(), win_bytes, fill, &a, &d_tail, &nr, &gat));
+    const VrWin* d_win = (const VrWin*)d_tail;
+    u64* sc = a.sc;
+    u64* h = (u64*)c->h_pinned;
     // ---- records, left-alignment, the windows
-    SCCG_TRY(buf(c, B_VR_REC3, (size_t)nr * 2 + 2, &a.rec3));
-    a.recf = a.rec3 + nr + 1;
     u64 *P = nullptr, *wt = nullptr;
     SCCG_TRY(buf(c, B_VR_P, (size_t)nr + 1, &P));
     SCCG_TRY(buf(c, B_VR_WIN, 5 * (size_t)n_windows, &wt));
     u64 *woff = wt, *waoff = wt + n_windows, *wlo = wt + 2 * n_windows;
+    const unsigned grid = (unsigned)(c->sm_count > 0 ? c->sm_count : 1) * 8u;
     const unsigned rg = nr ? (div_up((long long)nr, VR_T) < grid ? div_up((long long)nr, VR_T) : grid) : 1;
     SCCG_CK(cudaEventRecord(c->ev[3], c->stream));
-    LAUNCH(c, vr_emit_k, dim3(grid), dim3(VR_T), 0, a);
-    LAUNCH(c, vr_align_k, dim3(rg), dim3(VR_T), 0, a, nr);
+    SCCG_TRY(vr_records_emit(c, a, nr));
     LAUNCH(c, vr_altlen_k, dim3(rg), dim3(VR_T), 0, (const sccg_variant*)a.recf, nr, P);
     SCCG_TRY(vr_scan<VrSum>(c, P, P, nullptr, nr, P + nr));
     LAUNCH(c, vr_win_k, dim3(div_up(n_windows, VR_T)), dim3(VR_T), 0, (const sccg_variant*)a.recf, nr, (const u64*)P, d_win, (u64)n_windows, a.rlen, woff, waoff, wlo);

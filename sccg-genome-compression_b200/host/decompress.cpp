@@ -39,6 +39,23 @@
 // following one (N if neither exists); substitutions and complex records are not padded.  ID, QUAL, FILTER and INFO are '.'.
 // REF and ALT hold ASCII letters only (IUPAC codes included): when a record's REF or ALT would hold any other byte (D and R
 // may hold any byte but '\n'), the command names the record's position, exits 1 and writes no variants.vcf.
+//
+// Additive: `decompress --liftover <bed> --archives <list> [--from reference|archive] <reference_file> <output_folder>` lifts
+// BED regions between reference coordinates and the coordinates of each archive's own sequence (sccg_archive_liftover;
+// archives unpacked and opened as above) and writes <output_folder>/lifted.bed.  --from reference (the default): every
+// region is lifted into every archive, archive by archive in list order and region by region in BED order (as regions.fa).
+// --from archive: column 1 of each line must be the stem of a listed archive (hits.bed of --search feeds back directly) and
+// lines keep their order; a line that names no listed archive is reported, the command exits 1 and writes no lifted.bed.
+// One line per lifted region: "chrom start end name same strand subst records flags source", tab-separated: chrom the
+// target system (the archive stem, or CHROM as variants.vcf names it), name BED column 4 and strand BED column 6 ("." when
+// absent), same / subst / records / flags as sccg_lift reports them, source "system:start-end" of the input interval.
+//
+// Additive: `decompress --regions <bed> --archives <list> --reference-coords <reference_file> <output_folder>` extracts every
+// BED region, given in reference coordinates, from every archive: one sccg_archive_liftover call, then one
+// sccg_archive_extract call of the lifted pieces.  regions.fa holds the records and labels of `--regions --archives`, with
+// the BED's reference coordinates in the label (the same gene carries the same label in every archive); a minus-strand
+// record holds the reverse complement of the lifted piece.
+#include <algorithm>
 #include <cstdlib>
 #include <filesystem>
 #include <iostream>
@@ -106,7 +123,8 @@ static int decompress_one(Worker& w, const Job& job, Timing& tm, bool verbose) {
 // BED lines: "name start end [more columns]", separated by tabs or spaces; blank lines and "#", "track", "browser" lines are
 // skipped.  false (with a message) on anything else.
 // with_strand: column 6, when present, must be "+", "-" or "." (strand 1 for "-")
-struct BedRegion { std::string name; int64_t start, end; int strand = 0; };
+// label / strand_text: column 4 and column 6 as written ("." when absent); line: the line number
+struct BedRegion { std::string name; int64_t start, end; int strand = 0; std::string label = ".", strand_text = "."; int64_t line = 0; };
 static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std::string* err, bool with_strand = false) {
     std::istringstream in(text);
     std::string line;
@@ -136,6 +154,9 @@ static bool parse_bed(const std::string& text, std::vector<BedRegion>* out, std:
             r.strand = f[5] == "-";
         }
         r.name = f[0];
+        if (f.size() >= 4) r.label = f[3];
+        if (f.size() >= 6) r.strand_text = f[5];
+        r.line = no;
         out->push_back(r);
     }
     return true;
@@ -424,6 +445,28 @@ static int search_archives(int argc, char* argv[]) {
     return 0;
 }
 
+// the reference FASTA's symbols and its CHROM: the first word of its first header line (the file stem when there is none);
+// false (with a message) when it cannot be read
+static bool reference_symbols(const std::string& ref_path, std::string* ref, std::string* chrom) {
+    std::string ref_file;
+    if (!sccg_host::read_file(ref_path, ref_file)) { std::cerr << "Greska pri otvaranju reference: " << ref_path << "\n"; return false; }
+    sccg_host::parse_fasta(ref_file, false, *ref, nullptr);
+    chrom->clear();
+    for (size_t p = 0; p < ref_file.size();) {                              // the first header line's first word
+        const size_t e = ref_file.find('\n', p);
+        const std::string line = ref_file.substr(p, e == std::string::npos ? std::string::npos : e - p);
+        if (!line.empty() && line[0] == '>') {
+            const size_t w = line.find_first_of(" \t\r", 1);
+            *chrom = line.substr(1, w == std::string::npos ? std::string::npos : w - 1);
+            break;
+        }
+        if (e == std::string::npos) break;
+        p = e + 1;
+    }
+    if (chrom->empty()) *chrom = fs::path(ref_path).stem().string();
+    return true;
+}
+
 // the VCF of `--variants` (format in the header comment)
 static int variants_archives(int argc, char* argv[]) {
     const char *list_path = nullptr, *bed_path = nullptr;
@@ -445,21 +488,8 @@ static int variants_archives(int argc, char* argv[]) {
     }
     std::vector<std::string> arcs;
     if (!read_archive_list(list_path, &arcs)) return 1;
-    std::string ref_file, ref, chrom;
-    if (!sccg_host::read_file(ref_path, ref_file)) { std::cerr << "Greska pri otvaranju reference: " << ref_path << "\n"; return 1; }
-    sccg_host::parse_fasta(ref_file, false, ref, nullptr);
-    for (size_t p = 0; p < ref_file.size();) {                              // the first header line's first word
-        const size_t e = ref_file.find('\n', p);
-        const std::string line = ref_file.substr(p, e == std::string::npos ? std::string::npos : e - p);
-        if (!line.empty() && line[0] == '>') {
-            const size_t w = line.find_first_of(" \t\r", 1);
-            chrom = line.substr(1, w == std::string::npos ? std::string::npos : w - 1);
-            break;
-        }
-        if (e == std::string::npos) break;
-        p = e + 1;
-    }
-    if (chrom.empty()) chrom = fs::path(ref_path).stem().string();
+    std::string ref, chrom;
+    if (!reference_symbols(ref_path, &ref, &chrom)) return 1;
     for (const BedRegion& r : bed)
         if (r.end > (int64_t)ref.size()) { std::cerr << "Error: region " << r.name << ":" << r.start << "-" << r.end << " ends past the end of the reference (" << ref.size() << " bp)\n"; return 1; }
     sccg_ctx* ctx = resident_context(ref_path);
@@ -525,25 +555,145 @@ static int variants_archives(int argc, char* argv[]) {
     return 0;
 }
 
+// `--liftover` (lifted.bed) and `--regions --reference-coords` (regions.fa): BED regions lifted between the reference and the
+// archives of the list (format in the header comment).  from: 0 reference -> archive, 1 archive -> reference.
+static int lift_archives(const char* bed_path, const char* list_path, int from, bool extract, const std::string& ref_path, const std::string& out_dir) {
+    std::string bed_text, err, ref, chrom;
+    std::vector<BedRegion> bed;
+    if (!sccg_host::read_file(bed_path, bed_text)) { std::cerr << "Error opening BED file: " << bed_path << "\n"; return 1; }
+    if (!parse_bed(bed_text, &bed, &err, true)) { std::cerr << "Error: " << err << "\n"; return 1; }
+    std::vector<std::string> arcs, stems;
+    if (!read_archive_list(list_path, &arcs)) return 1;
+    for (const std::string& arc : arcs) stems.push_back(fs::path(arc).stem().string());
+    if (!reference_symbols(ref_path, &ref, &chrom)) return 1;
+    std::vector<int64_t> src_arc(bed.size(), 0);                             // --from archive: the archive each line names
+    for (size_t i = 0; i < bed.size(); ++i) {
+        const BedRegion& r = bed[i];
+        if (from == 1) {
+            const auto it = std::find(stems.begin(), stems.end(), r.name);
+            if (it == stems.end()) { std::cerr << "Error: BED line " << r.line << " names no listed archive: " << r.name << "\n"; return 1; }
+            src_arc[i] = it - stems.begin();
+        } else if (r.end > (int64_t)ref.size()) {
+            std::cerr << "Error: region " << r.name << ":" << r.start << "-" << r.end << " ends past the end of the reference (" << ref.size() << " bp)\n";
+            return 1;
+        }
+    }
+    sccg_ctx* ctx = resident_context(ref_path);
+    if (!ctx) return 1;
+    std::error_code ec;
+    if (!fs::exists(out_dir)) fs::create_directory(out_dir, ec);
+    int status = 1;
+    std::vector<sccg_archive*> open;
+    std::vector<sccg_lift_query> qs;
+    std::vector<size_t> q_bed;                                              // the BED line of each query
+    std::string text;
+    [&] {
+        for (const std::string& arc : arcs) {                               // unpacked one at a time: archives may share a file name
+            sccg_archive* a = open_archive_file(ctx, arc, out_dir);
+            if (!a) return;
+            open.push_back(a);
+        }
+        for (size_t i = 0; i < bed.size(); ++i) {
+            const BedRegion& r = bed[i];
+            if (from == 0) continue;
+            int64_t seq_len = 0;
+            sccg_archive_info(open[(size_t)src_arc[i]], &seq_len, nullptr, nullptr);
+            if (r.end > seq_len) { std::cerr << "Error: region " << r.name << ":" << r.start << "-" << r.end << " ends past the end of " << arcs[(size_t)src_arc[i]] << " (" << seq_len << " bp)\n"; return; }
+            qs.push_back(sccg_lift_query{src_arc[i], r.start, r.end, 1, 0});
+            q_bed.push_back(i);
+        }
+        if (from == 0)                                                      // archive by archive, region by region (as regions.fa)
+            for (size_t k = 0; k < open.size(); ++k)
+                for (size_t i = 0; i < bed.size(); ++i) { qs.push_back(sccg_lift_query{(int64_t)k, bed[i].start, bed[i].end, 0, 0}); q_bed.push_back(i); }
+        std::vector<sccg_lift> lifted(qs.size());
+        if (sccg_archive_liftover(ctx, open.data(), (int64_t)open.size(), qs.data(), (int64_t)qs.size(), lifted.data()) != SCCG_OK) {
+            std::cerr << "Error: " << sccg_last_error() << "\n";
+            return;
+        }
+        if (!extract) {
+            for (size_t j = 0; j < qs.size(); ++j) {
+                const BedRegion& r = bed[q_bed[j]];
+                const sccg_lift& l = lifted[j];
+                const std::string target = from ? chrom : stems[(size_t)qs[j].archive], source = from ? r.name : chrom;
+                text += target + "\t" + std::to_string(l.start) + "\t" + std::to_string(l.end) + "\t" + r.label + "\t" + std::to_string(l.same) + "\t" +
+                        r.strand_text + "\t" + std::to_string(l.subst) + "\t" + std::to_string(l.records) + "\t" + std::to_string(l.flags) + "\t" +
+                        source + ":" + std::to_string(r.start) + "-" + std::to_string(r.end) + "\n";
+            }
+            status = 0;
+            return;
+        }
+        // --reference-coords: the lifted pieces, one sccg_archive_extract call; records and labels as --regions --archives
+        std::vector<sccg_query> eq(qs.size());
+        int64_t total = 0, out_len = 0;
+        for (size_t j = 0; j < qs.size(); ++j) {
+            eq[j] = sccg_query{qs[j].archive, lifted[j].start, lifted[j].end, bed[q_bed[j]].strand};
+            total += lifted[j].end - lifted[j].start;
+        }
+        std::vector<char> seq((size_t)total + 1);
+        if (sccg_archive_extract(ctx, open.data(), (int64_t)open.size(), eq.data(), (int64_t)eq.size(), seq.data(), total, &out_len) != SCCG_OK) {
+            std::cerr << "Error: " << sccg_last_error() << "\n";
+            return;
+        }
+        text.reserve((size_t)total + (size_t)total / 50 + qs.size() * 48);
+        int64_t at = 0;
+        for (size_t j = 0; j < qs.size(); ++j) {
+            const BedRegion& r = bed[q_bed[j]];
+            text += ">" + stems[(size_t)qs[j].archive] + "::" + r.name + ":" + std::to_string(r.start) + "-" + std::to_string(r.end) + (r.strand ? "(-)" : "") + "\n";
+            for (int64_t p = eq[j].start; p < eq[j].end; p += 50) {
+                const int64_t n = eq[j].end - p < 50 ? eq[j].end - p : 50;
+                text.append(seq.data() + at, (size_t)n); text += '\n';
+                at += n;
+            }
+        }
+        status = 0;
+    }();
+    sccg_destroy(ctx);                                                      // (releases the archives)
+    if (status) return status;
+    if (!write_output(out_dir + (extract ? "/regions.fa" : "/lifted.bed"), text)) { std::cerr << "Error opening output file: " << out_dir << "\n"; return 1; }
+    return 0;
+}
+
+static int liftover_archives(int argc, char* argv[]) {
+    const char* list_path = nullptr;
+    int from = 0;
+    int i = 3;
+    for (; i + 1 < argc - 2; i += 2) {
+        const std::string opt = argv[i], v = argv[i + 1];
+        if (opt == "--archives") list_path = argv[i + 1];
+        else if (opt == "--from") {
+            if (v != "reference" && v != "archive") { std::cerr << "Error: --from takes reference or archive\n"; return 1; }
+            from = v == "archive";
+        } else { std::cerr << "Error: unknown option " << opt << "\n"; return 1; }
+    }
+    if (i != argc - 2 || !list_path) { std::cerr << "Error: --liftover needs --archives <list>, then <reference_file> <output_folder>\n"; return 1; }
+    return lift_archives(argv[2], list_path, from, false, argv[argc - 2], argv[argc - 1]);
+}
+
 int main(int argc, char* argv[]) {
     const bool batch = argc >= 3 && std::string(argv[1]) == "--batch";
     const bool regions = argc == 6 && std::string(argv[1]) == "--regions";
     const bool archives = argc == 7 && std::string(argv[1]) == "--regions" && std::string(argv[3]) == "--archives";
+    const bool ref_coords = argc == 8 && std::string(argv[1]) == "--regions" && std::string(argv[3]) == "--archives" && std::string(argv[5]) == "--reference-coords";
+    const bool liftover = argc >= 6 && std::string(argv[1]) == "--liftover";
     const bool search = argc >= 7 && std::string(argv[1]) == "--search";
     const bool variants = argc >= 6 && std::string(argv[1]) == "--variants";
-    if (argc != 4 && !batch && !regions && !archives && !search && !variants) {          // decompression.cpp:283-286
+    if (argc != 4 && !batch && !regions && !archives && !ref_coords && !search && !variants && !liftover) {          // decompression.cpp:283-286
         std::cerr << "Usage: " << argv[0] << " <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --batch <list of such triples, one per line> [--gpus N]\n"
                   << "       " << argv[0] << " --regions <regions.bed> <compressed_file> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --regions <regions.bed> --archives <list of .7z files, one per line> <reference_file> <output_folder>\n"
                   << "       " << argv[0] << " --search <patterns.fa> --archives <list> [--regions <bed>] [--mismatches K | --edits K] [--strand both|+|-] <reference_file> <output_folder>\n"
-                  << "       " << argv[0] << " --variants --archives <list> [--regions <bed>] <reference_file> <output_folder>\n";
+                  << "       " << argv[0] << " --variants --archives <list> [--regions <bed>] <reference_file> <output_folder>\n"
+                  << "       " << argv[0] << " --liftover <bed> --archives <list> [--from reference|archive] <reference_file> <output_folder>\n"
+                  << "       " << argv[0] << " --regions <bed> --archives <list> --reference-coords <reference_file> <output_folder>\n";
         return 1;
     }
     try {
         if (archives) return extract_archives(argv[2], argv[4], argv[5], argv[6]);
         if (search) return search_archives(argc, argv);
         if (variants) return variants_archives(argc, argv);
+        if (liftover) return liftover_archives(argc, argv);
+        if (ref_coords) return lift_archives(argv[2], argv[4], 0, true, argv[6], argv[7]);
         if (regions) {
             Job job; job.a = argv[3]; job.b = argv[4]; job.out = argv[5];
             return extract_regions(argv[2], job);
